@@ -2,6 +2,7 @@
 """bench.py -- throughput of LaTok's tokenization hot path on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload tweets|mixed|docs|chars1b] [--impl reference]
+                    [--dump-outputs DIR]
 
 One step = one pass of the hot path (split mask + token spans + CSR offsets) over one batch of
 synthetic text.  Top-level line: BASELINE config #2, 1 M tweet-sized strings per GPU (seed 20240601).
@@ -18,6 +19,8 @@ Reported on ONE JSON line (rank 0):
                  ms per pass, and the same batch on one GPU in the same run (speed-up)
   python_dropin  (N=1) the Python drop-in: C-side packing of list[str], tokenize_batch, tokenize_packed().to_arrow()
   cpu_baseline   the compiled reference (oracle/_ref) on all host cores over a bounded sample (rank 0, N=1)
+--dump-outputs DIR writes the arrays the last timed step of the top-level measurement returned (rank 0) to DIR/*.npy,
+so that two builds can be compared output for output on the same seeded inputs (see dump_outputs).
 N > 1 is launched by torchrun (one rank per GPU); ranks hold different batches (weak scaling), there is
 no data-path collective; the span-count exchange is one all_gather of an int64 per rank.
 """
@@ -212,6 +215,7 @@ class ClockSampler(threading.Thread):
     def __init__(self, device_index):
         super().__init__(daemon=True)
         self.samples, self.reasons, self.max_mhz, self.stop_flag, self.ok = [], set(), None, False, False
+        self.paused = False             # set while the host works and the GPU idles (--dump-outputs)
         try:
             import pynvml
             pynvml.nvmlInit()
@@ -231,6 +235,9 @@ class ClockSampler(threading.Thread):
                  "sw_thermal_slowdown": getattr(nv, "nvmlClocksEventReasonSwThermalSlowdown", 0x20),
                  "sw_power_cap": getattr(nv, "nvmlClocksEventReasonSwPowerCap", 0x4)}
         while not self.stop_flag:
+            if self.paused:
+                time.sleep(0.004)
+                continue
             try:
                 self.samples.append(nv.nvmlDeviceGetClockInfo(self.h, nv.NVML_CLOCK_SM))
                 try:
@@ -318,9 +325,31 @@ def load_peak():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
-def measure_resident(cx: Ctx, host, what, steps, warmup, classify, wl_key, sample_clocks=True):
+DUMP_ARRAYS = ("splits", "char_offsets", "spans", "tok_offsets", "tok_feats")
+DUMP_BYTES_PER_ARRAY = 12 << 20                 # five arrays at most: 60 MB in all
+
+
+def dump_outputs(r, out_dir, seed=0):
+    """Writes the arrays of the BatchResult `r` as out_dir/<name>.npy: int8 arrays as float32, wider integers as
+    float64 (every value exact).  An array larger than DUMP_BYTES_PER_ARRAY keeps a sample of its rows, in order,
+    drawn with a fixed seed from its length alone: two builds that agree on the sizes dump the same rows."""
+    out_dir = Path(out_dir)
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name in DUMP_ARRAYS:
+        a = getattr(r, name)
+        if a is None:
+            continue
+        dtype = np.dtype(np.float32 if a.dtype.itemsize == 1 else np.float64)
+        keep = DUMP_BYTES_PER_ARRAY // (dtype.itemsize * int(np.prod(a.shape[1:], dtype=np.int64)))
+        if len(a) > keep:
+            a = a[np.sort(np.random.default_rng(seed).choice(len(a), keep, replace=False))]
+        np.save(out_dir / f"{name}.npy", a.astype(dtype))
+
+
+def measure_resident(cx: Ctx, host, what, steps, warmup, classify, wl_key, sample_clocks=True, dump_dir=None):
     """Device-resident pass: `host` = list of (buf, offsets) batches of this rank, rotated; returns the fields of a
-    bench record (value, ms_per_step, roofline, clocks, ...) plus the per-batch stats."""
+    bench record (value, ms_per_step, roofline, clocks, ...) plus the per-batch stats.  `dump_dir`: rank 0 writes the
+    results of the last timed step there (dump_outputs)."""
     from latok_b200 import _lib
     torch, eng, lib = cx.torch, cx.eng, cx.lib
     R = len(host)
@@ -350,6 +379,14 @@ def measure_resident(cx: Ctx, host, what, steps, warmup, classify, wl_key, sampl
     elapsed_ms = eng.timer_end()
     cx.barrier()
     launches = eng.launch_count() - launches0
+    if dump_dir and cx.rank == 0:
+        # before the launches below replace the last timed step's results; the clocks of the idle GPU meanwhile are
+        # not the clocks of the workload
+        if sampler:
+            sampler.paused = True
+        dump_outputs(eng.fetch(), dump_dir)
+        if sampler:
+            sampler.paused = False
     # per-launch duration of the dominant kernel, measured live (CUDA events around the tokenize kernel on the
     # stream it is launched on), one step at a time after the timed region
     kernel_ms = []
@@ -532,7 +569,9 @@ def python_dropin(cx: Ctx, hb, ho, n=200_000):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=200)
+    ap.add_argument("--steps", type=int, default=200,
+                    help="timed steps of the top-level measurement, on every workload (docs: each step is one pass over "
+                         "3.2 GB of text); up to 50 more follow, one at a time, for the per-launch kernel time")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="tweets", choices=list(WORKLOADS))
@@ -542,7 +581,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-others", action="store_true", help="skip other_configs / config5_strong / python_dropin")
     ap.add_argument("--strong-strings", type=int, default=0, help="override the size of the config-#5 batch (NOT the named config)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the results of the last timed step to DIR/<name>.npy "
+                    "(float32 / float64; arrays over 12 MB as a seeded sample of their rows)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference leg returns token counts only")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -602,8 +647,9 @@ def main():
         host = [strong_shard(*data.pop("strong"))]
     else:
         host = [data.pop(f"top{r}") for r in range(R)]
-    steps = args.steps if wl != "docs" else min(args.steps, 20)
-    top, stats = measure_resident(cx, host, what, steps, args.warmup, classify, wl if not args.strings else "")
+    steps = args.steps
+    top, stats = measure_resident(cx, host, what, steps, args.warmup, classify, wl if not args.strings else "",
+                                  dump_dir=args.dump_outputs)
     if world > 1:
         # the path's only cross-GPU datum: per-rank token counts, to rebase global token offsets
         counts = torch.zeros(world, device="cuda", dtype=torch.int64)

@@ -9,9 +9,8 @@
  * Parity status: PINNED.  tests/test_oracle_cpu.py checks every function here
  * against (a) the reference's only golden vector, the executed notebook cell
  * notebooks/scratch/LaTokenizer.ipynb:1263-1430 (tests/golden/notebook_cell.json),
- * (b) fixtures produced by the reference's own latok.c compiled in the build
- * container (oracle/Makefile target `ref`, generator tests/golden/make_golden.py),
- * and (c) when oracle/_ref is present, live differential fuzzing against it.
+ * and (b) fixtures produced by the reference's own latok.c compiled in the build
+ * container (oracle/Makefile target `ref`, generator tests/golden/make_golden.py).
  *
  * Each function cites the reference lines it restates (paths relative to the
  * reference checkout).  The code is a plain sequential restatement: one string

@@ -282,14 +282,18 @@ def test_table_regeneration_rules_reproduce_ucd11():
         assert rc.read_ranges(out) == feat
 
 
+def load_bench():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", ROOT / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
 def test_bench_config5_batch_shards_cover_the_batch():
     """bench.py --workload chars1b: every rank builds the same batch and keeps its byte-balanced range of whole
     strings; the ranges tile the batch and are balanced to within one string."""
-    import importlib.util
-    root = Path(__file__).resolve().parent.parent
-    spec = importlib.util.spec_from_file_location("bench_mod", root / "bench.py")
-    bench = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(bench)
+    bench = load_bench()
     from latok_b200.sharding import shard_ranges, slice_shard
     buf, off = bench.make_batch("chars1b", 6000, 0)
     buf2, off2 = bench.make_batch("chars1b", 6000, 0)
@@ -303,6 +307,38 @@ def test_bench_config5_batch_shards_cover_the_batch():
         assert np.array_equal(np.concatenate([p[0] for p in parts]), buf)
         sizes = [len(p[0]) for p in parts]
         assert max(sizes) - min(sizes) <= 2 * int(np.diff(off).max())
+
+
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs: every array of the result as float32 / float64 .npy with exact values, the ones over
+    the per-array budget as the same seeded, ordered sample of rows on every call, under 64 MB in all."""
+    bench = load_bench()
+    from latok_b200.engine import BatchResult
+    S, C_, T = 1000, 4_000_000, 1_000_000
+    rng = np.random.default_rng(1)
+    r = BatchResult(S, C_, T, splits=rng.integers(0, 3, C_).astype(np.int8),
+                    char_offsets=np.linspace(0, C_, S + 1).astype(np.int64) + (1 << 40),
+                    spans=np.stack([np.arange(T), 3 * np.arange(T)], axis=1).astype(np.int32),
+                    tok_offsets=np.linspace(0, T, S + 1).astype(np.int64),
+                    tok_feats=rng.integers(-128, 128, (T, 25)).astype(np.int8))
+    for d in ("a", "b"):
+        bench.dump_outputs(r, tmp_path / d)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == sorted(f"{n}.npy" for n in bench.DUMP_ARRAYS)
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) < 64 << 20
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f))
+    got = {f[:-4]: np.load(tmp_path / "a" / f) for f in files}
+    assert got["splits"].dtype == got["tok_feats"].dtype == np.float32
+    assert got["spans"].dtype == got["char_offsets"].dtype == got["tok_offsets"].dtype == np.float64
+    assert np.array_equal(got["char_offsets"], r.char_offsets) and np.array_equal(got["tok_offsets"], r.tok_offsets)
+    rows = got["spans"][:, 0].astype(np.int64)                 # spans row i is (i, 3 i): the sample's row numbers
+    assert 0 < len(rows) < T and np.all(np.diff(rows) > 0) and np.array_equal(got["spans"][:, 1], 3 * rows)
+    assert 0 < len(got["splits"]) < C_ and set(np.unique(got["splits"])) <= {0.0, 1.0, 2.0}
+    n = len(got["tok_feats"])
+    assert 0 < n < T and got["tok_feats"].shape[1] == 25
+    pick = np.sort(np.random.default_rng(0).choice(T, n, replace=False))
+    assert np.array_equal(got["tok_feats"], r.tok_feats[pick])
 
 
 def test_native_csv_reader_matches_python_csv_json(tmp_path):

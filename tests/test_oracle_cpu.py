@@ -2,18 +2,16 @@
   * the reference's one stored golden vector (executed notebook cell),
   * committed outputs of the compiled reference on the fixture corpus (tests/golden),
   * sha256 digests of the compiled reference over 12 300 fuzz strings,
-  * every code point's class as read off the compiled reference,
-  * and, where oracle/_ref is present, a live differential fuzz against it.
+  * and every code point's class as read off the compiled reference.
 No GPU needed."""
 import hashlib
 import json
 import zlib
 
 import numpy as np
-import pytest
 
 import corpus
-from oracle import oracle, ref_driver
+from oracle import oracle
 
 
 def words_to_matrix(words):
@@ -138,40 +136,3 @@ def test_block_mask_scan_form():
                     start = i + 1
         assert np.array_equal(got, want), (a1, a2, got, want)
 
-
-@pytest.mark.skipif(not ref_driver.available(), reason="oracle/_ref not built")
-def test_live_differential_against_compiled_reference():
-    ext = ref_driver.ext()
-    texts = [t for t in corpus.fuzz_strings(2024, 3000, 90) + corpus.fuzz_strings(2025, 2000, 90, "marks") if t]
-    for t in texts:
-        m_ref = ext._gen_parse_matrix(t)
-        m = oracle.parse_matrix(t)
-        assert np.array_equal(m, m_ref), t
-        assert np.array_equal(oracle.split_mask(m), ref_driver.gen_split_mask(m_ref)), t
-        assert oracle.tokens(t) == list(ref_driver.tokenize(t)), t
-        sp, ft = ref_driver.featurize_arrays(t)
-        s = oracle.split_mask(m)
-        osp, _ = oracle.spans(s, m)
-        assert np.array_equal(osp, sp), t
-        assert np.array_equal(oracle.token_feats(m, osp), ft), t
-    # the three extension functions on raw arrays
-    rng = np.random.default_rng(9)
-    for _ in range(500):
-        n = int(rng.integers(1, 60))
-        a1 = (rng.random(n) < 0.15).astype(np.int8)
-        a2 = (rng.random(n) < 0.2).astype(np.int8)
-        assert np.array_equal(oracle.block_mask(a1, a2), ext._gen_block_mask(a1, a2))
-        m = rng.integers(0, 3, size=(25, n)).astype(np.int8)
-        for idx in oracle.DEFAULT_RULES:
-            assert np.array_equal(oracle.combine_rows(m, idx), ext._combine_matrix_rows(m, idx))
-        rows = rng.integers(0, 25, size=int(rng.integers(1, 8))).astype(np.int8)
-        assert np.array_equal(oracle.combine_rows(m, rows), ext._combine_matrix_rows(m, rows))
-
-
-@pytest.mark.skipif(ref_driver.ref_python() is None, reason="needs the reference checkout")
-def test_restated_glue_matches_reference_python():
-    rp = ref_driver.ref_python()
-    for t in corpus.FIXTURES + [x for x in corpus.fuzz_strings(77, 500, 60) if x]:
-        m = rp._gen_parse_matrix(t)
-        assert np.array_equal(ref_driver.gen_split_mask(m), rp.gen_split_mask(m))
-        assert list(ref_driver.tokenize(t)) == list(rp.tokenize(t))
