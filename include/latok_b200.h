@@ -137,6 +137,41 @@ LATOK_B200_API int latok_b200_device_results(latok_b200_engine *e, const int8_t 
                               const int32_t **spans, const int64_t **tok_offsets,
                               const int8_t **tok_feats, const int8_t **matrix);
 
+/* ---- token vocabulary: corpus token counts and integer token ids on the device ------------------
+ * The counterpart of a `collections.Counter` over the tokens of tokenize_batch, or of a dict lookup per token, without
+ * a Python string per token (no counterpart in the reference, which yields token strings, default_tokenizer.py:151-158).
+ * A vocabulary lives on one device; its keys are the exact trimmed token bytes (what fetch_token_bytes ranges select:
+ * `text[s:e].strip()` as UTF-8 with lone surrogates encoded as 'surrogatepass' does); ids are dense, 0 .. n_keys - 1,
+ * in the order of first occurrence (within a batch: token order).  A batch commits all at once or not at all.
+ * Device memory held: the hash table (16 + 8 bytes per slot, at least 2 slots per key, power-of-two capacity, grown
+ * 4x when the load passes one half), the key arena (key bytes + 16 bytes per key: offsets and counts) and 8 bytes per
+ * token of the largest batch; encode also uses the engine's 16 bytes per token for the token byte ranges.
+ * LATOK_B200_VOCAB_HASH_BITS=n (read at creation; tests only) keeps n bits of the hash to force collisions. */
+typedef struct latok_b200_vocab latok_b200_vocab;
+/* An empty vocabulary on e's device, sized for expected_keys keys (more grow the table). */
+LATOK_B200_API int latok_b200_vocab_create(latok_b200_engine *e, int64_t expected_keys, latok_b200_vocab **out);
+LATOK_B200_API int latok_b200_vocab_destroy(latok_b200_vocab *v);
+/* The tokens of the engine's (oldest) batch in flight (needs LATOK_B200_SPANS and the submitted text still in place, as
+ * for fetch_token_bytes).  add != 0: every token is counted, keys not in the vocabulary get the next ids; add == 0:
+ * read-only, a token not in the vocabulary gets unk_id.  ids: int32 [T] in token order (CSR = tok_offsets of fetch),
+ * in host memory or, with on_device != 0, in device memory (4-byte aligned); NULL skips them.  cap_tokens = room in
+ * ids (EINVAL when the batch has more tokens).  Runs on the engine's compute stream after the batch's kernels;
+ * EINVAL for a vocabulary on another device, or one that would pass 2^31 - 1 keys (nothing is committed then). */
+LATOK_B200_API int latok_b200_vocab_encode(latok_b200_engine *e, latok_b200_vocab *v, int add, int32_t unk_id,
+                                           int64_t cap_tokens, int32_t *ids, int on_device);
+/* keys, their bytes, and the slots of the hash table (load = n_keys / table_slots); any pointer may be NULL */
+LATOK_B200_API int latok_b200_vocab_size(latok_b200_vocab *v, int64_t *n_keys, int64_t *key_bytes, int64_t *table_slots);
+/* Keys in id order into host buffers (any may be NULL): bytes [key_bytes], offsets [n_keys + 1] (key i =
+ * bytes[offsets[i] : offsets[i + 1]]), counts int64 [n_keys].  cap_keys / cap_bytes = room, as in fetch. */
+LATOK_B200_API int latok_b200_vocab_export(latok_b200_vocab *v, int64_t cap_keys, int64_t cap_bytes,
+                                           uint8_t *bytes, int64_t *offsets, int64_t *counts);
+/* Adds n_keys keys (host bytes + offsets [n_keys + 1]) with the ids n_keys_before + position and the given counts
+ * (NULL: 0).  A key that is empty, repeated, or already in the vocabulary is EINVAL (nothing is added then). */
+LATOK_B200_API int latok_b200_vocab_import(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *bytes,
+                                           const int64_t *offsets, int64_t n_keys, const int64_t *counts);
+/* device time of the last encode / import (token byte ranges included; harness) */
+LATOK_B200_API int latok_b200_vocab_last_ms(latok_b200_vocab *v, float *ms);
+
 /* ---- measurement hooks (harness only) ----------------------------------------------------- */
 /* CUDA-event bracket on the engine's compute stream around any number of submits. */
 LATOK_B200_API int latok_b200_timer_begin(latok_b200_engine *e);

@@ -3,6 +3,7 @@ spans -> per-token feature sums) as hand-written sm_100a CUDA behind LaTok's own
 
     from latok_b200.core.default_tokenizer import tokenize, featurize, tokenize_batch
     import latok_b200; latok_b200.install_as_latok()   # `import latok.core.default_tokenizer` now resolves here
+    from latok_b200.vocab import Vocab     # token counts and integer token ids on the GPU (Counter / dict lookup)
 
 Everything numeric happens in liblatok_b200.so (C ABI: include/latok_b200.h).  There is no CPU
 fallback: without the library or without a CUDA device the compute calls raise.

@@ -65,6 +65,13 @@ def load():
         "latok_b200_gen_parse_matrix": (C.c_int, [vp, vp, i64, P(i64), vp]),
         "latok_b200_gen_block_mask": (C.c_int, [vp, vp, i64, vp, i64, i64, vp]),
         "latok_b200_combine_matrix_rows": (C.c_int, [vp, vp, i64, i64, i64, i64, vp, i32, i32, vp]),
+        "latok_b200_vocab_create": (C.c_int, [vp, i64, P(vp)]),
+        "latok_b200_vocab_destroy": (C.c_int, [vp]),
+        "latok_b200_vocab_encode": (C.c_int, [vp, vp, i32, C.c_int32, i64, vp, i32]),
+        "latok_b200_vocab_size": (C.c_int, [vp, P(i64), P(i64), P(i64)]),
+        "latok_b200_vocab_export": (C.c_int, [vp, i64, i64, vp, vp, vp]),
+        "latok_b200_vocab_import": (C.c_int, [vp, vp, vp, vp, i64, vp]),
+        "latok_b200_vocab_last_ms": (C.c_int, [vp, P(C.c_float)]),
     }
     for name, (res, args) in proto.items():
         fn = getattr(L, name)

@@ -16,7 +16,7 @@ PKG = Path(__file__).resolve().parent
 ROOT = PKG.parent
 CSRC = PKG / "csrc"
 LIB = PKG / "liblatok_b200.so"
-SOURCES = [CSRC / "latok_kernels.cu", CSRC / "latok_tok5.cu", CSRC / "latok_tokbytes.cu", CSRC / "latok_capi.cu", CSRC / "latok_reader.cpp"]
+SOURCES = [CSRC / "latok_kernels.cu", CSRC / "latok_tok5.cu", CSRC / "latok_tokbytes.cu", CSRC / "latok_vocab.cu", CSRC / "latok_capi.cu", CSRC / "latok_reader.cpp"]
 HEADERS = [CSRC / "latok_internal.h", CSRC / "latok_bits.h", CSRC / "latok_device.cuh", ROOT / "include" / "latok_b200.h"]
 GEN = CSRC / "_gen" / "latok_tables.h"
 RANGES = PKG / "data" / "ucd11_latok_classes.txt"

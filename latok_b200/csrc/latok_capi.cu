@@ -71,6 +71,22 @@ struct PinBuf {
     void release() { if (p) cudaFreeHost(p); p = nullptr; cap = 0; }
 };
 
+// grows b to at least n elements, keeping its first `keep` (written on stream s)
+template <class T>
+int grow_keep(DevBuf<T> &b, size_t n, size_t keep, cudaStream_t s)
+{
+    if (n <= b.cap) return 0;
+    const size_t want = n > 2 * b.cap ? n : 2 * b.cap;
+    T *p = nullptr;
+    CU(cudaMalloc((void **)&p, want * sizeof(T)));
+    if (keep) CU(cudaMemcpyAsync(p, b.p, keep * sizeof(T), cudaMemcpyDeviceToDevice, s));
+    CU(cudaStreamSynchronize(s));
+    if (b.p) cudaFree(b.p);
+    b.p = p;
+    b.cap = want;
+    return 0;
+}
+
 uint32_t row_mask(const int8_t *row, int cols, bool &ok)
 {
     uint32_t m = 0;
@@ -644,6 +660,22 @@ int latok_b200_in_flight(latok_b200_engine *e, int *n)
     return LATOK_B200_OK;
 }
 
+// token byte ranges of batch b into d_out (int64 [T,2], device) on the compute stream, after the batch's kernels
+static int enqueue_token_bytes(latok_b200_engine *e, Batch &b, long long *d_out)
+{
+    if (int r = e->d_blk_local.ensure((size_t)token_bytes_words(b.n_bytes))) return r;
+    if (int r = e->d_group_tot.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
+    if (int r = e->d_group_pref.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
+    cudaStream_t s = e->stream;
+    CU(cudaStreamWaitEvent(s, b.ev_kdone, 0));
+    CU(cudaEventRecord(e->ev_b0, s));
+    CU(launch_token_bytes(b.cur_in, b.n_bytes, b.cur_off, b.d_char_off.p, b.d_tok_off.p, b.n_strings, b.n_tokens, b.d_spans.p,
+                          d_out, e->d_blk_local.p, e->d_group_tot.p, e->d_group_pref.p, e->d_table.p, e->tl, e->n_sm, s));
+    CU(cudaEventRecord(e->ev_b1, s));
+    e->launches += 3;
+    return 0;
+}
+
 int latok_b200_fetch_token_bytes(latok_b200_engine *e, int64_t cap_tokens, int64_t *byte_spans, int on_device)
 {
     FRONT(e, b);
@@ -656,16 +688,8 @@ int latok_b200_fetch_token_bytes(latok_b200_engine *e, int64_t cap_tokens, int64
     if (on_device && ((uintptr_t)byte_spans & 15u) != 0) return fail(LATOK_B200_EINVAL, "a device byte_spans array must be 16-byte aligned");
     long long *d_out = on_device ? (long long *)byte_spans : nullptr;
     if (!on_device) { if (int r = e->d_tok_bytes.ensure(2 * T)) return r; d_out = e->d_tok_bytes.p; }
-    if (int r = e->d_blk_local.ensure((size_t)token_bytes_words(b.n_bytes))) return r;
-    if (int r = e->d_group_tot.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
-    if (int r = e->d_group_pref.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
+    if (int r = enqueue_token_bytes(e, b, d_out)) return r;
     cudaStream_t s = e->stream;
-    CU(cudaStreamWaitEvent(s, b.ev_kdone, 0));
-    CU(cudaEventRecord(e->ev_b0, s));
-    CU(launch_token_bytes(b.cur_in, b.n_bytes, b.cur_off, b.d_char_off.p, b.d_tok_off.p, b.n_strings, b.n_tokens, b.d_spans.p,
-                          d_out, e->d_blk_local.p, e->d_group_tot.p, e->d_group_pref.p, e->d_table.p, e->tl, e->n_sm, s));
-    CU(cudaEventRecord(e->ev_b1, s));
-    e->launches += 3;
     if (!on_device) CU(cudaMemcpyAsync(byte_spans, d_out, T * 2 * sizeof(long long), cudaMemcpyDeviceToHost, s));
     CU(cudaEventRecord(b.ev_kdone, s));          // the set's inputs are in use until here
     CU(cudaStreamSynchronize(s));
@@ -801,6 +825,281 @@ int latok_b200_combine_matrix_rows(latok_b200_engine *e, const int8_t *m, int64_
     e->launches += 1;
     CU(cudaMemcpyAsync(out, e->d_scratch2.p, (size_t)m_cols, cudaMemcpyDeviceToHost, e->stream));
     CU(cudaStreamSynchronize(e->stream));
+    return LATOK_B200_OK;
+}
+
+// ---- token vocabulary (kernels: latok_vocab.cu) ---------------------------------------------------------------------
+struct latok_b200_vocab {
+    int device = 0;
+    unsigned long long hmask = ~0ULL;
+    long long cap = 0;                              // table slots, a power of two; the load limit is cap / 2 keys
+    long long n_keys = 0, key_bytes = 0;
+    DevBuf<VocabSlot> table;
+    DevBuf<unsigned long long> first_occ;           // [cap]
+    DevBuf<uint8_t> arena;                          // key bytes in id order
+    DevBuf<long long> key_off;                      // [n_keys + 1]
+    DevBuf<long long> counts;                       // [n_keys]
+    DevBuf<uint32_t> slot;                          // per token of the largest batch: its slot
+    DevBuf<int32_t> rank;                           // per token: first-occurrence flags, then new ids, then the ids
+    DevBuf<uint8_t> scan_tmp, imp_bytes;
+    DevBuf<longlong2> imp_rng;
+    DevBuf<VocabStatus> st;
+    PinBuf<VocabStatus> h_st;
+    cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
+    float last_ms = 0.f;
+};
+
+static VocabParams vocab_params(latok_b200_vocab *v)
+{
+    VocabParams p;
+    memset(&p, 0, sizeof p);
+    p.table = v->table.p; p.mask = (unsigned long long)v->cap - 1; p.hmask = v->hmask;
+    p.arena = v->arena.p; p.key_off = v->key_off.p; p.n_keys = v->n_keys;
+    p.first_occ = v->first_occ.p; p.slot = v->slot.p; p.rank = v->rank.p;
+    p.counts = reinterpret_cast<unsigned long long *>(v->counts.p); p.st = v->st.p;
+    p.limit = (unsigned long long)(v->cap / 2 > v->n_keys ? v->cap / 2 - v->n_keys : 0);
+    return p;
+}
+
+// an empty table of `cap` slots that holds the committed keys: drops the claims of a batch that did not commit
+static int vocab_rebuild(latok_b200_vocab *v, long long cap, int n_sm, cudaStream_t s)
+{
+    if (cap > (1LL << 31)) return fail(LATOK_B200_ENOMEM, "a vocabulary table holds at most 2^31 slots");
+    if (cap != v->cap) {
+        CU(cudaStreamSynchronize(s));
+        if (int r = v->table.ensure((size_t)cap)) return r;
+        if (int r = v->first_occ.ensure((size_t)cap)) return r;
+        v->cap = cap;
+    }
+    CU(cudaMemsetAsync(v->table.p, 0, (size_t)cap * sizeof(VocabSlot), s));
+    CU(cudaMemsetAsync(v->st.p, 0, sizeof(VocabStatus), s));
+    CU(launch_vocab(VOCAB_REHASH, vocab_params(v), 0, n_sm, s));
+    return 0;
+}
+
+// claims the keys text[rng[k].x, rng[k].y) (k < n) that the vocabulary lacks: *n_new keys of *new_bytes bytes, claimed
+// but not committed.  A batch that passes the load limit grows the table 4x and runs again.
+static int vocab_insert(latok_b200_vocab *v, const uint8_t *text, const longlong2 *rng, long long n, int n_sm, cudaStream_t s,
+                        long long *n_new, long long *new_bytes)
+{
+    if (int r = v->slot.ensure((size_t)n)) return r;
+    if (int r = v->rank.ensure((size_t)n + 1)) return r;
+    for (int attempt = 0; attempt < 24; ++attempt) {
+        VocabParams p = vocab_params(v);
+        p.text = text; p.rng = rng; p.n = n;
+        CU(cudaMemsetAsync(v->first_occ.p, 0xFF, (size_t)v->cap * sizeof(unsigned long long), s));
+        CU(cudaMemsetAsync(v->st.p, 0, sizeof(VocabStatus), s));
+        CU(launch_vocab(VOCAB_INSERT, p, 0, n_sm, s));
+        CU(launch_vocab(VOCAB_FLAG, p, 0, n_sm, s));
+        CU(cudaEventRecord(v->ev[1], s));
+        CU(cudaMemcpyAsync(v->h_st.p, v->st.p, sizeof(VocabStatus), cudaMemcpyDeviceToHost, s));
+        CU(cudaStreamSynchronize(s));
+        const VocabStatus st = *v->h_st.p;
+        if (!st.overflow) { *n_new = (long long)st.n_new; *new_bytes = (long long)st.new_bytes; return 0; }
+        if (int r = vocab_rebuild(v, v->cap * 4, n_sm, s)) return r;
+    }
+    return fail(LATOK_B200_EINTERNAL, "vocabulary insert did not converge");
+}
+
+// gives the claimed keys of vocab_insert the ids n_keys .. n_keys + n_new - 1 in token order and copies them into the arena
+static int vocab_commit(latok_b200_vocab *v, const uint8_t *text, const longlong2 *rng, long long n, long long n_new,
+                        long long new_bytes, int n_sm, cudaStream_t s)
+{
+    if (v->n_keys + n_new > INT32_MAX) {
+        if (int r = vocab_rebuild(v, v->cap, n_sm, s)) return r;
+        CU(cudaStreamSynchronize(s));
+        return fail(LATOK_B200_EINVAL, "a vocabulary holds at most 2^31 - 1 keys");
+    }
+    CU(cudaEventRecord(v->ev[2], s));
+    if (!n_new) return 0;
+    if (int r = grow_keep(v->arena, (size_t)(v->key_bytes + new_bytes), (size_t)v->key_bytes, s)) return r;
+    if (int r = grow_keep(v->key_off, (size_t)(v->n_keys + n_new + 1), (size_t)v->n_keys + 1, s)) return r;
+    if (int r = grow_keep(v->counts, (size_t)(v->n_keys + n_new), (size_t)v->n_keys, s)) return r;
+    CU(cudaMemsetAsync(v->counts.p + v->n_keys, 0, (size_t)n_new * sizeof(long long), s));
+    VocabParams p = vocab_params(v);
+    p.text = text; p.rng = rng; p.n = n;
+    size_t need = 0, need1 = 0;
+    CU(vocab_scan(0, nullptr, &need, p, n_new, v->key_bytes, s));
+    CU(vocab_scan(1, nullptr, &need1, p, n_new, v->key_bytes, s));
+    if (need1 > need) need = need1;
+    if (need > v->scan_tmp.cap) { CU(cudaStreamSynchronize(s)); if (int r = v->scan_tmp.ensure(need)) return r; }
+    CU(vocab_scan(0, v->scan_tmp.p, &need, p, n_new, v->key_bytes, s));
+    CU(launch_vocab(VOCAB_LENS, p, n_new, n_sm, s));
+    CU(vocab_scan(1, v->scan_tmp.p, &need, p, n_new, v->key_bytes, s));
+    CU(launch_vocab(VOCAB_COMMIT, p, n_new, n_sm, s));
+    v->n_keys += n_new;
+    v->key_bytes += new_bytes;
+    return 0;
+}
+
+static float elapsed(cudaEvent_t a, cudaEvent_t b)
+{
+    float ms = 0.f;
+    if (cudaEventElapsedTime(&ms, a, b) != cudaSuccess) { cudaGetLastError(); ms = 0.f; }
+    return ms;
+}
+
+int latok_b200_vocab_create(latok_b200_engine *e, int64_t expected_keys, latok_b200_vocab **out)
+{
+    if (!out) return fail(LATOK_B200_EINVAL, "out is NULL");
+    *out = nullptr;
+    if (!e) return fail(LATOK_B200_EINVAL, "engine is NULL");
+    if (expected_keys < 0 || expected_keys > INT32_MAX) return fail(LATOK_B200_EINVAL, "expected_keys must be in [0, 2^31 - 1]");
+    if (int r = set_device(e)) return r;
+    latok_b200_vocab *v = new (std::nothrow) latok_b200_vocab();
+    if (!v) return fail(LATOK_B200_ENOMEM, "out of host memory");
+    v->device = e->device;
+    // test seam: keep only the low n bits of the hash, so that tests can force collisions and long probe chains
+    if (const char *hb = getenv("LATOK_B200_VOCAB_HASH_BITS")) {
+        const int bits = atoi(hb);
+        if (bits >= 1 && bits < 64) v->hmask = (1ULL << bits) - 1;
+    }
+    long long cap = 64;
+    while (cap < 2 * expected_keys) cap <<= 1;
+    const int rc = [&]() -> int {
+        for (cudaEvent_t &ev : v->ev) CU(cudaEventCreate(&ev));
+        if (int r = v->st.ensure(1)) return r;
+        if (int r = v->h_st.ensure(1)) return r;
+        if (int r = v->key_off.ensure(1, true)) return r;
+        if (int r = v->table.ensure((size_t)cap)) return r;
+        if (int r = v->first_occ.ensure((size_t)cap)) return r;
+        v->cap = cap;
+        CU(cudaMemset(v->table.p, 0, (size_t)cap * sizeof(VocabSlot)));
+        CU(cudaDeviceSynchronize());
+        return 0;
+    }();
+    if (rc) { latok_b200_vocab_destroy(v); return rc; }
+    *out = v;
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_destroy(latok_b200_vocab *v)
+{
+    if (!v) return LATOK_B200_OK;
+    cudaSetDevice(v->device);
+    v->table.release(); v->first_occ.release(); v->arena.release(); v->key_off.release(); v->counts.release();
+    v->slot.release(); v->rank.release(); v->scan_tmp.release(); v->imp_bytes.release(); v->imp_rng.release();
+    v->st.release(); v->h_st.release();
+    for (cudaEvent_t ev : v->ev) if (ev) cudaEventDestroy(ev);
+    delete v;
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_encode(latok_b200_engine *e, latok_b200_vocab *v, int add, int32_t unk_id, int64_t cap_tokens,
+                            int32_t *ids, int on_device)
+{
+    if (!v) return fail(LATOK_B200_EINVAL, "vocabulary is NULL");
+    FRONT(e, b);
+    if (v->device != e->device) return fail(LATOK_B200_EINVAL, "the vocabulary is on device %d, the engine on device %d", v->device, e->device);
+    if (int r = size_batch(e, b)) return r;
+    if (!(b.what & LATOK_B200_SPANS)) return fail(LATOK_B200_ESTATE, "spans were not requested at submit");
+    const long long T = b.n_tokens;
+    if (cap_tokens < T) return fail(LATOK_B200_EINVAL, "cap_tokens = %lld, the batch has %lld tokens", (long long)cap_tokens, T);
+    if (ids && on_device && ((uintptr_t)ids & 3u) != 0) return fail(LATOK_B200_EINVAL, "a device ids array must be 4-byte aligned");
+    v->last_ms = 0.f;
+    if (!T || (!add && !ids)) return LATOK_B200_OK;
+    if (int r = e->d_tok_bytes.ensure(2 * (size_t)T)) return r;
+    if (int r = v->rank.ensure((size_t)T + 1)) return r;
+    cudaStream_t s = e->stream;
+    CU(cudaStreamWaitEvent(s, b.ev_kdone, 0));
+    CU(cudaEventRecord(v->ev[0], s));
+    if (int r = enqueue_token_bytes(e, b, e->d_tok_bytes.p)) return r;
+    const longlong2 *rng = reinterpret_cast<const longlong2 *>(e->d_tok_bytes.p);
+    VocabParams p;
+    if (add) {
+        long long n_new = 0, new_bytes = 0;
+        if (int r = vocab_insert(v, b.cur_in, rng, T, e->n_sm, s, &n_new, &new_bytes)) return r;
+        if (int r = vocab_commit(v, b.cur_in, rng, T, n_new, new_bytes, e->n_sm, s)) return r;
+        p = vocab_params(v);
+        p.ids = ids ? (on_device ? ids : v->rank.p) : nullptr;
+        p.text = b.cur_in; p.rng = rng; p.n = T;
+        CU(launch_vocab(VOCAB_COUNT, p, 0, e->n_sm, s));
+        CU(cudaEventRecord(v->ev[3], s));
+        e->launches += 6;
+    } else {
+        p = vocab_params(v);
+        p.ids = on_device ? ids : v->rank.p;
+        p.unk = unk_id;
+        p.text = b.cur_in; p.rng = rng; p.n = T;
+        CU(launch_vocab(VOCAB_LOOKUP, p, 0, e->n_sm, s));
+        CU(cudaEventRecord(v->ev[1], s));
+        e->launches += 1;
+    }
+    if (ids && !on_device) CU(cudaMemcpyAsync(ids, p.ids, (size_t)T * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CU(cudaEventRecord(b.ev_kdone, s));          // the set's inputs are in use until here
+    CU(cudaStreamSynchronize(s));
+    v->last_ms = elapsed(v->ev[0], v->ev[1]) + (add ? elapsed(v->ev[2], v->ev[3]) : 0.f);
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_size(latok_b200_vocab *v, int64_t *n_keys, int64_t *key_bytes, int64_t *table_slots)
+{
+    if (!v) return fail(LATOK_B200_EINVAL, "vocabulary is NULL");
+    if (n_keys) *n_keys = v->n_keys;
+    if (key_bytes) *key_bytes = v->key_bytes;
+    if (table_slots) *table_slots = v->cap;
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_export(latok_b200_vocab *v, int64_t cap_keys, int64_t cap_bytes, uint8_t *bytes, int64_t *offsets,
+                            int64_t *counts)
+{
+    if (!v) return fail(LATOK_B200_EINVAL, "vocabulary is NULL");
+    if ((offsets || counts) && cap_keys < v->n_keys)
+        return fail(LATOK_B200_EINVAL, "cap_keys = %lld, the vocabulary has %lld keys", (long long)cap_keys, v->n_keys);
+    if (bytes && cap_bytes < v->key_bytes)
+        return fail(LATOK_B200_EINVAL, "cap_bytes = %lld, the keys have %lld bytes", (long long)cap_bytes, v->key_bytes);
+    CU(cudaSetDevice(v->device));
+    if (bytes && v->key_bytes) CU(cudaMemcpy(bytes, v->arena.p, (size_t)v->key_bytes, cudaMemcpyDeviceToHost));
+    if (offsets) CU(cudaMemcpy(offsets, v->key_off.p, ((size_t)v->n_keys + 1) * sizeof(long long), cudaMemcpyDeviceToHost));
+    if (counts && v->n_keys) CU(cudaMemcpy(counts, v->counts.p, (size_t)v->n_keys * sizeof(long long), cudaMemcpyDeviceToHost));
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_import(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *bytes, const int64_t *offsets,
+                            int64_t n_keys, const int64_t *counts)
+{
+    if (!e || !v) return fail(LATOK_B200_EINVAL, "engine or vocabulary is NULL");
+    if (v->device != e->device) return fail(LATOK_B200_EINVAL, "the vocabulary is on device %d, the engine on device %d", v->device, e->device);
+    if (n_keys < 0) return fail(LATOK_B200_EINVAL, "n_keys must be >= 0");
+    if (n_keys == 0) return LATOK_B200_OK;
+    if (!offsets || !bytes) return fail(LATOK_B200_EINVAL, "must specify the key bytes and offsets (n_keys + 1 entries)");
+    if (offsets[0] != 0) return fail(LATOK_B200_EINVAL, "offsets[0] must be 0");
+    for (int64_t i = 0; i < n_keys; ++i)
+        if (offsets[i + 1] <= offsets[i]) return fail(LATOK_B200_EINVAL, "key %lld is empty (offsets must increase)", (long long)i);
+    if (v->n_keys + n_keys > INT32_MAX) return fail(LATOK_B200_EINVAL, "a vocabulary holds at most 2^31 - 1 keys");
+    if (int r = set_device(e)) return r;
+    cudaStream_t s = e->stream;
+    const long long nb = offsets[n_keys];
+    std::vector<longlong2> rng((size_t)n_keys);
+    for (int64_t i = 0; i < n_keys; ++i) rng[(size_t)i] = make_longlong2(offsets[i], offsets[i + 1]);
+    CU(cudaStreamSynchronize(s));
+    if (int r = v->imp_bytes.ensure((size_t)nb)) return r;
+    if (int r = v->imp_rng.ensure((size_t)n_keys)) return r;
+    CU(cudaMemcpyAsync(v->imp_bytes.p, bytes, (size_t)nb, cudaMemcpyHostToDevice, s));
+    CU(cudaMemcpyAsync(v->imp_rng.p, rng.data(), (size_t)n_keys * sizeof(longlong2), cudaMemcpyHostToDevice, s));
+    CU(cudaEventRecord(v->ev[0], s));
+    long long n_new = 0, new_bytes = 0;
+    if (int r = vocab_insert(v, v->imp_bytes.p, v->imp_rng.p, n_keys, e->n_sm, s, &n_new, &new_bytes)) return r;
+    if (n_new != n_keys) {
+        if (int r = vocab_rebuild(v, v->cap, e->n_sm, s)) return r;
+        CU(cudaStreamSynchronize(s));
+        return fail(LATOK_B200_EINVAL, "duplicate keys: %lld of the %lld keys are new to the vocabulary", n_new, (long long)n_keys);
+    }
+    const long long first = v->n_keys;
+    if (int r = vocab_commit(v, v->imp_bytes.p, v->imp_rng.p, n_keys, n_new, new_bytes, e->n_sm, s)) return r;
+    if (counts) CU(cudaMemcpyAsync(v->counts.p + first, counts, (size_t)n_keys * sizeof(long long), cudaMemcpyHostToDevice, s));
+    CU(cudaEventRecord(v->ev[3], s));
+    CU(cudaStreamSynchronize(s));
+    e->launches += 5;
+    v->last_ms = elapsed(v->ev[0], v->ev[1]) + elapsed(v->ev[2], v->ev[3]);
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_last_ms(latok_b200_vocab *v, float *ms)
+{
+    if (!v || !ms) return fail(LATOK_B200_EINVAL, "vocabulary or ms is NULL");
+    *ms = v->last_ms;
     return LATOK_B200_OK;
 }
 

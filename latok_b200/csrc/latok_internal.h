@@ -158,4 +158,38 @@ cudaError_t launch_token_bytes(const uint8_t *in, long long n_bytes, const long 
                                long long *out, unsigned *word_local, unsigned *group_tot, unsigned long long *group_pref,
                                const uint8_t *table_blob, const TableLayout &tl, int n_sm, cudaStream_t s);
 
+// token vocabulary (latok_vocab.cu)
+constexpr unsigned long long VOCAB_COMMITTED = 1ULL << 63;
+struct __align__(16) VocabSlot { unsigned long long hash, ref; };    // hash 0: empty
+struct VocabStatus {
+    unsigned long long claims;     // slots claimed by the insert launch
+    unsigned long long n_new;      // keys new in the batch, and their bytes (flag kernel)
+    unsigned long long new_bytes;
+    unsigned overflow;             // load limit passed or a probe sequence without a slot: the batch is run again
+    unsigned pad;
+};
+struct VocabParams {
+    VocabSlot *table;
+    unsigned long long mask;       // capacity - 1 (capacity a power of two)
+    unsigned long long hmask;      // hash bits kept (LATOK_B200_VOCAB_HASH_BITS, a test seam)
+    const uint8_t *text;           // the launch's keys: key k = text[rng[k].x, rng[k].y)
+    const longlong2 *rng;
+    long long n;
+    uint8_t *arena;                // committed key id = arena[key_off[id], key_off[id + 1])
+    long long *key_off;
+    long long n_keys;
+    unsigned long long *first_occ; // [capacity]
+    uint32_t *slot;                // [n]
+    int32_t *rank;                 // [n + 1]
+    int32_t *ids;                  // [n] or NULL
+    int32_t unk;
+    unsigned long long *counts;    // [n_keys] or NULL
+    VocabStatus *st;
+    unsigned long long limit;      // new claims the load limit allows in this launch
+};
+enum VocabPhase { VOCAB_INSERT, VOCAB_LOOKUP, VOCAB_FLAG, VOCAB_LENS, VOCAB_COMMIT, VOCAB_COUNT, VOCAB_REHASH };
+cudaError_t launch_vocab(VocabPhase phase, const VocabParams &p, long long n_new, int n_sm, cudaStream_t s);
+cudaError_t vocab_scan(int which, void *tmp, size_t *tmp_bytes, const VocabParams &p, long long n_new, long long key_bytes,
+                       cudaStream_t s);
+
 }  // namespace latok

@@ -3,11 +3,13 @@
 scripts/timing/time_tokenizer.py:25-123 (same input format, same flags, same --outfile TSV), SURVEY 8 f3.
 
     python tools/time_tokenizer.py <csv or csv.gz: one record per row, JSON-encoded text in column 1>
-        [--split | --matrix | --features] [--outfile tokens.tsv] [--batch 200000] [--device 0]
+        [--split | --matrix | --features] [--outfile tokens.tsv] [--counts counts.tsv] [--batch 200000] [--device 0]
 
 The reference calls the tokenizer once per line; here lines are packed into batches (flat UTF-8 + offsets) by a
 reader thread while the GPU works on the previous batch, and `--outfile` is written from the token byte ranges
-(latok_b200_fetch_token_bytes) with NumPy gathers -- no Python string is created per token.
+(latok_b200_fetch_token_bytes) with NumPy gathers -- no Python string is created per token.  `--counts` counts the
+tokens of all rows in one vocabulary on the GPU (latok_b200.vocab) and writes `token<TAB>count` lines, most common first
+(equal counts in order of first occurrence).
 """
 from __future__ import annotations
 
@@ -77,6 +79,7 @@ def main():
     ap.add_argument("--features", action="store_true", help="featurize the tokens")
     ap.add_argument("--mincount", type=int, default=100000, help="rows between progress lines")
     ap.add_argument("--outfile", help="write the tokens of every row, tab-separated, one row per line")
+    ap.add_argument("--counts", help="write `token\tcount` per distinct token of the file, most common first")
     ap.add_argument("--batch", type=int, default=200_000, help="rows per GPU batch")
     ap.add_argument("--batch-bytes", type=int, default=64 << 20, help="native reader: UTF-8 bytes per GPU batch at most")
     ap.add_argument("--device", type=int, default=0)
@@ -88,6 +91,8 @@ def main():
     from latok_b200.engine import Engine, FEATS, MATRIX, SPANS, SPLITS
     split, matrix = (False, False) if args.outfile else (args.split, args.matrix)
     what = SPLITS if split else MATRIX if matrix else (SPANS | FEATS) if args.features else SPANS
+    if args.counts:
+        what |= SPANS
 
     q: "queue.Queue" = queue.Queue(maxsize=2)
     done = threading.Event()
@@ -117,6 +122,10 @@ def main():
     t_start = time.perf_counter()
     print(f"{datetime.now()}: Beginning tokenization...")
     with Engine(args.device) as e:
+        vocab = None
+        if args.counts:
+            from latok_b200.vocab import Vocab
+            vocab = Vocab(e)
         while True:
             item = q.get()
             if item is None:
@@ -128,6 +137,8 @@ def main():
             e.submit(buf, off, what)
             r = e.fetch()
             bs = e.token_bytes() if out is not None else None
+            if vocab is not None:
+                vocab.encode_oldest(add=True, want_ids=False)
             gpu_s += time.perf_counter() - t0
             if out is not None:
                 t0 = time.perf_counter()
@@ -140,6 +151,11 @@ def main():
                 dt = time.perf_counter() - t_start
                 print(f"{datetime.now()}: {rows} lines, {rows / dt:.0f} lines/s, {n_bytes / dt / 1e6:.1f} MB/s", file=sys.stderr)
                 next_report += args.mincount
+        if vocab is not None:
+            with open(args.counts, "wb") as f:
+                f.write("".join(f"{t}\t{c}\n" for t, c in vocab.most_common()).encode("utf-8", "surrogatepass"))
+            n_distinct = len(vocab)
+            vocab.close()
     done.set()
     if out is not None:
         out.close()
@@ -148,7 +164,7 @@ def main():
     print(json.dumps({"lines": rows, "bytes": n_bytes, "tokens": n_tokens, "seconds": dt, "lines_per_s": rows / dt,
                       "MB_per_s": n_bytes / dt / 1e6, "gpu_call_seconds": gpu_s, "write_seconds": write_s,
                       "mode": "split" if split else "matrix" if matrix else "features" if args.features else "tokenize",
-                      "reader": args.reader}))
+                      "reader": args.reader, "distinct_tokens": None if vocab is None else n_distinct}))
     return 0
 
 
