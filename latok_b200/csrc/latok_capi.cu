@@ -3,7 +3,7 @@
 // Owns device / pinned memory, streams and the packed Unicode class table, validates arguments
 // (the reference reports errors with PyErr_SetString(PyExc_ValueError, ...), latok.c:40-50,
 // 151-171, 292-312; here they become status codes + latok_b200_last_error()) and launches the
-// kernels of latok_kernels.cu.  There is no CPU implementation of the path in this library.
+// kernels.  There is no CPU implementation of the path in this library.
 #include "../../include/latok_b200.h"
 #include "latok_internal.h"
 #include "_gen/latok_tables.h"
@@ -178,10 +178,10 @@ struct latok_b200_engine {
     DevBuf<IncRec> inc;
     DevBuf<OpenSums> osum;
     DevBuf<uint32_t> d_planes;
-    DevBuf<unsigned long long> span_scratch;
     DevBuf<long long> d_tok_bytes;                  // token byte ranges (latok_b200_fetch_token_bytes)
-    DevBuf<unsigned> d_blk_local, d_group_tot;
+    DevBuf<unsigned> d_blk_local, d_group_tot;      // characters in front of every 32-byte word (launch_char_prefix)
     DevBuf<unsigned long long> d_group_pref;
+    DevBuf<uint32_t> d_starts;                      // string-start bitmap of the parse matrix
     float last_token_bytes_ms = 0.f;
     unsigned epoch = 0;
     long long launches = 0;
@@ -228,7 +228,6 @@ static int build_table(latok_b200_engine *e)
     TableLayout &tl = e->tl;
     int o = 0;
     auto take = [&](int bytes) { int r = o; o += (bytes + 15) & ~15; return r; };
-    tl.lut3 = take(3 * LUT_ENTRIES * 4);
     tl.lutv = take(256 * 4);
     tl.ascii_feat = take(128 * 2);
     tl.class_feat = take(16 * 2);
@@ -244,18 +243,7 @@ static int build_table(latok_b200_engine *e)
     tl.high_last = LATOK_HIGH_RUNS[0][1];
     tl.high_feat = LATOK_HIGH_RUNS[0][2];
     std::vector<uint8_t> blob((size_t)tl.total, 0);
-    tl.high_class = 0;
-    for (uint32_t c = 0; c < 16; ++c) if (LATOK_CLASS_FEAT[c] == tl.high_feat) tl.high_class = c;
     {
-        uint32_t *lut3 = reinterpret_cast<uint32_t *>(blob.data() + tl.lut3);
-        for (int e = 0; e < LUT_ENTRIES; ++e) {
-            const uint32_t f = e < 128 ? LATOK_ASCII_FEAT[e] : (e < 256 ? 0u : LATOK_CLASS_FEAT[e - 256]);
-            for (int k = 0; k < 3; ++k) {
-                uint32_t w = 0;
-                for (int b = 0; b < 4; ++b) w |= ((f >> (4 * k + b)) & 1u) << (8 * b);
-                lut3[k * LUT_ENTRIES + e] = w;
-            }
-        }
         uint32_t *lutv = reinterpret_cast<uint32_t *>(blob.data() + tl.lutv);
         for (int i = 0; i < 256; ++i) {
             uint32_t w = 0;
@@ -328,8 +316,8 @@ int latok_b200_destroy(latok_b200_engine *e)
     cudaSetDevice(e->device);
     for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out}) if (st) cudaStreamSynchronize(st);
     e->d_table.release(); e->d_scratch.release(); e->d_scratch2.release(); e->d_scratch3.release();
-    e->agg.release(); e->inc.release(); e->osum.release(); e->d_planes.release(); e->span_scratch.release();
-    e->d_tok_bytes.release(); e->d_blk_local.release(); e->d_group_tot.release(); e->d_group_pref.release();
+    e->agg.release(); e->inc.release(); e->osum.release(); e->d_planes.release();
+    e->d_tok_bytes.release(); e->d_blk_local.release(); e->d_group_tot.release(); e->d_group_pref.release(); e->d_starts.release();
     for (Batch &b : e->set) b.release();
     for (cudaEvent_t ev : {e->ev_t0, e->ev_t1, e->ev_b0, e->ev_b1}) if (ev) cudaEventDestroy(ev);
     for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out}) if (st) cudaStreamDestroy(st);
@@ -386,31 +374,40 @@ __global__ void narrow_spans_kernel(const int2 *spans, uint32_t *out, Result *re
     if (over) atomicOr(&res->error, 16u);
 }
 
+// characters in front of every 32-byte word of batch b (launch_char_prefix) on the compute stream
+static int enqueue_char_prefix(latok_b200_engine *e, Batch &b)
+{
+    if (int r = e->d_blk_local.ensure((size_t)char_prefix_words(b.n_bytes))) return r;
+    if (int r = e->d_group_tot.ensure((size_t)char_prefix_groups(b.n_bytes))) return r;
+    if (int r = e->d_group_pref.ensure((size_t)char_prefix_groups(b.n_bytes))) return r;
+    CU(launch_char_prefix(b.cur_in, b.n_bytes, e->d_blk_local.p, e->d_group_tot.p, e->d_group_pref.p, e->stream));
+    e->launches += 2;
+    return 0;
+}
+
 static int run_device(latok_b200_engine *e, Batch &b)
 {
-    // the matrix mode runs the v4 kernel (one CTA per 7 936-byte tile); everything else (split mask, spans, token
-    // features) runs v5 (one warp per range, a tile = the ranges of one CTA) in one of its two geometries: short strings
-    // (3 KB ranges, 11 compute warps per CTA) or long strings (4 KB ranges, 9 warps: fewer range boundaries inside
-    // space-free runs), by the average string length of the batch; token features: always the long one
-    // (LATOK_B200_GEOMETRY=short|long overrides)
-    const bool words = (b.what & LATOK_B200_MATRIX) != 0, feats = (b.what & LATOK_B200_FEATS) != 0;
-    const bool use5 = !words && !getenv("LATOK_B200_FORCE_V4");
+    // The tokenize kernel (one warp per range, a tile = the ranges of one CTA) runs in one of its two geometries: short
+    // strings (3 KB ranges, 11 compute warps per CTA) or long strings (4 KB ranges, 9 warps: fewer range boundaries
+    // inside space-free runs), by the average string length of the batch; token features: always the long one
+    // (LATOK_B200_GEOMETRY=short|long overrides).  It also gives the character counts and the offsets check of a
+    // matrix-only batch.  The parse matrix follows it on the same stream.
+    const bool feats = (b.what & LATOK_B200_FEATS) != 0;
     bool shortg = b.n_bytes < 4096LL * (b.n_strings > 0 ? b.n_strings : 1);
     if (feats) shortg = false;      // the token-feature instantiation lives on registers (25 planes per lane): 96 beat 24 warps per SM
     if (const char *g = getenv("LATOK_B200_GEOMETRY")) shortg = g[0] == 's';
     const int range5 = shortg ? tokenize5_range_bytes_short() : tokenize5_range_bytes();
     const int nw5 = shortg ? tokenize5_ranges_per_tile_short() : tokenize5_ranges_per_tile();
-    const int unit = use5 ? range5 : TILE;
-    const long long nunits = b.n_bytes / unit + 1;
-    const long long ntiles = use5 ? (nunits + nw5 - 1) / nw5 : nunits;
+    const long long nunits = b.n_bytes / range5 + 1;
+    const long long ntiles = (nunits + nw5 - 1) / nw5;
     const size_t plane_words = shortg ? tokenize5_plane_words_short(nunits) : tokenize5_plane_words(nunits);
     if (int r = b.d_first.ensure((size_t)nunits + 1)) return r;
     // the status word of every aggregate record carries the launch epoch, so records are zeroed only when (re)allocated
     // (agg / inc / osum / planes are shared by the two sets: tokenize kernels run one after the other on one stream)
     if ((size_t)ntiles > e->agg.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->agg.ensure((size_t)ntiles, true)) return r; }
     if ((size_t)ntiles > e->inc.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->inc.ensure((size_t)ntiles)) return r; }
-    if (feats && (size_t)(use5 ? nunits : ntiles) > e->osum.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->osum.ensure((size_t)(use5 ? nunits : ntiles), true)) return r; }
-    if (feats && use5 && plane_words > e->d_planes.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->d_planes.ensure(plane_words)) return r; }
+    if (feats && (size_t)nunits > e->osum.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->osum.ensure((size_t)nunits, true)) return r; }
+    if (feats && plane_words > e->d_planes.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->d_planes.ensure(plane_words)) return r; }
     if (int r = b.d_splits.ensure((size_t)b.n_bytes + 64)) return r;
     if (int r = b.d_char_off.ensure((size_t)b.n_strings + 1)) return r;
     if (int r = b.d_tok_off.ensure((size_t)b.n_strings + 1)) return r;
@@ -429,33 +426,37 @@ static int run_device(latok_b200_engine *e, Batch &b)
     p.in = b.cur_in; p.n_bytes = b.n_bytes; p.offsets = b.cur_off; p.n_strings = b.n_strings;
     p.tile_first_str = b.d_first.p; p.ntiles = ntiles; p.nranges = nunits;
     p.splits = b.d_splits.p; p.char_off = b.d_char_off.p; p.spans = b.d_spans.p; p.tok_off = b.d_tok_off.p;
-    p.feats = b.d_feats.p; p.matrix = b.d_matrix.p;
+    p.feats = b.d_feats.p;
     p.cap_tokens = (long long)(b.d_spans.cap / 2);
-    p.what = b.what & 15u;
+    p.what = b.what & 7u;
     p.agg = e->agg.p; p.inc = e->inc.p; p.osum = e->osum.p; p.planes = e->d_planes.p; p.epoch = e->epoch;
     p.ticket = &b.d_result.p->ticket; p.ticket_base = 0;
     p.result = b.d_result.p;
     p.table_blob = e->d_table.p; p.tl = e->tl; p.rules = e->rules;
-    int grid = e->n_sm * (!use5 ? tokenize_ctas_per_sm(e->tl, e->rules.is_default != 0, words, feats)
-                          : shortg ? tokenize5_ctas_per_sm_short(e->tl, e->rules.is_default != 0, feats)
-                                   : tokenize5_ctas_per_sm(e->tl, e->rules.is_default != 0, feats));
+    int grid = e->n_sm * (shortg ? tokenize5_ctas_per_sm_short(e->tl, e->rules.is_default != 0, feats)
+                                 : tokenize5_ctas_per_sm(e->tl, e->rules.is_default != 0, feats));
     if ((long long)grid > ntiles) grid = (int)ntiles;
-    if (!use5) { if (int r = e->span_scratch.ensure((size_t)grid * 2 * SPAN_SCRATCH)) return r; }
-    p.span_scratch = e->span_scratch.p;
 
     // The string index of this batch is built on the aux stream, so that with back-to-back submits it overlaps the
     // tokenize kernel of the previous batch (the two sets alternate).
     if (b.inputs_on_stream) CU(cudaStreamWaitEvent(e->aux, b.ev_h2d, 0));    // host submit: the offsets arrive on the copy-in stream
     CU(cudaStreamWaitEvent(e->aux, b.ev_kdone, 0));            // this set's previous batch has been tokenized
     CU(cudaMemsetAsync(b.d_result.p, 0, sizeof(Result), e->aux));
-    CU(launch_tile_index(b.cur_off, b.n_strings, b.n_bytes, b.d_first.p, nunits, unit, b.d_result.p, e->aux));
+    CU(launch_tile_index(b.cur_off, b.n_strings, b.n_bytes, b.d_first.p, nunits, range5, b.d_result.p, e->aux));
     CU(cudaEventRecord(b.ev_index, e->aux));
     if (b.inputs_on_stream) CU(cudaStreamWaitEvent(e->stream, b.ev_h2d, 0));
     CU(cudaStreamWaitEvent(e->stream, b.ev_index, 0));
     CU(cudaEventRecord(b.ev_k0, e->stream));
-    CU(!use5 ? launch_tokenize(p, grid, e->stream) : shortg ? launch_tokenize5_short(p, grid, e->stream) : launch_tokenize5(p, grid, e->stream));
+    CU(shortg ? launch_tokenize5_short(p, grid, e->stream) : launch_tokenize5(p, grid, e->stream));
     CU(cudaEventRecord(b.ev_k1, e->stream));
     e->launches += 2;
+    if (b.what & LATOK_B200_MATRIX) {
+        if (int r = enqueue_char_prefix(e, b)) return r;
+        if (int r = e->d_starts.ensure((size_t)char_prefix_words(b.n_bytes))) return r;
+        CU(launch_parse_matrix(b.cur_in, b.n_bytes, b.cur_off, b.n_strings, e->d_starts.p, e->d_blk_local.p, e->d_group_pref.p,
+                               e->d_table.p, e->tl, b.d_matrix.p, b.d_result.p, e->n_sm, e->stream));
+        e->launches += 2;
+    }
     if (b.what & LATOK_B200_SPANS16) {
         narrow_spans_kernel<<<e->n_sm * 8, 256, 0, e->stream>>>(reinterpret_cast<const int2 *>(b.d_spans.p), b.d_spans16.p, b.d_result.p, p.cap_tokens);
         CU(cudaGetLastError());
@@ -663,16 +664,14 @@ int latok_b200_in_flight(latok_b200_engine *e, int *n)
 // token byte ranges of batch b into d_out (int64 [T,2], device) on the compute stream, after the batch's kernels
 static int enqueue_token_bytes(latok_b200_engine *e, Batch &b, long long *d_out)
 {
-    if (int r = e->d_blk_local.ensure((size_t)token_bytes_words(b.n_bytes))) return r;
-    if (int r = e->d_group_tot.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
-    if (int r = e->d_group_pref.ensure((size_t)token_bytes_groups(b.n_bytes))) return r;
     cudaStream_t s = e->stream;
     CU(cudaStreamWaitEvent(s, b.ev_kdone, 0));
     CU(cudaEventRecord(e->ev_b0, s));
+    if (int r = enqueue_char_prefix(e, b)) return r;
     CU(launch_token_bytes(b.cur_in, b.n_bytes, b.cur_off, b.d_char_off.p, b.d_tok_off.p, b.n_strings, b.n_tokens, b.d_spans.p,
-                          d_out, e->d_blk_local.p, e->d_group_tot.p, e->d_group_pref.p, e->d_table.p, e->tl, e->n_sm, s));
+                          d_out, e->d_blk_local.p, e->d_group_pref.p, e->d_table.p, e->tl, e->n_sm, s));
     CU(cudaEventRecord(e->ev_b1, s));
-    e->launches += 3;
+    e->launches += 1;
     return 0;
 }
 

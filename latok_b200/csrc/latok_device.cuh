@@ -1,16 +1,12 @@
-// latok_device.cuh -- device helpers shared by the tokenize kernels (latok_kernels.cu: v4, token-feature / matrix
-// modes; latok_tok5.cu: v5, split mask + spans): PTX wrappers, Unicode class look-up, the scalar rule evaluation
-// used on rare paths, the look-ahead walk and the decoupled look-back.
+// latok_device.cuh -- device helpers shared by the kernels (latok_tok5.cu: tokenize; latok_kernels.cu: parse matrix;
+// latok_tokbytes.cu: token byte ranges): PTX wrappers, Unicode class look-up, the context features, the scalar rule
+// evaluation used on rare paths, the look-ahead walk and the decoupled look-back.
 #pragma once
 #include "latok_internal.h"
 #include "latok_bits.h"
 
 namespace latok {
 
-// ---- word layout: bits 0..24 = the 25 feature columns (offsets.py:24-48), then flags ------------
-constexpr uint32_t FIRSTBIT = 1u << 25;   // character starts a string
-constexpr uint32_t LASTBIT = 1u << 26;    // character ends a string
-constexpr uint32_t FEATMASK = (1u << NFEAT) - 1;
 constexpr int NEG = -(1 << 28);           // "-infinity" of the (max,+) backlog functions
 constexpr unsigned SPIN_LIMIT = 1u << 23; // watchdog for look-back spins
 
@@ -22,7 +18,6 @@ __device__ __forceinline__ uint32_t range_mask(int base, int lo, int hi)
 {
     return mask_lt(hi - base) & ~mask_lt(lo - base);
 }
-__device__ __forceinline__ int widx(int c) { return 1 + c + ((c + 32) >> 5); }  // bank-skewed slot of character c >= -1
 
 struct Fn { int u, v; };  // x -> max(x + u, v)
 __device__ __forceinline__ Fn fn_id() { return Fn{0, NEG}; }
@@ -31,12 +26,6 @@ __device__ __forceinline__ Fn fn_compose(Fn f, Fn g)  // g after f
     return Fn{max(f.u + g.u, NEG), max(max(f.v + g.u, g.v), NEG)};
 }
 __device__ __forceinline__ int fn_apply(Fn f, int x) { return max(x + f.u, f.v); }
-
-#ifdef LATOK_PROFILE
-#define PROF(i) do { if (threadIdx.x == 32) { long long _t = clock64(); atomicAdd(&p.result->prof[i], (unsigned long long)(_t - _prof_t)); _prof_t = _t; } } while (0)
-#else
-#define PROF(i) do { } while (0)
-#endif
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 
@@ -56,10 +45,6 @@ __device__ __forceinline__ bool mbar_try_wait(void *bar, uint32_t phase)
                  "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
                  "selp.u32 %0, 1, 0, P1;\n\t}" : "=r"(ok) : "r"(smem_u32(bar)), "r"(phase) : "memory");
     return ok != 0u;
-}
-__device__ __forceinline__ void mbar_wait(void *bar, uint32_t phase)
-{
-    while (!mbar_try_wait(bar, phase)) { }
 }
 // TMA 1-D bulk copy global -> shared, completion signalled on an mbarrier (SASS: UBLKCP)
 __device__ __forceinline__ void tma_load_1d(void *dst, const void *src, uint32_t bytes, void *bar)
@@ -422,27 +407,9 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
 __device__ __forceinline__ void nb_sync(int id, int cnt) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(cnt) : "memory"); }
 __device__ __forceinline__ void nb_arrive(int id, int cnt) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(cnt) : "memory"); }
 
-// LUT entry (256 + class) of the multi-byte character whose lead byte is p[0] >= 0xC0
-__device__ __forceinline__ uint32_t mb_entry(const uint8_t *p, const Tables &t, uint32_t high_class)
-{
-    const uint32_t b0 = p[0];
-    if (b0 >= 0xF8u) return 256u;  // invalid lead: class 0 (no features)
-    uint32_t cp;
-    if (b0 < 0xE0u) cp = ((b0 & 0x1Fu) << 6) | (p[1] & 0x3Fu);
-    else if (b0 < 0xF0u) cp = ((b0 & 0x0Fu) << 12) | ((p[1] & 0x3Fu) << 6) | (p[2] & 0x3Fu);
-    else cp = ((b0 & 0x07u) << 18) | ((p[1] & 0x3Fu) << 12) | ((p[2] & 0x3Fu) << 6) | (p[3] & 0x3Fu);
-    if (cp < 0x80u) return cp;     // over-long form of an ASCII character
-    if (cp < t.low_limit) {
-        const uint32_t blk = t.stage1[cp >> 7];
-        const uint32_t b = t.stage2[blk * 64u + ((cp & 127u) >> 1)];
-        return 256u + ((cp & 1u) ? (b >> 4) : (b & 15u));
-    }
-    return (cp >= t.high_first && cp <= t.high_last) ? 256u + high_class : 256u;
-}
-
 // Feature word of the multi-byte character whose four bytes (lead byte >= 0xC0 in the low byte, then up to three
 // continuation bytes; whatever follows a shorter character is ignored) are `v` -- the same decode and look-up as
-// mb_entry + the feature tables, without the length branches, so that lanes holding 2-, 3- and 4-byte characters
+// classify_at, without the length branches, so that lanes holding 2-, 3- and 4-byte characters
 // stay converged and two characters can be in flight at once.
 __device__ __forceinline__ uint32_t mb_features(uint32_t v, const Tables &t)
 {

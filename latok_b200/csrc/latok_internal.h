@@ -1,29 +1,11 @@
-// Internal structures shared by the kernels (latok_kernels.cu) and the C-ABI host layer (latok_capi.cu).
+// Internal structures shared by the kernels (latok_tok5.cu, latok_kernels.cu, latok_tokbytes.cu, latok_vocab.cu) and
+// the C-ABI host layer (latok_capi.cu).
 #pragma once
 #include "_gen/latok_table_types.h"   // latok_stage1_t (8 bits for UCD 11, 16 when a newer UCD needs more than 256 blocks)
 #include <cuda_runtime.h>
 #include <stdint.h>
 
 namespace latok {
-
-// ---- tiling geometry ------------------------------------------------------------------------
-// One CTA processes one "window" of WINB bytes: a left halo (context for the first owned
-// character), TILE owned bytes, and a right halo used for NEXT/AFTER_NEXT context and to close
-// the whitespace chunk that is still open at the end of the owned range.  Thread t handles window
-// bytes [32t, 32t+32): thread 0 is the left halo, threads 1..END_OWNED_THREAD-1 own their bytes,
-// the remaining threads are the right halo.
-constexpr int NT = 256;                 // threads per CTA
-constexpr int NWARP = NT / 32;
-constexpr int LHALO = 32;               // thread 0
-constexpr int WINB = NT * 32;           // 8192
-constexpr int RHALO = 224;              // 7 threads
-constexpr int TILE = WINB - LHALO - RHALO;  // 7936 = 62 * 128 B
-constexpr int TRUST_MARGIN = 12;        // chars starting in the last 12 window bytes lack full forward context
-constexpr int FIRST_OWNED_THREAD = LHALO / 32;
-constexpr int END_OWNED_THREAD = (LHALO + TILE) / 32;
-constexpr int LUT_ENTRIES = 272;        // 256 byte values (>= 0x80: no features) + 16 non-ASCII classes
-constexpr int SPAN_STAGE = 1536;        // tokens staged in shared memory per tile before the coalesced write
-constexpr int SPAN_SCRATCH = WINB + 64; // per CTA and slot: global stage for tiles with more tokens than that
 
 // v5 kernel (latok_tok5.cu): one warp analyses a "range" (V5_RS steps of 1 KB, the last V5_HALO bytes shared with the
 // next range), a tile is the V5_NW ranges of one CTA
@@ -47,7 +29,6 @@ constexpr int MAX_RULE_ROWS = 15;
 // packed Unicode class table blob (built by latok_capi.cu from _gen/latok_tables.h)
 struct TableLayout {
     // byte offsets inside the blob; every section is 16-byte aligned
-    int lut3;         // u32[3][LUT_ENTRIES]: word k, byte b = feature 4k+b of the entry (bit 0)
     int lutv;         // u32[256]: 4 split-mask bytes for (value bit-plane 0 nibble | bit-plane 1 nibble << 4)
     int ascii_feat;   // u16[128]
     int class_feat;   // u16[16]
@@ -56,7 +37,7 @@ struct TableLayout {
     int total;        // multiple of 16
     int stage1_len, stage2_len;
     uint32_t low_limit;
-    uint32_t high_first, high_last, high_feat, high_class;  // the single non-empty run above low_limit
+    uint32_t high_first, high_last, high_feat;  // the single non-empty run above low_limit
 };
 
 struct RuleSet {
@@ -111,14 +92,12 @@ struct Params {
     int32_t *spans;
     long long *tok_off;
     int8_t *feats;
-    int8_t *matrix;
     long long cap_tokens;
     uint32_t what;
     AggRec *agg;
     IncRec *inc;
     OpenSums *osum;
     uint32_t *planes;     // v5 token-feature mode: the 25 feature planes of every lane-word, [range][step][25][32 lanes]
-    void *span_scratch;   // int2 [grid][2][SPAN_SCRATCH]
     unsigned epoch;
     unsigned long long *ticket;
     unsigned long long ticket_base;
@@ -128,8 +107,6 @@ struct Params {
     RuleSet rules;
 };
 
-size_t tokenize_smem_bytes(const TableLayout &tl, bool want_words, bool want_feats);
-int tokenize_ctas_per_sm(const TableLayout &tl, bool is_default, bool want_words, bool want_feats);
 // the v5 kernel exists in two geometries (latok_tok5.cu is compiled twice): long strings / short strings (_short)
 int tokenize5_range_bytes();
 int tokenize5_ranges_per_tile();
@@ -143,20 +120,29 @@ size_t tokenize5_plane_words_short(long long nranges);
 cudaError_t launch_tokenize5_short(const Params &p, int grid, cudaStream_t s);
 cudaError_t launch_tile_index(const long long *offsets, long long n_strings, long long n_bytes,
                               long long *tile_first_str, long long ntiles, int tile_bytes, Result *result, cudaStream_t s);
-cudaError_t launch_tokenize(const Params &p, int grid, cudaStream_t s);
 cudaError_t launch_block_mask(const int8_t *a1, long long s1, const int8_t *a2, long long s2, long long n,
                               int8_t *out, unsigned char *scratch, cudaStream_t s);
 cudaError_t launch_combine_rows(const int8_t *m, long long m_rows, long long m_cols, long long stride_r,
                                 long long stride_c, const int8_t *idx, int idx_rows, int idx_cols,
                                 int8_t *out, cudaStream_t s);
 
-// token spans as trimmed byte ranges of the flat buffer (latok_tokbytes.cu)
-long long token_bytes_words(long long n_bytes);
-long long token_bytes_groups(long long n_bytes);
+// characters in front of every 32-byte word of the text: group_pref[w / TB_GROUP] + word_local[w] (latok_tokbytes.cu)
+constexpr int TB_WORD = 32;              // bytes per counted word (one 32-bit lead mask)
+constexpr int TB_GROUP = 4096;           // words per group (128 KB of text)
+long long char_prefix_words(long long n_bytes);
+long long char_prefix_groups(long long n_bytes);
+cudaError_t launch_char_prefix(const uint8_t *in, long long n_bytes, unsigned *word_local, unsigned *group_tot,
+                               unsigned long long *group_pref, cudaStream_t s);
+// token spans as trimmed byte ranges of the flat buffer (latok_tokbytes.cu), after launch_char_prefix
 cudaError_t launch_token_bytes(const uint8_t *in, long long n_bytes, const long long *offsets, const long long *char_off,
                                const long long *tok_off, long long n_strings, long long n_tokens, const int32_t *spans,
-                               long long *out, unsigned *word_local, unsigned *group_tot, unsigned long long *group_pref,
+                               long long *out, const unsigned *word_local, const unsigned long long *group_pref,
                                const uint8_t *table_blob, const TableLayout &tl, int n_sm, cudaStream_t s);
+// the int8 [C,25] parse matrix (latok_kernels.cu), after launch_char_prefix; starts: char_prefix_words(n_bytes) words
+cudaError_t launch_parse_matrix(const uint8_t *in, long long n_bytes, const long long *offsets, long long n_strings,
+                                uint32_t *starts, const unsigned *word_local, const unsigned long long *group_pref,
+                                const uint8_t *table_blob, const TableLayout &tl, int8_t *matrix, const Result *result,
+                                int n_sm, cudaStream_t s);
 
 // token vocabulary (latok_vocab.cu)
 constexpr unsigned long long VOCAB_COMMITTED = 1ULL << 63;

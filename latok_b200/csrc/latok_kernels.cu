@@ -1,1098 +1,96 @@
-// latok_kernels.cu -- sm_100a kernels for LaTok's tokenization hot path.
+// latok_kernels.cu -- the parse matrix and the stand-alone helpers of the C ABI.
 //
-// One persistent kernel (tokenize_kernel) makes a single pass over the flat UTF-8 buffer (bit-plane form,
-// 32 characters per register):
+//   parse_matrix_kernel   the int8 [C,25] feature matrix (_gen_parse_matrix, latok.c:31-138): one warp per 32-byte word
+//                         of the batch, one lane per byte; every character's 12 class bits plus its context bits
+//   string_starts_kernel  the bitmap of string starts that tells parse_matrix_kernel where strings begin and end
+//   tile_index_kernel     first string of every tokenize range, and the check of the offsets array
+//   block_mask_kernel     stand-alone _gen_block_mask
+//   combine_rows_kernel   stand-alone _combine_matrix_rows
 //
-//   TMA bulk copy of a 16 KB window (owned tile + halos) into shared memory
-//   phase 1  byte space : lead-byte detection, UTF-8 decode, class-table lookup (shared memory)
-//                         -> 12 base feature bits per character           (latok.c:15-29, 77-98)
-//   phase 2a char space : prev / next / after-next context features        (latok.c:68-73, 99-134)
-//                         + rule evaluation split_cnt / mark / sym         (latok.c:318-341 with
-//                           default_tokenizer.py:49-55, 80-91, 100-102)
-//   chain 1  decoupled look-back: character count, current string start, block-mask backlog
-//   phase 2b block mask in scan form (latok.c:218-244), closing the chunk that is open at the
-//            tile end from the right halo (or a look-ahead walk for very long chunks)
-//   phase 3  split values (default_tokenizer.py:121-132), token start/end flags
-//            (default_tokenizer.py:148-158)
-//   chain 2  decoupled look-back: token ordinal (+ feature sums of the token open at the boundary)
-//   phase 4  emission: int8 split mask, int32 spans, CSR offsets, int8 token feature sums
-//            (latok.c:342-354), int8 feature matrix
-//
-// No tensor cores: nothing on this path is a dense contraction; the bound is HBM bandwidth.
+// The tokenize kernel itself (split mask, spans, CSR offsets, token features) is in latok_tok5.cu.
+// No tensor cores: nothing here is a dense contraction.
 #include "latok_device.cuh"
 
 namespace latok {
 
 // =====================================================================================================
-// tokenize_kernel (v4): bit-planes in registers, one speculative look-back chain, chunk-aligned tiles,
-// warp-specialised: warp 0 = service warp (tile tickets, TMA loads, string-start maps, aggregate publish,
-// look-back), warps 1..8 = compute warps.  The compute warps stage a tile's outputs in shared memory, hand
-// its aggregate to the service warp and go on with the next tile; the outputs of tile k-1 are written once its
-// prefix has arrived, so the look-back latency is off the compute warps' critical path.
-// =====================================================================================================
-constexpr int VPAD = 256;      // staging slack in front of the first owned character
-constexpr int NTS = 32;        // service warp
-constexpr int NTHREADS = NT + NTS;
-constexpr int NBUF = 3;        // window buffers: one being computed, one staged for output, one being loaded
-// named barriers (0 is __syncthreads, used during set-up only)
-enum { BAR_C = 1, BAR_AGG = 2, BAR_PRE = 4, BAR_LOADED = 6, BAR_FREE = 9 };
-
-__device__ __forceinline__ int cbar_or(int pred)   // __syncthreads_or over the compute warps
+// Bit o of `starts` is set when a string begins at byte o; offsets[n_strings] = n_bytes sets bit n_bytes, so the bitmap
+// has n_bytes / 32 + 1 words (zeroed by the caller).  Empty strings set the bit of the string after them.
+__global__ void string_starts_kernel(const long long *offsets, long long n_strings, uint32_t *starts, const Result *result)
 {
-    int r;
-    asm volatile("{\n\t.reg .pred p, q;\n\tsetp.ne.s32 p, %1, 0;\n\tbar.red.or.pred q, 1, 256, p;\n\tselp.s32 %0, 1, 0, q;\n\t}" : "=r"(r) : "r"(pred) : "memory");
-    return r;
-}
-#define CBAR() nb_sync(BAR_C, NT)
-
-struct Slot {            // per-tile state handed from the compute warps to the service warp and to the output stage
-    long long tile;
-    int c_lo, c_hi, n_own, ntok, last_tile;
-    int lft_rel;         // last owned string start relative to c_lo, or -1
-    int v_tile;          // backlog leaving the tile
-    int nbf;             // tokens counted before the first owned string start (their indices still lack G_in - base_in)
-    int end0, end0_rel;  // first split that ends the token left open by earlier tiles (-1: none); relative like above?
-    int span_global;     // spans staged in the global scratch (more tokens than the shared-memory stage holds)
-    unsigned long long G_in, base_in, K_in;   // mailbox, written by the service warp
-    int x_in, redo;
-};
-
-struct SmemPlan {
-    int mbar, scal, slots, tile[NBUF], table, spans[2], startbits, leadmask[2], cpref[2], emit[2], tokpref[2], split, edge, scratch, words, tails, total;
-};
-__host__ __device__ inline SmemPlan smem_plan(int table_bytes, bool want_words, bool want_tails = false)
-{
-    SmemPlan s; int o = 0;
-    auto take = [&](int bytes) { int r = o; o += (bytes + 15) & ~15; return r; };
-    s.mbar = take(32);
-    s.scal = take(256);
-    s.slots = take(2 * (int)sizeof(Slot));
-    for (int b = 0; b < NBUF; ++b) s.tile[b] = take(WINB + VPAD + 64);   // window bytes; re-used as the split-value stage
-    s.table = take(table_bytes);
-    for (int i = 0; i < 2; ++i) s.spans[i] = take(SPAN_STAGE * 8 + 16);
-    s.startbits = take(NBUF * NT * 4);
-    for (int i = 0; i < 2; ++i) { s.leadmask[i] = take(NT * 4); s.cpref[i] = take((NT + 1) * 4); s.emit[i] = take(NT * 4); s.tokpref[i] = take((NT + 1) * 4); }
-    s.split = take(NT * 4);
-    s.edge = take(NWARP * 16 * 4);
-    s.scratch = take(1024);
-    s.words = take(want_words ? (WINB + WINB / 32 + 64) * 4 : 0);
-    s.tails = take(want_tails ? NT * 8 * 4 : 0);      // token-feature mode: per thread, feature sums of its open tail + flag
-    s.total = o;
-    return s;
-}
-size_t tokenize_smem_bytes(const TableLayout &tl, bool want_words, bool want_feats) { return (size_t)smem_plan(tl.total, want_words, want_feats).total; }
-
-struct Scalars {          // block-shared scalars
-    long long tile_id[NBUF];
-    int tma_used[NBUF];
-    int c_lo, c_hi, lo_found, hi_found;
-    int need_walk, far;
-    int v_tile, x_end;
-    int end0, end0_rel, nbf;
-};
-
-
-// 4x4 byte transpose: four accumulators (8 characters each, one byte per feature) -> four 32-character planes
-__device__ __forceinline__ void planes4(const uint32_t a[4], uint32_t &p0, uint32_t &p1, uint32_t &p2, uint32_t &p3)
-{
-    const uint32_t t0 = __byte_perm(a[0], a[1], 0x5140), t1 = __byte_perm(a[0], a[1], 0x7362);
-    const uint32_t t2 = __byte_perm(a[2], a[3], 0x5140), t3 = __byte_perm(a[2], a[3], 0x7362);
-    p0 = __byte_perm(t0, t2, 0x5410); p1 = __byte_perm(t0, t2, 0x7632);
-    p2 = __byte_perm(t1, t3, 0x5410); p3 = __byte_perm(t1, t3, 0x7632);
+    if (ld_volatile_u32(&result->error) & 2u) return;  // offsets failed validation in tile_index_kernel
+    const long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (s > n_strings) return;
+    const long long o = offsets[s];
+    atomicOr(&starts[o >> 5], 1u << (o & 31));
 }
 
-// In-register 32x32 bit-matrix transpose: planes (bit j of a[f]) -> per-character words (bit f of a[j])
-__device__ __forceinline__ void transpose32(uint32_t a[32])
+// bytes of the UTF-8 character whose lead byte is b
+__device__ __forceinline__ int utf8_len(uint32_t b) { return b < 0xC0u ? 1 : b < 0xE0u ? 2 : b < 0xF0u ? 3 : 4; }
+
+// One warp per 32-byte word w, lane l on byte 32 w + l.  Row of a character = characters in front of its word
+// (launch_char_prefix) + lead bytes in front of it in the word.  The class words of the next and after-next
+// characters come from the word itself or from the 8 bytes after it (lanes 0..7 also classify those), the previous
+// character's from the word or from the 4 bytes in front of it (lanes 8..11).  The rows of a word are contiguous: they
+// are staged in shared memory and written as consecutive bytes.
+constexpr int PM_WARPS = 8;
+__global__ void __launch_bounds__(PM_WARPS * 32) parse_matrix_kernel(const uint8_t *in, long long n_bytes, const uint32_t *starts,
+                                                                     const unsigned *word_local, const unsigned long long *group_pref,
+                                                                     const uint8_t *table_blob, const TableLayout tl, int8_t *matrix,
+                                                                     const Result *result)
 {
-#pragma unroll
-    for (int j = 16; j != 0; j >>= 1) {
-        const uint32_t m = j == 16 ? 0x0000FFFFu : j == 8 ? 0x00FF00FFu : j == 4 ? 0x0F0F0F0Fu : j == 2 ? 0x33333333u : 0x55555555u;
-#pragma unroll
-        for (int k = 0; k < 32; ++k) {
-            if ((k & j) == 0) {
-                const uint32_t t = ((a[k] >> j) ^ a[k + j]) & m;
-                a[k] ^= t << j;
-                a[k + j] ^= t;
-            }
-        }
-    }
-}
-
-
-
-template <bool kDefault, bool kWords, bool kFeats>
-__global__ void __launch_bounds__(NTHREADS, kWords ? 1 : 2) tokenize_kernel(const Params p)
-{
-    extern __shared__ __align__(128) unsigned char smem[];
-    const SmemPlan sp = smem_plan(p.tl.total, kWords, kFeats);
-    constexpr bool kSync = kWords || kFeats;       // these modes write a tile's outputs with its prefix in hand (not one tile behind)
-    unsigned long long *mbar = reinterpret_cast<unsigned long long *>(smem + sp.mbar);   // [NBUF]
-    Scalars &sc = *reinterpret_cast<Scalars *>(smem + sp.scal);
-    Slot *slots = reinterpret_cast<Slot *>(smem + sp.slots);
-    uint8_t *tableS = smem + sp.table;
-    uint32_t *startbitsS = reinterpret_cast<uint32_t *>(smem + sp.startbits);   // [NBUF][NT]
-    uint32_t *splitS = reinterpret_cast<uint32_t *>(smem + sp.split);
-    uint32_t *edgeS = reinterpret_cast<uint32_t *>(smem + sp.edge);
-    int *scratch = reinterpret_cast<int *>(smem + sp.scratch);
-    uint32_t *wordS = reinterpret_cast<uint32_t *>(smem + sp.words);
-    uint32_t *tailS = reinterpret_cast<uint32_t *>(smem + sp.tails);
+    __shared__ uint32_t rowS[PM_WARPS][32];
+    if (ld_volatile_u32(&result->error) & 2u) return;  // offsets failed validation: the start bitmap was not built
     constexpr unsigned FULL = 0xFFFFFFFFu;
-
-    if (ld_volatile_u32(&p.result->error) & 2u) return;  // offsets failed validation in tile_index_kernel
-
-    // one-time per CTA: tables into shared memory, mbarrier init, clean start-bit maps
-    for (int i = threadIdx.x; i < p.tl.total / 16; i += NTHREADS)
-        reinterpret_cast<uint4 *>(tableS)[i] = __ldg(reinterpret_cast<const uint4 *>(p.table_blob) + i);
-    for (int i = threadIdx.x; i < NBUF * NT; i += NTHREADS) startbitsS[i] = 0;
-    if (threadIdx.x == 0) { for (int b = 0; b < NBUF; ++b) mbar_init(mbar + b, 1); }
-    __syncthreads();
-    const bool want_feats = (p.what & 4u) != 0u, want_matrix = (p.what & 8u) != 0u;
-    const bool want_spans = (p.what & 2u) != 0u, want_splits = (p.what & 1u) != 0u;
-    int2 *span_scratch = reinterpret_cast<int2 *>(p.span_scratch) + (size_t)blockIdx.x * 2 * SPAN_SCRATCH;
-
-    // =================================================================================================
-    // service warp
-    // =================================================================================================
-    if (threadIdx.x < NTS) {
-        const int lane = threadIdx.x;
-        // Start loading window `t` into buffer `b`: TMA bulk copy of the 16-byte aligned interior, plain loads for
-        // the ragged ends, and the string-start bitmap.
-        auto begin_load = [&](long long t, int b) {
-            uint8_t *tileS = smem + sp.tile[b];
-            const long long w0 = t * (long long)TILE - LHALO;
-            const long long lo = w0 < 0 ? 0 : w0;
-            long long hi = w0 + WINB;
-            const long long full16 = p.n_bytes & ~15LL;
-            if (hi > full16) hi = full16;
-            const int tma_bytes = hi > lo ? int(hi - lo) : 0;
-            if (lane == 0) {
-                sc.tma_used[b] = tma_bytes > 0;
-                if (tma_bytes > 0) {
-                    fence_proxy_async();
-                    mbar_expect_tx(mbar + b, (uint32_t)tma_bytes);
-                    tma_load_1d(tileS + (lo - w0), p.in + lo, (uint32_t)tma_bytes, mbar + b);
-                }
-            }
-            const int a_end = int(lo - w0);
-            const int b_beg = a_end + tma_bytes;
-            for (int i = lane; i < a_end; i += NTS) tileS[i] = 0;
-            for (int i = b_beg + lane; i < WINB + 16; i += NTS) {
-                const long long g = w0 + i;
-                tileS[i] = (g >= 0 && g < p.n_bytes) ? p.in[g] : (uint8_t)0;
-            }
-            uint32_t *sbm = startbitsS + b * NT;
-            const long long wend = w0 + WINB;
-            for (long long s = p.tile_first_str[t] + lane; s <= p.n_strings; s += NTS) {
-                const long long o = p.offsets[s];
-                if (o >= wend) break;
-                const int wb = int(o - w0);
-                atomicOr(&sbm[wb >> 5], 1u << (wb & 31));
-            }
-        };
-        auto fetch_and_load = [&](int b) {
-            long long t = 0;
-            if (lane == 0) t = (long long)(atomicAdd(p.ticket, 1ull) - p.ticket_base);
-            t = __shfl_sync(FULL, t, 0);
-            if (lane == 0) sc.tile_id[b] = t;
-            if (t < p.ntiles) begin_load(t, b);
-            __syncwarp();
-            nb_arrive(BAR_LOADED + b, NTHREADS);
-            return t;
-        };
-        long long ids[NBUF];
-        ids[0] = fetch_and_load(0);
-        ids[1] = fetch_and_load(1);
-        ids[2] = 0;
-        for (int k = 0;; ++k) {
-            const int b = k % NBUF, s = k & 1;
-            const long long tile = b == 0 ? ids[0] : (b == 1 ? ids[1] : ids[2]);
-            if (tile >= p.ntiles) break;
-            nb_sync(BAR_AGG + s, NTHREADS);          // the compute warps have staged tile k and filled its slot
-            Slot &sl = slots[s];
-            const int n_own = sl.n_own, ntok = sl.ntok, lft_rel = sl.lft_rel, v_tile = sl.v_tile;
-            if (lane == 0) {
-                uint4 r;
-                r.x = (p.epoch << 2) | 1u;
-                r.y = (unsigned)n_own | ((lft_rel >= 0 ? (unsigned)(lft_rel + 1) : 0u) << 16);
-                r.z = (unsigned)ntok | ((unsigned)v_tile << 16);
-                r.w = 0;
-                st_rec(p.agg + tile, r);
-            }
-            const Prefix pre = lookback(tile, p, lane);
-            if (lane == 0) {
-                sl.G_in = pre.G; sl.base_in = pre.base; sl.K_in = pre.K; sl.x_in = pre.x; sl.redo = pre.x != 0;
-                if (pre.x == 0) {
-                    // inclusive prefix (a tile that does receive a backlog recomputes first and publishes it itself)
-                    IncRec *ir = p.inc + tile;
-                    uint4 a, bq;
-                    const unsigned long long Gn = pre.G + (unsigned long long)n_own, Kn = pre.K + (unsigned long long)ntok;
-                    const unsigned long long Bn = lft_rel >= 0 ? pre.G + (unsigned long long)lft_rel : pre.base;
-                    a.x = (unsigned)Gn; a.y = (unsigned)(Gn >> 32); a.z = (unsigned)Bn; a.w = (unsigned)(Bn >> 32);
-                    bq.x = (unsigned)Kn; bq.y = (unsigned)(Kn >> 32); bq.z = (unsigned)v_tile; bq.w = 0;
-                    st_rec(ir, a); st_rec(reinterpret_cast<uint4 *>(ir) + 1, bq);
-                    __threadfence();
-                    uint4 r;
-                    r.x = (p.epoch << 2) | 2u;
-                    r.y = (unsigned)n_own | ((lft_rel >= 0 ? (unsigned)(lft_rel + 1) : 0u) << 16);
-                    r.z = (unsigned)ntok | ((unsigned)v_tile << 16);
-                    r.w = 0;
-                    st_rec(p.agg + tile, r);
-                }
-            }
-            __syncwarp();
-            nb_arrive(BAR_PRE + s, NTHREADS);
-            if (k >= 1) nb_sync(BAR_FREE + (k - 1) % NBUF, NTHREADS);   // buffer of tile k-1 written out
-            const long long t2 = fetch_and_load((k + 2) % NBUF);
-            if ((k + 2) % NBUF == 0) ids[0] = t2; else if ((k + 2) % NBUF == 1) ids[1] = t2; else ids[2] = t2;
-        }
-        return;
-    }
-
-    // =================================================================================================
-    // compute warps
-    // =================================================================================================
-    const int tid = threadIdx.x - NTS, lane = tid & 31, warp = tid >> 5;
     Tables tb;
-    tb.ascii_feat = reinterpret_cast<const uint16_t *>(tableS + p.tl.ascii_feat);
-    tb.class_feat = reinterpret_cast<const uint16_t *>(tableS + p.tl.class_feat);
-    tb.stage1 = reinterpret_cast<const latok_stage1_t *>(tableS + p.tl.stage1);
-    tb.stage2 = tableS + p.tl.stage2;
-    tb.low_limit = p.tl.low_limit; tb.high_first = p.tl.high_first; tb.high_last = p.tl.high_last; tb.high_feat = p.tl.high_feat;
-    const uint32_t *lut0 = reinterpret_cast<const uint32_t *>(tableS + p.tl.lut3);
-    const uint32_t *lut1 = lut0 + LUT_ENTRIES, *lut2 = lut1 + LUT_ENTRIES;
-    const uint32_t *lutv = reinterpret_cast<const uint32_t *>(tableS + p.tl.lutv);
-#ifdef LATOK_PROFILE
-    long long _prof_t = clock64();
-#endif
-    uint32_t phase_bits = 0;   // mbarrier phase per buffer
-
-    // ---- output stage: everything comes from the slot and the staged shared-memory state of that tile
-    auto emit = [&](int s, int b) {
-        const Slot &sl = slots[s];
-        const long long tile = sl.tile;
-        const long long w0 = tile * (long long)TILE - LHALO;
-        const int c_lo = sl.c_lo, c_hi = sl.c_hi, n_own = sl.n_own, ntok_tile = sl.ntok;
-        const bool last_tile = sl.last_tile != 0;
-        const unsigned long long G_in = sl.G_in, K_in = sl.K_in;
-        const int D = (int)(long long)(G_in - sl.base_in);    // characters of the open string before this tile
-        const uint8_t *valS = smem + sp.tile[b];
-        const uint32_t *leadmaskS = reinterpret_cast<const uint32_t *>(smem + sp.leadmask[s]);
-        const int *cprefS = reinterpret_cast<const int *>(smem + sp.cpref[s]);
-        const uint32_t *emitS = reinterpret_cast<const uint32_t *>(smem + sp.emit[s]);
-        const int *tokprefS = reinterpret_cast<const int *>(smem + sp.tokpref[s]);
-        if (K_in + (unsigned long long)ntok_tile > (unsigned long long)p.cap_tokens && tid == 0) atomicOr(&p.result->error, 4u);
-        // consistency check: a prefix can never exceed the input size (catches chain corruption instead of faulting)
-        if (G_in + (unsigned long long)n_own > (unsigned long long)p.n_bytes || K_in + (unsigned long long)ntok_tile > (unsigned long long)p.n_bytes ||
-            n_own < 0 || ntok_tile < 0) {
-            if (tid == 0 && atomicOr(&p.result->error, 8u) == 0u) {
-                p.result->prof[8] = (unsigned long long)tile; p.result->prof[9] = G_in; p.result->prof[10] = K_in;
-                p.result->prof[11] = (unsigned long long)(long long)n_own; p.result->prof[12] = (unsigned long long)(long long)ntok_tile;
-                p.result->prof[13] = (unsigned long long)(long long)c_lo; p.result->prof[14] = (unsigned long long)(long long)c_hi;
-            }
-            return;
-        }
-        if (want_splits && n_own > 0) {
-            // dst[j] <-> valS[VPAD + j]; 16-byte global chunks are assembled from the (differently aligned) staging words
-            int8_t *dst = p.splits + G_in;
-            const int a16 = int(G_in & 15ull);
-            const int head = (16 - a16) & 15;
-            const int nh = head < n_own ? head : n_own;
-            if (tid < nh) dst[tid] = (int8_t)valS[VPAD + tid];
-            const int nchunks = (n_own - nh) >> 4;
-            const uint32_t *sw = reinterpret_cast<const uint32_t *>(valS);
-            const int sbyte = VPAD + nh;                    // staging byte of chunk 0
-            const int shb = 8 * (sbyte & 3);
-            uint4 *d4 = reinterpret_cast<uint4 *>(dst + nh);
-            for (int i = tid; i < nchunks; i += NT) {
-                const uint32_t *q = sw + ((sbyte + 16 * i) >> 2);
-                uint4 v;
-                if (shb == 0) { v.x = q[0]; v.y = q[1]; v.z = q[2]; v.w = q[3]; }
-                else {
-                    const uint32_t q0 = q[0], q1 = q[1], q2 = q[2], q3 = q[3], q4 = q[4];
-                    v.x = __funnelshift_r(q0, q1, shb); v.y = __funnelshift_r(q1, q2, shb);
-                    v.z = __funnelshift_r(q2, q3, shb); v.w = __funnelshift_r(q3, q4, shb);
-                }
-                d4[i] = v;
-            }
-            const int done = nh + (nchunks << 4);
-            if (tid < n_own - done) dst[done + tid] = (int8_t)valS[VPAD + done + tid];
-        }
-        if (want_spans) {
-            const int2 *src = sl.span_global ? span_scratch + (size_t)s * SPAN_SCRATCH : reinterpret_cast<const int2 *>(smem + sp.spans[s]) + 1;
-            const int nbf = sl.nbf;
-            int2 *dst = reinterpret_cast<int2 *>(p.spans) + K_in;
-            for (int i = tid; i < ntok_tile; i += NT) {
-                int2 v = src[i];
-                if (i < nbf) { v.x += D; if (v.y >= 0) v.y += D; }
-                if ((long long)K_in + i < p.cap_tokens) {
-                    if (v.y >= 0) dst[i] = v;
-                    else p.spans[2 * (K_in + i)] = v.x;        // still open: a later tile writes the end
-                }
-            }
-            if (tid == 0 && sl.end0 >= 0) {
-                const long long k = (long long)K_in - 1;
-                if (k >= 0 && k < p.cap_tokens) p.spans[2 * k + 1] = sl.end0 + (sl.end0_rel ? D : 0);
-            }
-        }
-        if (kWords && want_matrix) {
-            int8_t *dst = p.matrix + G_in * NFEAT;
-            const int nb = n_own * NFEAT;
-            for (int j = tid; j < nb; j += NT) {
-                const int c = j / NFEAT, f = j - c * NFEAT;
-                dst[j] = (int8_t)((wordS[widx(c_lo + c)] >> f) & 1u);
-            }
-        }
-        // per-string CSR offsets for the strings whose first character position is owned by this tile
-        {
-            auto cidx = [&](int wb) -> int {
-                int t = wb >> 5;
-                if (t >= NT) return cprefS[NT];
-                return cprefS[t] + __popc(leadmaskS[t] & mask_lt(wb & 31));
-            };
-            const long long wend = w0 + WINB;
-            for (long long q = p.tile_first_str[tile] + tid; q <= p.n_strings; q += NT) {
-                const long long o = p.offsets[q];
-                if (o >= wend) break;
-                const int wb = int(o - w0);
-                const int c = cidx(wb);
-                const bool mine = last_tile ? (c >= c_lo) : (c >= c_lo && c < c_hi);
-                if (!mine) continue;
-                p.char_off[q] = (long long)(G_in + (unsigned long long)(c - c_lo));
-                const int t = wb >> 5;
-                p.tok_off[q] = (long long)K_in + tokprefS[t] + __popc(emitS[t] & mask_lt(c - cprefS[t]));
-            }
-        }
-        if (last_tile && tid == 0) {
-            p.result->n_chars = G_in + (unsigned long long)n_own;
-            p.result->n_tokens = K_in + (unsigned long long)ntok_tile;
-        }
-    };
-
-    int k = 0, redo_k = -1;
-    bool drained = false;
-    for (;;) {
-        const bool is_redo = redo_k >= 0;
-        const int wk = is_redo ? redo_k : k;
-        const int bcur = wk % NBUF, scur = wk & 1;
-        uint8_t *tileS = smem + sp.tile[bcur];
-        uint8_t *valS = tileS;            // the window bytes are dead after phase 1
-        uint32_t *sbm = startbitsS + bcur * NT;
-        uint32_t *leadmaskS = reinterpret_cast<uint32_t *>(smem + sp.leadmask[scur]);
-        int *cprefS = reinterpret_cast<int *>(smem + sp.cpref[scur]);
-        uint32_t *emitS = reinterpret_cast<uint32_t *>(smem + sp.emit[scur]);
-        int *tokprefS = reinterpret_cast<int *>(smem + sp.tokpref[scur]);
-        int2 *spanS = reinterpret_cast<int2 *>(smem + sp.spans[scur]);
-        long long tile = 0;
-        int x_tile_in = 0;
-        bool have_work = true;
-        PROF(9);
-        if (is_redo) {
-            // a backlog does enter this tile (rare): fetch its window again and recompute with it
-            tile = slots[scur].tile; x_tile_in = slots[scur].x_in;
-            const long long w0r = tile * (long long)TILE - LHALO;
-            for (int i = tid; i < WINB + 16; i += NT) {
-                const long long g = w0r + i;
-                tileS[i] = (g >= 0 && g < p.n_bytes) ? p.in[g] : (uint8_t)0;
-            }
-            sbm[tid] = 0;
-            CBAR();
-            const long long wend = w0r + WINB;
-            for (long long q = p.tile_first_str[tile] + tid; q <= p.n_strings; q += NT) {
-                const long long o = p.offsets[q];
-                if (o >= wend) break;
-                const int wb = int(o - w0r);
-                atomicOr(&sbm[wb >> 5], 1u << (wb & 31));
-            }
-            CBAR();
-        } else {
-            nb_sync(BAR_LOADED + bcur, NTHREADS);
-            tile = sc.tile_id[bcur];
-            if (tile >= p.ntiles) have_work = false;
-            else if (sc.tma_used[bcur]) { mbar_wait(mbar + bcur, (phase_bits >> bcur) & 1u); phase_bits ^= 1u << bcur; }
-        }
-        PROF(0);
-        if (have_work) {
-        const long long w0 = tile * (long long)TILE - LHALO;
-        if (tid == 0) { sc.need_walk = 0; sc.far = 0; sc.lo_found = 0; sc.hi_found = 0; sc.end0 = -1; sc.end0_rel = 0; sc.nbf = -1; }
-
-        // ------------------------------------------------------------------ phase 1: bytes -> bit-planes
-        const int wb0 = tid * 32;
-        const uint32_t sb = sbm[tid];
-        sbm[tid] = 0;                       // leave the bitmap clean for the tile after next
-        uint32_t lead, mbl;                 // lead bytes / lead bytes of multi-byte characters (byte positions)
-        int vhi, nvalid;                    // valid bytes: [vlo, vhi) of this thread's 32
-        uint32_t acc0[4], acc1[4], acc2[4];
-        {
-            const uint4 q0 = *reinterpret_cast<const uint4 *>(tileS + wb0);
-            const uint4 q1 = *reinterpret_cast<const uint4 *>(tileS + wb0 + 16);
-            const uint32_t wds[8] = {q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w};
-            uint32_t leadbits = 0, hib = 0;
-#pragma unroll
-            for (int j = 0; j < 8; ++j) {
-                uint32_t t = (wds[j] & 0xC0C0C0C0u) ^ 0x80808080u;   // byte == 0  <=>  continuation byte
-                uint32_t m = (t | (t << 1)) & 0x80808080u;
-                leadbits |= (((m >> 7) * 0x10204080u) >> 28) << (4 * j);
-                hib |= ((((wds[j] & 0x80808080u) >> 7) * 0x10204080u) >> 28) << (4 * j);
-            }
-            const long long g0 = w0 + wb0;
-            const int vlo = g0 < 0 ? int(-g0 < 32 ? -g0 : 32) : 0;
-            const long long rem = p.n_bytes - g0;
-            vhi = rem <= 0 ? 0 : (rem >= 32 ? 32 : int(rem));
-            const uint32_t valid = vhi > vlo ? (mask_lt(vhi) & ~mask_lt(vlo)) : 0u;
-            nvalid = vhi > vlo ? vhi - vlo : 0;
-            lead = (leadbits & valid) | sb;
-            mbl = leadbits & hib & valid;     // bytes >= 0xC0 inside the data
-            // every byte through the feature LUT (bytes >= 0x80 and padding map to "no features")
-#pragma unroll
-            for (int g = 0; g < 4; ++g) {
-                uint32_t a0 = 0, a1 = 0, a2 = 0;
-#pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    const uint32_t b = (wds[2 * g + (j >> 2)] >> ((j & 3) * 8)) & 0xFFu;
-                    a0 += lut0[b] << j; a1 += lut1[b] << j; a2 += lut2[b] << j;
-                }
-                acc0[g] = a0; acc1[g] = a1; acc2[g] = a2;
-            }
-        }
-        // patch in the multi-byte characters (decode + two-stage class table)
-        {
-            uint32_t mm = mbl;
-            while (mm) {
-                const int k = __ffs(mm) - 1; mm &= mm - 1;
-                const uint32_t e = mb_entry(tileS + wb0 + k, tb, p.tl.high_class);
-                const uint32_t x0 = lut0[e] << (k & 7), x1 = lut1[e] << (k & 7), x2 = lut2[e] << (k & 7);
-                const int g = k >> 3;
-#pragma unroll
-                for (int q = 0; q < 4; ++q)
-                    if (g == q) { acc0[q] |= x0; acc1[q] |= x1; acc2[q] |= x2; }
-            }
-        }
-        uint32_t P[12];
-        planes4(acc0, P[0], P[1], P[2], P[3]);
-        planes4(acc1, P[4], P[5], P[6], P[7]);
-        planes4(acc2, P[8], P[9], P[10], P[11]);
-        uint32_t Fm = sb;
-        // byte space -> character space: squeeze out the continuation-byte positions
-        {
-            uint32_t del = lead ? (~lead & mask_lt(vhi)) : 0u;
-#pragma unroll
-            for (int f = 0; f < 12; ++f) P[f] &= lead;
-            while (del) {
-                const int top = 31 - __clz(del);
-                const int r = __clz(~(del << (31 - top)));       // run length of deleted bytes ending at `top`
-                const int c = top - r;                            // last kept position below the run (may be -1)
-                const uint32_t keep = mask_lt(c + 1);
-#pragma unroll
-                for (int f = 0; f < 12; ++f) P[f] = (P[f] & keep) | ((P[f] >> r) & ~keep);
-                Fm = (Fm & keep) | ((Fm >> r) & ~keep);
-                del &= keep;
-            }
-        }
-        PROF(1);
-        const int n = __popc(lead);                     // characters of this thread (incl. the end-of-data terminator)
-
-        // ---- character-count scan + neighbour exchange (one barrier)
-        const uint32_t myLB = n > 0 ? ((((P[PL_A] >> (n - 1)) & 1u)) | (((P[PL_N] >> (n - 1)) & 1u) << 1) |
-                                       (((P[PL_LO] >> (n - 1)) & 1u) << 2) | (((P[PL_SP] >> (n - 1)) & 1u) << 3) |
-                                       (((P[PL_SY] >> (n - 1)) & 1u) << 4))
-                                    : 0u;
-        int nscan = n;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) { const int t = __shfl_up_sync(FULL, nscan, d); if (lane >= d) nscan += t; }
-        uint32_t LB = __shfl_up_sync(FULL, myLB, 1);
-        uint32_t XA = __shfl_down_sync(FULL, P[PL_A], 1), XN = __shfl_down_sync(FULL, P[PL_N], 1);
-        uint32_t XLO = __shfl_down_sync(FULL, P[PL_LO], 1), XSP = __shfl_down_sync(FULL, P[PL_SP], 1);
-        uint32_t XAT = __shfl_down_sync(FULL, P[PL_AT], 1), XSL = __shfl_down_sync(FULL, P[PL_SL], 1);
-        uint32_t XF = __shfl_down_sync(FULL, Fm, 1);
-        if (lane == 0) {
-            uint32_t *e = edgeS + warp * 16;
-            e[0] = P[PL_A]; e[1] = P[PL_N]; e[2] = P[PL_LO]; e[3] = P[PL_SP]; e[4] = P[PL_AT]; e[5] = P[PL_SL]; e[6] = Fm;
-        }
-        if (lane == 31) { edgeS[warp * 16 + 8] = myLB; scratch[warp] = nscan; }
-        leadmaskS[tid] = lead;
-        CBAR();  // (B)
-        int c0 = nscan - n, c_end = 0;
-#pragma unroll
-        for (int w = 0; w < NWARP; ++w) { const int t = scratch[w]; if (w < warp) c0 += t; c_end += t; }
-        cprefS[tid] = c0;
-        if (tid == 0) cprefS[NT] = c_end;
-        if (lane == 31) {
-            if (warp + 1 < NWARP) {
-                const uint32_t *e = edgeS + (warp + 1) * 16;
-                XA = e[0]; XN = e[1]; XLO = e[2]; XSP = e[3]; XAT = e[4]; XSL = e[5]; XF = e[6];
-            } else { XA = XN = XLO = XSP = XAT = XSL = XF = 0; }
-        }
-        if (lane == 0) LB = warp > 0 ? edgeS[(warp - 1) * 16 + 8] : 0u;
-
-        // ------------------------------------------------------------------ phase 2a: context planes + rules
-        const bool term_in_win = p.n_bytes < w0 + WINB;
-        const long long g0 = w0 + wb0;
-        const bool has_term = p.n_bytes >= g0 && p.n_bytes < g0 + 32;
-        const uint32_t REAL = mask_lt(n - (has_term ? 1 : 0));
-        // characters with complete forward context (everything but the last few bytes of the window)
-        uint32_t TRUST = tid >= FIRST_OWNED_THREAD ? REAL : 0u;
-        if (tid == NT - 1 && !term_in_win) TRUST &= mask_lt(__popc(lead & mask_lt(32 - TRUST_MARGIN)));
-
-        auto next1 = [&](uint32_t X, uint32_t Xn) -> uint32_t {
-            const uint32_t l = X | __funnelshift_lc(0u, Xn, n), h = __funnelshift_lc(Xn, 0u, n);
-            return __funnelshift_r(l, h, 1);
+    tb.ascii_feat = reinterpret_cast<const uint16_t *>(table_blob + tl.ascii_feat);
+    tb.class_feat = reinterpret_cast<const uint16_t *>(table_blob + tl.class_feat);
+    tb.stage1 = reinterpret_cast<const latok_stage1_t *>(table_blob + tl.stage1); tb.stage2 = table_blob + tl.stage2;
+    tb.low_limit = tl.low_limit; tb.high_first = tl.high_first; tb.high_last = tl.high_last; tb.high_feat = tl.high_feat;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    uint32_t *rows = rowS[warp];
+    const long long nwords = n_bytes / TB_WORD + 1;
+    for (long long w = (long long)blockIdx.x * PM_WARPS + warp; w < nwords; w += (long long)gridDim.x * PM_WARPS) {
+        const long long base = w * TB_WORD, pos = base + lane;
+        const long long xpos = lane < 8 ? base + 32 + lane : base - 12 + lane;
+        const uint32_t b = pos < n_bytes ? in[pos] : 0x80u;
+        const uint32_t xb = lane < 12 && xpos >= 0 && xpos < n_bytes ? in[xpos] : 0x80u;
+        const bool lead = (b & 0xC0u) != 0x80u, xlead = (xb & 0xC0u) != 0x80u;
+        const unsigned leads = __ballot_sync(FULL, lead), xleads = __ballot_sync(FULL, xlead);
+        if (!leads) continue;
+        const uint32_t cw = lead ? classify_at(in + pos, tb) : 0u, xw = xlead ? classify_at(in + xpos, tb) : 0u;
+        // value v of the byte q = 0 .. 39 of the word (q >= 32: the bytes after it, held by lanes 0..7)
+        auto at = [&](uint32_t v, uint32_t xv, int q) {
+            const uint32_t a = __shfl_sync(FULL, v, q & 31), c = __shfl_sync(FULL, xv, (q - 32) & 31);
+            return q < 32 ? a : c;
         };
-        auto next2 = [&](uint32_t X, uint32_t Xn) -> uint32_t {
-            const uint32_t l = X | __funnelshift_lc(0u, Xn, n), h = __funnelshift_lc(Xn, 0u, n);
-            return __funnelshift_r(l, h, 2);
-        };
-        const uint32_t Lm_raw = next1(Fm, XF);           // character ends a string (next one starts a string)
-        const uint32_t L2m = next2(Fm, XF);
-        const uint32_t nF = ~Lm_raw, aF = ~(Lm_raw | L2m), pF = ~Fm;
-        const uint32_t Sraw = P[PL_SP];
-
-        // ---- chunk-aligned ownership: the tile owns the characters from just after the first closer found in
-        // the SEARCH bytes after its nominal start up to (and including) the first closer found in the SEARCH
-        // bytes after its nominal end; both neighbours look at the same bytes, so they agree.
-        {
-            const uint32_t CLr = (Sraw | Lm_raw) & REAL;
-            // characters whose lead byte lies in [nominal boundary, nominal boundary + SEARCH)
-            uint32_t cand = 0; bool lo_side = false, hi_side = false;
-            if (tid >= FIRST_OWNED_THREAD && tid < FIRST_OWNED_THREAD + RHALO / 32) { lo_side = true; cand = CLr; if (tid == FIRST_OWNED_THREAD + RHALO / 32 - 1) cand &= mask_lt(__popc(lead & mask_lt(32 - TRUST_MARGIN))); }
-            if (tid >= END_OWNED_THREAD) { hi_side = true; cand = CLr; if (tid == NT - 1) cand &= mask_lt(__popc(lead & mask_lt(32 - TRUST_MARGIN))); }
-            const unsigned blo = __ballot_sync(FULL, lo_side && cand != 0u), bhi = __ballot_sync(FULL, hi_side && cand != 0u);
-            if (lo_side && cand != 0u && (blo & mask_lt(lane)) == 0u && tile > 0) { sc.c_lo = c0 + __ffs(cand); sc.lo_found = 1; }
-            if (hi_side && cand != 0u && (bhi & mask_lt(lane)) == 0u) { sc.c_hi = c0 + __ffs(cand); sc.hi_found = 1; }
-        }
-        uint32_t full[25];
-#pragma unroll
-        for (int f = 0; f < 12; ++f) full[f] = P[f];
-        full[12] = ((P[PL_A] << 1) | (LB & 1u)) & pF;                 // PREV_ALPHA
-        full[13] = next1(P[PL_A], XA) & nF;                           // NEXT_ALPHA
-        full[14] = ((P[PL_N] << 1) | ((LB >> 1) & 1u)) & pF;          // PREV_ALPHA_NUM
-        full[15] = next1(P[PL_N], XN) & nF;                           // NEXT_ALPHA_NUM
-        full[16] = ((P[PL_LO] << 1) | ((LB >> 2) & 1u)) & pF;         // PREV_LOWER
-        full[17] = next1(P[PL_LO], XLO) & nF;                         // NEXT_LOWER
-        full[18] = ((P[PL_SP] << 1) | ((LB >> 3) & 1u)) | Fm;         // PREV_SPACE  (start of string = space)
-        full[19] = next1(P[PL_SP], XSP) | Lm_raw;                     // NEXT_SPACE  (end of string = space)
-        full[20] = ((P[PL_SY] << 1) | ((LB >> 4) & 1u)) & pF;         // PREV_SYMBOL
-        full[21] = next1(P[PL_AT], XAT) & nF;                         // NEXT_AT
-        full[22] = next1(P[PL_SL], XSL) & nF;                         // NEXT_SLASH
-        full[23] = next2(P[PL_A], XA) & aF;                           // AFTER_NEXT_ALPHA
-        full[24] = next2(P[PL_SL], XSL) & aF;                         // AFTER_NEXT_SLASH
-
-        // ---- rules: split count, mark, sym (combine_matrix_rows 2-D, latok.c:318-341) as bit-sliced counters
-        uint32_t CNT[4], SYC[4], Mraw;
-        if (kDefault) {
-            // C_SPLIT: SPACE + SYMBOL + PREV_SYMBOL + UPPER*NEXT_LOWER + UPPER*PREV_LOWER (default_tokenizer.py:49-55)
-            const uint32_t t1 = full[5], t2 = full[6], t3 = full[20], t4 = full[4] & full[17], t5 = full[4] & full[16];
-            const uint32_t s1 = t1 ^ t2 ^ t3, c1 = (t1 & t2) | (t3 & (t1 ^ t2));
-            const uint32_t s2 = t4 ^ t5, c2 = t4 & t5;
-            CNT[0] = s1 ^ s2;
-            const uint32_t c3 = s1 & s2;
-            CNT[1] = c1 ^ c2 ^ c3;
-            CNT[2] = (c1 & c2) | (c3 & (c1 ^ c2));
-            CNT[3] = 0;
-            // C_MASK (default_tokenizer.py:80-91)
-            Mraw = (full[7] & full[18] & full[13]) | (full[11] & full[18] & full[21] & full[23]) |
-                   (full[8] & full[14] & full[15]) | (full[9] & full[22] & full[24] & full[12]);
-            // C_SYM: SYMBOL*NEXT_SPACE (default_tokenizer.py:100-102)
-            SYC[0] = full[6] & full[19]; SYC[1] = SYC[2] = SYC[3] = 0;
-        } else {
-            auto term = [&](uint32_t mask) -> uint32_t {
-                uint32_t a = 0xFFFFFFFFu;
-#pragma unroll
-                for (int f = 0; f < NFEAT; ++f) a &= full[f] | (((mask >> f) & 1u) - 1u);
-                return a;
-            };
-            auto add1 = [&](uint32_t c[4], uint32_t t) {
-#pragma unroll
-                for (int b = 0; b < 4; ++b) { const uint32_t k = c[b] & t; c[b] ^= t; t = k; }
-            };
-#pragma unroll
-            for (int b = 0; b < 4; ++b) { CNT[b] = 0; SYC[b] = 0; }
-            Mraw = 0;
-            for (int i = 0; i < p.rules.n_split; ++i) add1(CNT, term(p.rules.split[i]));
-            for (int i = 0; i < p.rules.n_mask; ++i) Mraw |= term(p.rules.mask[i]);
-            for (int i = 0; i < p.rules.n_sym; ++i) add1(SYC, term(p.rules.sym[i]));
-        }
-        if (kWords) {
-            // per-character 25-bit words (+ FIRST / LAST flags) for the token-feature and matrix emitters
-            uint32_t a[32];
-#pragma unroll
-            for (int f = 0; f < 25; ++f) a[f] = full[f];
-            a[25] = Fm; a[26] = Lm_raw;
-#pragma unroll
-            for (int f = 27; f < 32; ++f) a[f] = 0;
-            transpose32(a);
-#pragma unroll
-            for (int j = 0; j < 32; ++j)
-                if (j < n) wordS[widx(c0 + j)] = a[j];
-        }
-        CBAR();  // (C) boundaries
-        PROF(2);
-
-        auto cidx = [&](int wb) -> int {  // characters starting at window bytes < wb
-            int t = wb >> 5;
-            if (t >= NT) return cprefS[NT];
-            return cprefS[t] + __popc(leadmaskS[t] & mask_lt(wb & 31));
-        };
-        // tile-relative character indices of the owned range [c_lo, c_hi)
-        const bool last_tile = tile == p.ntiles - 1;
-        const int c_lo = sc.lo_found ? sc.c_lo : cprefS[FIRST_OWNED_THREAD];
-        int c_hi;
-        if (last_tile) c_hi = cidx(int(p.n_bytes - w0));
-        else c_hi = sc.hi_found ? sc.c_hi : cprefS[END_OWNED_THREAD];
-        const bool closed = last_tile || sc.hi_found;      // the owned range ends at a chunk closer
-        const int n_own = c_hi - c_lo;
-        const uint32_t OWN = range_mask(c0, c_lo, c_hi) & REAL;
-        // characters the block mask is evaluated on: the owned ones, plus (only when the last owned chunk is
-        // still open) the trusted halo, where it may close
-        const uint32_t ACT = closed ? OWN : (range_mask(c0, c_lo, 0x7FFFFFFF) & TRUST);
-        const uint32_t S = Sraw & ACT, Mm = Mraw & ACT, FmA = Fm & ACT, Lm = Lm_raw & ACT;
-        const uint32_t CL = S | Lm;        // characters that close a whitespace chunk
-
-        // last string start among the owned characters (tile-relative), and for each thread the latest one before it
-        int lf_excl;
-        {
-            const uint32_t FO = Fm & OWN;
-            const int mine = FO ? c0 + 31 - __clz(FO) : -1;
-            const unsigned has = __ballot_sync(FULL, FO != 0u);
-            const unsigned below = has & mask_lt(lane);
-            const int src = below ? 31 - __clz(below) : 0;
-            const int got = __shfl_sync(FULL, mine, src);
-            lf_excl = below ? got : -1;
-            const int wlast = __shfl_sync(FULL, mine, has ? 31 - __clz(has) : 0);
-            const int wfirst = __shfl_sync(FULL, FO ? c0 + __ffs(FO) - 1 : 0, has ? __ffs(has) - 1 : 0);
-            if (lane == 0) { scratch[128 + warp] = has ? wlast : -1; scratch[136 + warp] = has ? wfirst : 0x7FFFFFFF; }
-            // owned marks / spaces (for the backlog transfer function of the tile)
-            const int cm = __reduce_add_sync(FULL, __popc(Mraw & OWN)), cs = __reduce_add_sync(FULL, __popc(Sraw & OWN));
-            if (lane == 0) { scratch[144 + warp] = cm; scratch[152 + warp] = cs; }
-        }
-
-        // token-feature mode: 25 population counts of the feature planes over a set of this thread's characters, one byte
-        // per feature (uint8 wrap-around like combine_matrix_rows 1-D, latok.c:342-354)
-        auto plane_sums = [&](uint32_t frag, unsigned acc[7]) {
-#pragma unroll
-            for (int f = 0; f < NFEAT; ++f) acc[f >> 2] += (unsigned)__popc(full[f] & frag) << (8 * (f & 3));   // <= 32 each: no carry
-        };
-        // add the open tails of the threads before `t` until one of them holds the token's first character (a split)
-        auto walk_threads = [&](int t, unsigned acc[7], bool &hit) {
-            for (; t >= FIRST_OWNED_THREAD && !hit; --t) {
-                const uint4 a = *reinterpret_cast<const uint4 *>(tailS + t * 8), b = *reinterpret_cast<const uint4 *>(tailS + t * 8 + 4);
-                acc[0] = __vadd4(acc[0], a.x); acc[1] = __vadd4(acc[1], a.y); acc[2] = __vadd4(acc[2], a.z); acc[3] = __vadd4(acc[3], a.w);
-                acc[4] = __vadd4(acc[4], b.x); acc[5] = __vadd4(acc[5], b.y); acc[6] = __vadd4(acc[6], b.z);
-                hit = b.w != 0u;
-            }
-        };
-        // feature sums of the token still open at the end of the owned range (one thread; token-feature mode)
-        auto publish_open_sums = [&]() {
-            unsigned acc[7] = {0, 0, 0, 0, 0, 0, 0}; bool hit = false;
-            if (n_own > 0) walk_threads(NT - 1, acc, hit);
-            uint4 a, b, c4;
-            a.x = hit ? 1u : 0u; a.y = a.z = a.w = 0;
-            b.x = acc[0]; b.y = acc[1]; b.z = acc[2]; b.w = acc[3];
-            c4.x = acc[4]; c4.y = acc[5]; c4.z = acc[6]; c4.w = 0;
-            uint4 *o = reinterpret_cast<uint4 *>(p.osum + tile);
-            st_rec(o, a); st_rec(o + 1, b); st_rec(o + 2, c4);
-        };
-        uint32_t HOT = 0, Zm = 0, SPLIT = 0, E = 0, V[5];
-        int ntok_tile = 0, tp = 0, slow = 0;
-        {
-            // ---- backlog relaxation: every thread starts from 0, carries are propagated until nothing changes
-            int xin = 0, out = 0, warp_seed = warp == 0 ? x_tile_in : 0, pub = 0;
-            if (Mm) out = eval_backlog(0, Mm, FmA, S, Lm, HOT); else HOT = 0;
-            for (;;) {
-                for (;;) {
-                    int nx = __shfl_up_sync(FULL, out, 1);
-                    if (lane == 0) nx = warp_seed;
-                    const bool ch = nx != xin;
-                    if (!__any_sync(FULL, ch)) break;
-                    if (ch) { xin = nx; if (xin != 0 || Mm) out = eval_backlog(xin, Mm, FmA, S, Lm, HOT); else { out = 0; HOT = 0; } }
-                }
-                const int o31 = __shfl_sync(FULL, out, 31);
-                const bool ch = o31 != pub;
-                pub = o31;
-                if (lane == 31) scratch[64 + warp] = o31;
-                if (!cbar_or(ch ? 1 : 0)) break;   // (D)
-                const int seed = warp > 0 ? scratch[64 + warp - 1] : x_tile_in;
-                CBAR();
-                warp_seed = seed;
-            }
-            // backlog after the last owned character (tile transfer function at 0) and at the end of ACT
-            if (closed) { if (tid == NT - 1) { sc.v_tile = out; sc.x_end = out; } }
-            else { if (tid == END_OWNED_THREAD - 1) sc.v_tile = out; if (tid == NT - 1) sc.x_end = out; }
-
-            // ---- blank the chunks whose closer is hot: flood HOT downwards to the previous closer
-            Zm = HOT;
-            {
-                uint32_t pr = ~CL;
-                Zm |= pr & (Zm >> 1); pr &= pr >> 1;
-                Zm |= pr & (Zm >> 2); pr &= pr >> 2;
-                Zm |= pr & (Zm >> 4); pr &= pr >> 4;
-                Zm |= pr & (Zm >> 8); pr &= pr >> 8;
-                Zm |= pr & (Zm >> 16);
-            }
-            const bool hasCL = CL != 0u;
-            const bool firstHot = hasCL && (HOT & (CL & (0u - CL))) != 0u;
-            int cin;
-            {
-                const unsigned H = __ballot_sync(FULL, hasCL), FH = __ballot_sync(FULL, firstHot);
-                if (lane == 0) { scratch[80 + 2 * warp] = H != 0u; scratch[80 + 2 * warp + 1] = H ? ((FH >> (__ffs(H) - 1)) & 1u) : 0u; }
-                // an owned range that does not end at a closer: the last owned chunk may need the look-ahead walk
-                if (!closed && warp == NWARP - 1) {
-                    const unsigned above = lane == 31 ? 0u : (H & (0xFFFFFFFFu << (lane + 1)));
-                    if (tid == END_OWNED_THREAD - 1) {
-                        const int nr = __popc(ACT);
-                        if (nr > 0 && ((CL >> (nr - 1)) & 1u) == 0u && above == 0u) sc.need_walk = 1;
-                    }
-                }
-                CBAR();  // (E)
-                const unsigned above = lane == 31 ? 0u : (H & (0xFFFFFFFFu << (lane + 1)));
-                if (above) cin = (FH >> (__ffs(above) - 1)) & 1u;
-                else {
-                    cin = 2;
-                    for (int w2 = warp + 1; w2 < NWARP; ++w2)
-                        if (scratch[80 + 2 * w2]) { cin = scratch[80 + 2 * w2 + 1]; break; }
-                }
-            }
-            if (sc.need_walk) {
-                if (sc.x_end >= 1) { if (tid == 0) sc.far = 1; }
-                else if (warp == 0) {
-                    bool any = walk_ahead(p, tb, w0 + WINB - TRUST_MARGIN, lane);
-                    if (lane == 0) { sc.far = any ? 1 : 0; if (!is_redo) atomicAdd(&p.result->walks, 1ull); }
-                }
-                CBAR();
-            }
-            if (cin == 1 || (cin == 2 && sc.far)) {
-                const uint32_t top = hasCL ? ~((2u << (31 - __clz(CL))) - 1u) : 0xFFFFFFFFu;
-                Zm |= top;
-            }
-
-            // ---- split values: splits = split_cnt * block_mask + sym; splits[0] = 1 (default_tokenizer.py:121-132)
-            const uint32_t keepm = ~Zm | Sraw;             // block mask = 1
-            {
-                uint32_t carry = 0;
-#pragma unroll
-                for (int b = 0; b < 4; ++b) {
-                    const uint32_t x = CNT[b] & keepm, y = SYC[b];
-                    V[b] = x ^ y ^ carry;
-                    carry = (x & y) | (carry & (x ^ y));
-                }
-                V[4] = carry;
-                V[0] |= Fm;
-#pragma unroll
-                for (int b = 1; b < 5; ++b) V[b] &= ~Fm;
-            }
-            SPLIT = V[0] | V[1] | V[2] | V[3] | V[4];
-            const uint32_t PS = (Sraw << 1) | ((LB >> 3) & 1u);                // previous character is a space
-            E = ((SPLIT & ~Sraw) | (~SPLIT & PS & ~Fm)) & OWN;                 // a token is counted at this character
-            int tscan = __popc(E);
-            const int mytok = tscan;
-#pragma unroll
-            for (int d = 1; d < 32; d <<= 1) { const int t = __shfl_up_sync(FULL, tscan, d); if (lane >= d) tscan += t; }
-            if (lane == 31) scratch[96 + warp] = tscan;
-            emitS[tid] = E; splitS[tid] = SPLIT;
-            slow = cbar_or((want_splits && nvalid == 32 && n < 4) ? 1 : 0);  // (F) malformed UTF-8 only
-            tp = tscan - mytok; ntok_tile = 0;
-#pragma unroll
-            for (int w = 0; w < NWARP; ++w) { const int t = scratch[96 + w]; if (w < warp) tp += t; ntok_tile += t; }
-
-        }
-        PROF(3);
-        {   // latest owned string start in the warps before this one
-            int lfw = -1;
-#pragma unroll
-            for (int w = 0; w < NWARP; ++w) if (w < warp) lfw = max(lfw, scratch[128 + w]);
-            lf_excl = max(lf_excl, lfw);
-        }
-        int lft = -1, ffirst = 0x7FFFFFFF;
-#pragma unroll
-        for (int w = 0; w < NWARP; ++w) { lft = max(lft, scratch[128 + w]); ffirst = min(ffirst, scratch[136 + w]); }
-
-        // ------------------------------------------------------------------ phase 4: staging (no prefix needed)
-        tokprefS[tid] = tp;
-        if (tid == 0) tokprefS[NT] = ntok_tile;
-        const bool span_global = ntok_tile > SPAN_STAGE - 1;
-        // tokens counted before the first owned string start belong to the string that began in an earlier tile:
-        // their indices are staged relative to c_lo and get (G_in - base_in) added when they are written out
-        if (ffirst != 0x7FFFFFFF && c0 <= ffirst && ffirst < c0 + n) sc.nbf = tp + __popc(E & mask_lt(ffirst - c0));
-        if (want_spans) {
-            // one (start, end) pair per token; end = next split (a string start is always a split).
-            // splits that may end a token of this tile: owned ones, plus (closed range) the string start right after it
-            const uint32_t SPq = SPLIT & mask_lt(n) & range_mask(c0, c_lo, closed ? c_hi + 1 : c_hi);
-            const int myfirst = SPq ? c0 + __ffs(SPq) - 1 : -1;
-            const unsigned hs = __ballot_sync(FULL, myfirst >= 0);
-            {
-                const int wf = __shfl_sync(FULL, myfirst, hs ? __ffs(hs) - 1 : 0);
-                if (lane == 0) scratch[160 + warp] = hs ? wf : -1;
-            }
-            CBAR();  // (H)
-            int nextsplit;     // tile index of the first split in the following threads (-1: none in this window)
-            {
-                const unsigned above = lane == 31 ? 0u : (hs & (0xFFFFFFFFu << (lane + 1)));
-                const int got = __shfl_sync(FULL, myfirst, above ? __ffs(above) - 1 : 0);
-                nextsplit = above ? got : -1;
-                if (!above) for (int w2 = warp + 1; w2 < NWARP; ++w2) if (scratch[160 + w2] >= 0) { nextsplit = scratch[160 + w2]; break; }
-            }
-            int2 *stage = span_global ? span_scratch + (size_t)scur * SPAN_SCRATCH : spanS + 1;
-            uint32_t ev = E;
-            int rank = 0;
-            int cbase = lf_excl >= 0 ? lf_excl : c_lo;       // idx = c - cbase (relative to c_lo until a string starts)
-            while (ev) {
-                const int i = __ffs(ev) - 1; ev &= ev - 1;
-                const uint32_t fb = Fm & OWN & mask_lt(i + 1);
-                if (fb) cbase = c0 + 31 - __clz(fb);
-                const uint32_t ab = (i == 31) ? 0u : (SPq & (0xFFFFFFFEu << i));
-                const int endc = ab ? c0 + __ffs(ab) - 1 : nextsplit;
-                const int sidx = c0 + i - (((SPLIT >> i) & 1u) ? 0 : 1) - cbase;
-                const int eidx = endc >= 0 ? endc - cbase : -1;
-                stage[tp + rank] = make_int2(sidx, eidx);
-                ++rank;
-            }
-            // the first split of the tile that follows a non-space character ends the token left open by earlier tiles
-            {
-                const uint32_t PSr = (Sraw << 1) | ((LB >> 3) & 1u);
-                // (in the last tile the end-of-data terminator counts: it ends the last token of the data)
-                const uint32_t END = SPLIT & ~PSr & mask_lt(n) & range_mask(c0, c_lo, last_tile ? c_hi + 1 : c_hi);
-                if (END) {
-                    const int i = __ffs(END) - 1;
-                    if (tp + __popc(E & mask_lt(i)) == 0) {
-                        const uint32_t fb = Fm & OWN & mask_lt(i);      // string starts strictly before the split
-                        const bool rel = !fb && lf_excl < 0;
-                        const int cb = fb ? c0 + 31 - __clz(fb) : (lf_excl >= 0 ? lf_excl : c_lo);
-                        sc.end0 = c0 + i - cb; sc.end0_rel = rel ? 1 : 0;
-                    }
-                }
-            }
-        }
-        // split values -> bytes -> staging buffer at VPAD + (tile character index - c_lo)
-        if (want_splits) {
-            uint32_t W[8];
-            if (kDefault) {
-                const uint32_t qlo = (V[0] & 0x0F0F0F0Fu) | ((V[1] & 0x0F0F0F0Fu) << 4);
-                const uint32_t qhi = ((V[0] >> 4) & 0x0F0F0F0Fu) | (V[1] & 0xF0F0F0F0u);
-#pragma unroll
-                for (int g = 0; g < 4; ++g) {
-                    W[2 * g] = lutv[(qlo >> (8 * g)) & 0xFFu];
-                    W[2 * g + 1] = lutv[(qhi >> (8 * g)) & 0xFFu];
-                }
-                if (V[2]) {
-#pragma unroll
-                    for (int g = 0; g < 8; ++g) W[g] += spread4((V[2] >> (4 * g)) & 15u) << 2;
-                }
-            } else {
-#pragma unroll
-                for (int g = 0; g < 8; ++g) {
-                    uint32_t w = 0;
-#pragma unroll
-                    for (int b = 0; b < 5; ++b) w += spread4((V[b] >> (4 * g)) & 15u) << b;
-                    W[g] = w;
-                }
-            }
-            uint32_t tailw = 0;       // the last 4 characters of this thread, for the next thread's first word
-            if (n >= 4) {
-                const int sft = n - 4;
-#pragma unroll
-                for (int b = 0; b < 5; ++b) tailw += spread4((V[b] >> sft) & 15u) << b;
-            }
-            uint32_t headw = __shfl_up_sync(FULL, tailw, 1);
-            if (lane == 31) edgeS[warp * 16 + 9] = tailw;
-            CBAR();  // (I0)
-            if (lane == 0) headw = warp > 0 ? edgeS[(warp - 1) * 16 + 9] : 0u;
-            const int o = VPAD + c0 - c_lo;                 // staging offset of this thread's first character
-            if (tid >= FIRST_OWNED_THREAD && o >= 4 && n > 0) {
-                if (!slow) {
-                    // words are written by the thread that owns their LAST byte: no partial words, no races
-                    const int s = o & 3;
-                    const int cnt = (s + n) >> 2;
-                    uint32_t *dst = reinterpret_cast<uint32_t *>(valS) + (o >> 2);
-                    const int sh = 32 - 8 * s;
-                    uint32_t prev = headw;
-#pragma unroll
-                    for (int i = 0; i < 8; ++i) {
-                        const uint32_t w = s ? __funnelshift_r(prev, W[i], sh) : W[i];
-                        if (i < cnt) dst[i] = w;
-                        prev = W[i];
-                    }
-                    if (8 < cnt) dst[8] = __funnelshift_r(prev, 0u, sh);
-                    // the thread that holds the last owned character flushes the trailing partial word byte by byte
-                    if (c0 < c_hi && c0 + n >= c_hi) {
-                        const int end = VPAD + n_own;
-                        for (int q = end & ~3; q < end; ++q) {
-                            const int j = q - o;
-                            const uint32_t src = j >= 0 ? W[j >> 2] >> ((j & 3) * 8) : headw >> ((4 + j) * 8);
-                            valS[q] = (uint8_t)(src & 0xFFu);
-                        }
-                    }
-                } else {
-                    for (int j = 0; j < n; ++j) {
-                        uint32_t v = 0;
-#pragma unroll
-                        for (int b = 0; b < 5; ++b) v |= ((V[b] >> j) & 1u) << b;
-                        valS[o + j] = (uint8_t)v;
-                    }
-                }
-            }
-        }
-        if (kFeats) {
-            // this thread's open tail: its owned characters from its last split on (all of them if it holds none)
-            const int low = max(c_lo - c0, 0), high = min(n, c_hi - c0);
-            const uint32_t rng = high > low ? (mask_lt(high) & ~mask_lt(low)) : 0u;
-            const uint32_t spl = SPLIT & rng;
-            const uint32_t frag = spl ? (rng & ~mask_lt(31 - __clz(spl))) : rng;
-            unsigned tl[7] = {0, 0, 0, 0, 0, 0, 0};
-            plane_sums(frag, tl);
-            *reinterpret_cast<uint4 *>(tailS + tid * 8) = make_uint4(tl[0], tl[1], tl[2], tl[3]);
-            *reinterpret_cast<uint4 *>(tailS + tid * 8 + 4) = make_uint4(tl[4], tl[5], tl[6], spl ? 1u : 0u);
-            CBAR();
-            if (tid == 0) { publish_open_sums(); __threadfence(); }
-        }
-        if (tid == 0) {
-            Slot &sl = slots[scur];
-            sl.tile = tile; sl.c_lo = c_lo; sl.c_hi = c_hi; sl.n_own = n_own; sl.ntok = ntok_tile; sl.last_tile = last_tile ? 1 : 0;
-            sl.lft_rel = lft >= 0 ? lft - c_lo : -1;
-            sl.span_global = span_global ? 1 : 0;
-        }
-        CBAR();  // (I) staging complete; sc.* final
-        if (tid == 0) {
-            Slot &sl = slots[scur];
-            sl.v_tile = sc.v_tile; sl.nbf = sc.nbf >= 0 ? sc.nbf : ntok_tile; sl.end0 = sc.end0; sl.end0_rel = sc.end0_rel;
-        }
-        PROF(4);
-        if (kFeats) {
-            // token-feature mode writes its rows with the prefix in hand (this mode is not pipelined)
-            // (named barriers count whole warps: re-converge first, thread 0 has just done single-thread work)
-            if (!is_redo) { __syncwarp(); nb_arrive(BAR_AGG + scur, NTHREADS); nb_sync(BAR_PRE + scur, NTHREADS); }
-            const bool need_redo = !is_redo && slots[scur].redo != 0;
-            if (!need_redo) {
-                const unsigned long long K_in = slots[scur].K_in;
-        if (kFeats) {
-            // every split that follows a non-space character ends a token: sum the feature planes back to its start
-            const uint32_t PSr = (Sraw << 1) | ((LB >> 3) & 1u);
-            uint32_t ev = SPLIT & ~PSr & mask_lt(n) & range_mask(c0, c_lo, last_tile ? c_hi + 1 : c_hi);
-            while (ev) {
-                const int i = __ffs(ev) - 1; ev &= ev - 1;
-                const long long k = (long long)K_in + tp + __popc(E & mask_lt(i)) - 1;
-                if (k < 0 || k >= p.cap_tokens) continue;
-                unsigned acc[7] = {0, 0, 0, 0, 0, 0, 0}; bool hit;
-                // the token's characters inside this thread's word: one population count per feature plane
-                {
-                    const int low = max(c_lo - c0, 0);
-                    const uint32_t below = SPLIT & mask_lt(i) & ~mask_lt(low);
-                    hit = below != 0u;
-                    const int sfrom = hit ? 31 - __clz(below) : low;
-                    plane_sums(mask_lt(i) & ~mask_lt(sfrom), acc);
-                }
-                if (!hit) walk_threads(tid - 1, acc, hit);             // it began in an earlier thread: add the open tails
-                for (long long t = tile - 1; !hit && t >= 0; --t) {      // token began in an earlier tile
-                    const uint4 *o = reinterpret_cast<const uint4 *>(p.osum + t);
-                    const uint4 a = ld_rec(o), b = ld_rec(o + 1), c4 = ld_rec(o + 2);
-                    acc[0] = __vadd4(acc[0], b.x); acc[1] = __vadd4(acc[1], b.y); acc[2] = __vadd4(acc[2], b.z);
-                    acc[3] = __vadd4(acc[3], b.w); acc[4] = __vadd4(acc[4], c4.x); acc[5] = __vadd4(acc[5], c4.y);
-                    acc[6] = __vadd4(acc[6], c4.z);
-                    hit = a.x != 0u;
-                }
-                // the 25-byte row starts at byte 25 k: whole words where they are ours alone, single bytes at the two ends
-                int8_t *row = p.feats + k * NFEAT;
-                const int head = (int)((0u - (unsigned)(k & 3)) & 3u);      // bytes in front of the first 4-byte boundary
-                auto put = [&](int hb) {                                     // hb = head, a compile-time constant per call
-                    for (int q = 0; q < hb; ++q) row[q] = (int8_t)((acc[0] >> (8 * q)) & 0xFFu);
-                    const int nw = (NFEAT - hb) >> 2;
-                    uint32_t *w = reinterpret_cast<uint32_t *>(row + hb);
-#pragma unroll
-                    for (int j = 0; j < 6; ++j)
-                        if (j < nw) w[j] = hb ? __funnelshift_r(acc[j], acc[j + 1], 8 * hb) : acc[j];
-                    for (int q = hb + 4 * nw; q < NFEAT; ++q) row[q] = (int8_t)((acc[q >> 2] >> (8 * (q & 3))) & 0xFFu);
-                };
-                if (head == 0) put(0); else if (head == 1) put(1); else if (head == 2) put(2); else put(3);
-            }
-        }
-
-            }
-        }
-        }  // have_work
-
-        if (is_redo) {
-            // publish the exact inclusive prefix of the recomputed tile, then write it out
-            if (tid == 0) {
-                Slot &sl = slots[scur];
-                IncRec *ir = p.inc + sl.tile;
-                uint4 a, bq;
-                const unsigned long long Gn = sl.G_in + (unsigned long long)sl.n_own, Kn = sl.K_in + (unsigned long long)sl.ntok;
-                const unsigned long long Bn = sl.lft_rel >= 0 ? sl.G_in + (unsigned long long)sl.lft_rel : sl.base_in;
-                a.x = (unsigned)Gn; a.y = (unsigned)(Gn >> 32); a.z = (unsigned)Bn; a.w = (unsigned)(Bn >> 32);
-                bq.x = (unsigned)Kn; bq.y = (unsigned)(Kn >> 32); bq.z = (unsigned)sl.v_tile; bq.w = 0;
-                st_rec(ir, a); st_rec(reinterpret_cast<uint4 *>(ir) + 1, bq);
-                __threadfence();
-                uint4 r = ld_rec(p.agg + sl.tile);
-                r.x = (p.epoch << 2) | 2u;
-                st_rec(p.agg + sl.tile, r);
-            }
-            emit(scur, bcur);
-            CBAR();
-            nb_arrive(BAR_FREE + bcur, NTHREADS);
-            redo_k = -1;
-            if (drained) break;
-            continue;
-        }
-        int j;   // tile whose outputs are written now
-        if (have_work) {
-            if (!kFeats) { __syncwarp(); nb_arrive(BAR_AGG + scur, NTHREADS); }
-            j = kSync ? k : k - 1;
-            ++k;
-        } else { j = kSync ? -1 : k - 1; drained = true; }
-        if (j >= 0) {
-            if (!kFeats) nb_sync(BAR_PRE + (j & 1), NTHREADS);
-            if (slots[j & 1].redo) { redo_k = j; continue; }
-            emit(j & 1, j % NBUF);
-            CBAR();
-            nb_arrive(BAR_FREE + j % NBUF, NTHREADS);
-        }
-        PROF(5);
-        if (drained) break;
+        const int np = lane + utf8_len(b), ap = np + utf8_len(at(b, xb, np));     // next and after-next character
+        const uint32_t nw = at(cw, xw, np), aw = at(cw, xw, ap);
+        const unsigned below = leads & mask_lt(lane), xbelow = xleads & 0xF00u;
+        const uint32_t pin = __shfl_sync(FULL, cw, below ? 31 - __clz(below) : 0);
+        const uint32_t pout = __shfl_sync(FULL, xw, xbelow ? 31 - __clz(xbelow) : 0);
+        const unsigned long long S = starts[w] | (w + 1 < nwords ? (unsigned long long)starts[w + 1] << 32 : 0ull);
+        const bool F = (S >> lane) & 1u, L = (S >> np) & 1u, L2 = (S >> ap) & 1u;
+        if (lead) rows[__popc(below)] = make_word(below ? pin : pout, cw, nw, aw, F, L, L2);
+        __syncwarp();
+        int8_t *dst = matrix + (group_pref[w / TB_GROUP] + word_local[w]) * NFEAT;
+        for (int i = lane; i < __popc(leads) * NFEAT; i += 32) dst[i] = (int8_t)((rows[i / NFEAT] >> (i % NFEAT)) & 1u);
+        __syncwarp();
     }
 }
 
-template <bool kDefault, bool kWords, bool kFeats>
-static cudaError_t launch_one(const Params &p, int grid, cudaStream_t s)
+cudaError_t launch_parse_matrix(const uint8_t *in, long long n_bytes, const long long *offsets, long long n_strings,
+                                uint32_t *starts, const unsigned *word_local, const unsigned long long *group_pref,
+                                const uint8_t *table_blob, const TableLayout &tl, int8_t *matrix, const Result *result,
+                                int n_sm, cudaStream_t s)
 {
-    const size_t smem = tokenize_smem_bytes(p.tl, kWords, kFeats);
-    static size_t configured = 0;
-    if (configured < smem) {
-        cudaError_t e = cudaFuncSetAttribute(tokenize_kernel<kDefault, kWords, kFeats>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return e;
-        configured = smem;
-    }
-    tokenize_kernel<kDefault, kWords, kFeats><<<grid, NTHREADS, smem, s>>>(p);
+    const long long nwords = n_bytes / TB_WORD + 1;
+    if (cudaError_t e = cudaMemsetAsync(starts, 0, (size_t)nwords * sizeof(uint32_t), s)) return e;
+    string_starts_kernel<<<(unsigned)((n_strings + 256) / 256), 256, 0, s>>>(offsets, n_strings, starts, result);
+    const long long want = (nwords + PM_WARPS - 1) / PM_WARPS, cap = (long long)n_sm * 8;
+    parse_matrix_kernel<<<(unsigned)(want < cap ? want : cap), PM_WARPS * 32, 0, s>>>(in, n_bytes, starts, word_local, group_pref,
+                                                                                    table_blob, tl, matrix, result);
     return cudaGetLastError();
-}
-
-template <bool kDefault, bool kWords, bool kFeats>
-static int ctas_one(const TableLayout &tl)
-{
-    int nb = 0;
-    const size_t smem = tokenize_smem_bytes(tl, kWords, kFeats);
-    cudaFuncSetAttribute(tokenize_kernel<kDefault, kWords, kFeats>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, tokenize_kernel<kDefault, kWords, kFeats>, NTHREADS, smem) != cudaSuccess) { cudaGetLastError(); return 1; }
-    return nb < 1 ? 1 : nb;
-}
-
-// v4 runs the token-feature (kFeats) and matrix (kWords) modes; the plain mode is kept for comparison (LATOK_B200_FORCE_V4)
-int tokenize_ctas_per_sm(const TableLayout &tl, bool is_default, bool want_words, bool want_feats)
-{
-    if (is_default) {
-        if (want_words) return want_feats ? ctas_one<true, true, true>(tl) : ctas_one<true, true, false>(tl);
-        return want_feats ? ctas_one<true, false, true>(tl) : ctas_one<true, false, false>(tl);
-    }
-    if (want_words) return want_feats ? ctas_one<false, true, true>(tl) : ctas_one<false, true, false>(tl);
-    return want_feats ? ctas_one<false, false, true>(tl) : ctas_one<false, false, false>(tl);
-}
-
-cudaError_t launch_tokenize(const Params &p, int grid, cudaStream_t s)
-{
-    const bool words = (p.what & 8u) != 0u, feats = (p.what & 4u) != 0u;
-    if (p.rules.is_default) {
-        if (words) return feats ? launch_one<true, true, true>(p, grid, s) : launch_one<true, true, false>(p, grid, s);
-        return feats ? launch_one<true, false, true>(p, grid, s) : launch_one<true, false, false>(p, grid, s);
-    }
-    if (words) return feats ? launch_one<false, true, true>(p, grid, s) : launch_one<false, true, false>(p, grid, s);
-    return feats ? launch_one<false, false, true>(p, grid, s) : launch_one<false, false, false>(p, grid, s);
 }
 
 // =====================================================================================================

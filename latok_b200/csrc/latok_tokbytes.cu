@@ -8,6 +8,7 @@
 //   lead_count_kernel   characters (non-continuation bytes) per 32-byte word, as an exclusive prefix inside each
 //                       group of 4096 words + one total per group (reads B, writes B/8)
 //   group_scan_kernel   exclusive prefix of the group totals (one CTA)
+//                       (these two are launch_char_prefix, which the parse matrix of latok_kernels.cu uses too)
 //   token_bytes_kernel  one lane per token: ASCII-only strings map index -> byte directly; other strings find the
 //                       word by a galloping search on the prefix and the byte by a select on the word's lead mask
 // All three are HBM/L2-bound integer kernels; no tensor cores.
@@ -15,8 +16,6 @@
 
 namespace latok {
 
-constexpr int TB_WORD = 32;              // bytes per counted word (one 32-bit lead mask)
-constexpr int TB_GROUP = 4096;           // words per CTA of lead_count_kernel (128 KB of text)
 constexpr int TB_CHUNK = 16;             // blocks of 32 tokens per warp visit (one string search per chunk)
 
 // bit j = byte j of the 32-byte word at `pos` begins a character (is not a UTF-8 continuation byte 10xxxxxx);
@@ -251,15 +250,22 @@ __global__ void __launch_bounds__(256) token_bytes_kernel(const TokBytesParams p
     }
 }
 
-cudaError_t launch_token_bytes(const uint8_t *in, long long n_bytes, const long long *offsets, const long long *char_off,
-                               const long long *tok_off, long long n_strings, long long n_tokens, const int32_t *spans,
-                               long long *out, unsigned *word_local, unsigned *group_tot, unsigned long long *group_pref,
-                               const uint8_t *table_blob, const TableLayout &tl, int n_sm, cudaStream_t s)
+cudaError_t launch_char_prefix(const uint8_t *in, long long n_bytes, unsigned *word_local, unsigned *group_tot,
+                               unsigned long long *group_pref, cudaStream_t s)
 {
-    const long long nwords = token_bytes_words(n_bytes), ngroups = token_bytes_groups(n_bytes);
-    if (n_strings == 0 || n_tokens == 0) return cudaSuccess;
+    const long long nwords = char_prefix_words(n_bytes), ngroups = char_prefix_groups(n_bytes);
     lead_count_kernel<<<(unsigned)ngroups, 1024, 0, s>>>(in, n_bytes, nwords, word_local, group_tot);
     group_scan_kernel<<<1, 1024, 0, s>>>(group_tot, ngroups, group_pref);
+    return cudaGetLastError();
+}
+
+// after launch_char_prefix on the same stream
+cudaError_t launch_token_bytes(const uint8_t *in, long long n_bytes, const long long *offsets, const long long *char_off,
+                               const long long *tok_off, long long n_strings, long long n_tokens, const int32_t *spans,
+                               long long *out, const unsigned *word_local, const unsigned long long *group_pref,
+                               const uint8_t *table_blob, const TableLayout &tl, int n_sm, cudaStream_t s)
+{
+    if (n_strings == 0 || n_tokens == 0) return cudaSuccess;
     TokBytesParams p;
     p.in = in; p.n_bytes = n_bytes; p.offsets = offsets; p.char_off = char_off; p.tok_off = tok_off;
     p.n_strings = n_strings; p.n_tokens = n_tokens;
@@ -271,7 +277,7 @@ cudaError_t launch_token_bytes(const uint8_t *in, long long n_bytes, const long 
     return cudaGetLastError();
 }
 
-long long token_bytes_words(long long n_bytes) { return n_bytes / TB_WORD + 1; }
-long long token_bytes_groups(long long n_bytes) { return (token_bytes_words(n_bytes) + TB_GROUP - 1) / TB_GROUP; }
+long long char_prefix_words(long long n_bytes) { return n_bytes / TB_WORD + 1; }
+long long char_prefix_groups(long long n_bytes) { return (char_prefix_words(n_bytes) + TB_GROUP - 1) / TB_GROUP; }
 
 }  // namespace latok

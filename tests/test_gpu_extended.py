@@ -69,7 +69,8 @@ def test_one_separator_drifting_through_long_strings(engine, sep):
 
 
 def test_token_bytes_around_words_and_groups(engine):
-    # token byte ranges: multi-byte strings around the 32-byte words and the 128 KB scan groups of latok_tokbytes.cu
+    # token byte ranges and the parse matrix: multi-byte strings around the 32-byte words and the 128 KB scan groups of
+    # the character prefix (latok_tokbytes.cu)
     from latok_b200.core.default_tokenizer import tokenize_packed
     from latok_b200.engine import pack_strings
     rng = np.random.default_rng(9)
@@ -80,6 +81,8 @@ def test_token_bytes_around_words_and_groups(engine):
     pt = tokenize_packed(*pack_strings(texts), engine=engine)
     for i, t in enumerate(texts):
         assert pt.tokens(i) == oracle.tokens(t), i
+    # the parse matrix uses the same per-word character prefix (and one warp per 32-byte word)
+    check_batch(engine, texts, 15, label="words and groups")
 
 
 def test_tokens_spanning_whole_ranges_and_tiles(engine):

@@ -12,9 +12,10 @@ from oracle import oracle
 pytestmark = pytest.mark.gpu
 
 ALL = 1 | 2 | 4 | 8
-# bytes owned per unit of work (latok_internal.h): a v5 range (one warp) and a v5 tile (the ranges of one CTA, one
-# look-back record) in both geometries of the kernel (long strings: 3 968-byte ranges x 9, short strings: 2 944 x 11),
-# and a v4 tile (matrix mode); tests place interesting things around multiples of each
+# bytes owned per unit of work (latok_internal.h): a range (one warp) and a tile (the ranges of one CTA, one look-back
+# record) in both geometries of the tokenize kernel (long strings: 3 968-byte ranges x 9, short strings: 2 944 x 11);
+# tests place interesting things around multiples of each, and around 7 936 bytes, a size that cuts ranges at
+# other phases
 RANGES = (3968, 2944)
 UNITS = (3968, 7936, 9 * 3968, 2944, 11 * 2944)
 TILE = 7936
@@ -39,10 +40,8 @@ def engine(request):
 
 def check_batch(engine, texts, what=ALL, rules=None, label=""):
     if (what & 12) and (what & 3):
-        # split mask + spans (+ token features) run the v5 kernel, anything with the matrix the v4 kernel: check them all
+        # the tokenize kernel has an instantiation with token features and one without: check both
         check_batch(engine, texts, what & 3, rules, label + " [splits+spans only]")
-    if (what & 8) and (what & 4):
-        check_batch(engine, texts, what & 7, rules, label + " [v5 with token features]")
     r = engine.run(texts, what)
     o = oracle.tokenize_batch(texts, rules=rules or oracle.DEFAULT_RULES, matrix=bool(what & 8), feats=bool(what & 4))
     assert r.n_chars == o["n_chars"], label
@@ -265,7 +264,7 @@ def test_bad_offsets_rejected(engine):
 def test_back_to_back_submits_alternate_index_sets(engine):
     """Several device-resident batches submitted without waiting in between (the string index of batch i+1 is built on
     an aux stream while batch i is tokenized; two index / result sets alternate): the results are those of the last one,
-    whichever kernel (v5 for split mask + spans, v4 with token features) each batch used."""
+    whichever kernel instantiation (split mask + spans, or with token features and the matrix) each batch used."""
     torch = pytest.importorskip("torch")
     from latok_b200.engine import pack_strings
     batches = [corpus.fuzz_strings(100 + i, 3000 + 700 * i, 60 + 30 * i, "mixed") for i in range(5)]

@@ -99,3 +99,18 @@ def test_config3_long_documents(engine):
     check_invariants(buf, off, r)
     assert fullcheck.compare_all(buf, off, r, target_bytes=8 << 20) == 16_000
     assert r.lookahead_walks > 0                 # the corpus does exercise the look-ahead walk
+
+
+def test_parse_matrix_past_2gb(engine):
+    """More than 86 M characters: the matrix passes 2^31 bytes (64-bit row offsets in parse_matrix_kernel).  The strings
+    whose rows lie past that byte, against the oracle."""
+    import synth
+    buf, off = synth.tweets(700_000)
+    r = engine.run_packed(buf, off, 8)
+    assert r.n_chars == int(((buf & 0xC0) != 0x80).sum()) and r.n_chars * 25 > 2 ** 31
+    first = int(np.searchsorted(r.char_offsets, 2 ** 31 // 25, side="right")) - 1       # holds the row at byte 2^31
+    raw = buf.tobytes()
+    S = len(off) - 1
+    for i in list(range(first, first + 2000)) + list(range(S - 2000, S)):
+        t = raw[off[i]:off[i + 1]].decode("utf-8")
+        assert np.array_equal(r.string_matrix(i), oracle.parse_matrix(t)), f"string {i}"
