@@ -16,8 +16,11 @@ PKG = Path(__file__).resolve().parent
 ROOT = PKG.parent
 CSRC = PKG / "csrc"
 LIB = PKG / "liblatok_b200.so"
-SOURCES = [CSRC / "latok_kernels.cu", CSRC / "latok_tok5.cu", CSRC / "latok_tokbytes.cu", CSRC / "latok_vocab.cu", CSRC / "latok_capi.cu", CSRC / "latok_reader.cpp"]
-HEADERS = [CSRC / "latok_internal.h", CSRC / "latok_bits.h", CSRC / "latok_device.cuh", ROOT / "include" / "latok_b200.h"]
+# compiled in parallel, each once; latok_tok5.cu and latok_tok5_short.cu hold the tokenize kernel's two geometries
+SOURCES = [CSRC / "latok_kernels.cu", CSRC / "latok_tok5.cu", CSRC / "latok_tok5_short.cu", CSRC / "latok_tokbytes.cu",
+           CSRC / "latok_vocab.cu", CSRC / "latok_capi.cu", CSRC / "latok_reader.cpp"]
+HEADERS = [CSRC / "latok_internal.h", CSRC / "latok_bits.h", CSRC / "latok_device.cuh", CSRC / "latok_tok5.cuh",
+           ROOT / "include" / "latok_b200.h"]
 GEN = CSRC / "_gen" / "latok_tables.h"
 RANGES = PKG / "data" / "ucd11_latok_classes.txt"
 
@@ -68,10 +71,6 @@ def _stale() -> bool:
     return any(d.stat().st_mtime > t for d in deps)
 
 
-# latok_tok5.cu is compiled a second time for the short-string geometry (see the head of that file)
-SHORT_DEFS = ["-DLATOK_V5_SHORT", "-DLATOK_V5_RS=3", "-DLATOK_V5_NW=11"]
-
-
 def build_library(force: bool = False, verbose: bool = False) -> Path:
     if not force and not _stale():
         return LIB
@@ -92,13 +91,11 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
     out = Path(os.environ.get("LATOK_B200_LIB_OUT") or LIB)
     nvcc = find_nvcc()
     with tempfile.TemporaryDirectory() as tmp:
-        jobs = [(src, [], Path(tmp) / (src.stem + ".o")) for src in SOURCES]
-        short_defs = os.environ["LATOK_SHORT_DEFS"].split() if os.environ.get("LATOK_SHORT_DEFS") else SHORT_DEFS     # (experiments)
-        jobs.append((CSRC / "latok_tok5.cu", short_defs, Path(tmp) / "latok_tok5_short.o"))
+        jobs = [(src, Path(tmp) / (src.stem + ".o")) for src in SOURCES]
 
         def compile_one(job):
-            src, defs, obj = job
-            cmd = [nvcc, *flags, *extra, *defs, "-c", str(src), "-o", str(obj)]
+            src, obj = job
+            cmd = [nvcc, *flags, *extra, "-c", str(src), "-o", str(obj)]
             if verbose:
                 print(" ".join(cmd))
             r = subprocess.run(cmd, capture_output=True, text=True)
@@ -111,7 +108,7 @@ def build_library(force: bool = False, verbose: bool = False) -> Path:
                 sys.stderr.write(log)
         if any(rc for rc, _ in results):
             raise subprocess.CalledProcessError(1, "nvcc -c")
-        cmd = [nvcc, *NVCC_FLAGS, *[str(o) for _, _, o in jobs], "-lz", "-o", str(out)]      # zlib: the csv.gz reader
+        cmd = [nvcc, *NVCC_FLAGS, *[str(o) for _, o in jobs], "-lz", "-o", str(out)]      # zlib: the csv.gz reader
         if verbose:
             print(" ".join(cmd))
         subprocess.run(cmd, check=True)

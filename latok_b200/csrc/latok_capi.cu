@@ -387,27 +387,17 @@ static int enqueue_char_prefix(latok_b200_engine *e, Batch &b)
 
 static int run_device(latok_b200_engine *e, Batch &b)
 {
-    // The tokenize kernel (one warp per range, a tile = the ranges of one CTA) runs in one of its two geometries: short
-    // strings (3 KB ranges, 11 compute warps per CTA) or long strings (4 KB ranges, 9 warps: fewer range boundaries
-    // inside space-free runs), by the average string length of the batch; token features: always the long one
-    // (LATOK_B200_GEOMETRY=short|long overrides).  It also gives the character counts and the offsets check of a
-    // matrix-only batch.  The parse matrix follows it on the same stream.
+    // The tokenize kernel, in the geometry its plan picks for the batch.  It also gives the character counts and the
+    // offsets check of a matrix-only batch.  The parse matrix follows it on the same stream.
     const bool feats = (b.what & LATOK_B200_FEATS) != 0;
-    bool shortg = b.n_bytes < 4096LL * (b.n_strings > 0 ? b.n_strings : 1);
-    if (feats) shortg = false;      // the token-feature instantiation lives on registers (25 planes per lane): 96 beat 24 warps per SM
-    if (const char *g = getenv("LATOK_B200_GEOMETRY")) shortg = g[0] == 's';
-    const int range5 = shortg ? tokenize5_range_bytes_short() : tokenize5_range_bytes();
-    const int nw5 = shortg ? tokenize5_ranges_per_tile_short() : tokenize5_ranges_per_tile();
-    const long long nunits = b.n_bytes / range5 + 1;
-    const long long ntiles = (nunits + nw5 - 1) / nw5;
-    const size_t plane_words = shortg ? tokenize5_plane_words_short(nunits) : tokenize5_plane_words(nunits);
-    if (int r = b.d_first.ensure((size_t)nunits + 1)) return r;
+    const Tok5Plan t5 = tokenize5_plan(b.n_bytes, b.n_strings, feats, e->tl, e->rules.is_default != 0, e->n_sm);
+    if (int r = b.d_first.ensure((size_t)t5.nranges + 1)) return r;
     // the status word of every aggregate record carries the launch epoch, so records are zeroed only when (re)allocated
     // (agg / inc / osum / planes are shared by the two sets: tokenize kernels run one after the other on one stream)
-    if ((size_t)ntiles > e->agg.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->agg.ensure((size_t)ntiles, true)) return r; }
-    if ((size_t)ntiles > e->inc.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->inc.ensure((size_t)ntiles)) return r; }
-    if (feats && (size_t)nunits > e->osum.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->osum.ensure((size_t)nunits, true)) return r; }
-    if (feats && plane_words > e->d_planes.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->d_planes.ensure(plane_words)) return r; }
+    if ((size_t)t5.ntiles > e->agg.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->agg.ensure((size_t)t5.ntiles, true)) return r; }
+    if ((size_t)t5.ntiles > e->inc.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->inc.ensure((size_t)t5.ntiles)) return r; }
+    if (feats && (size_t)t5.nranges > e->osum.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->osum.ensure((size_t)t5.nranges, true)) return r; }
+    if (feats && t5.plane_words > e->d_planes.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->d_planes.ensure(t5.plane_words)) return r; }
     if (int r = b.d_splits.ensure((size_t)b.n_bytes + 64)) return r;
     if (int r = b.d_char_off.ensure((size_t)b.n_strings + 1)) return r;
     if (int r = b.d_tok_off.ensure((size_t)b.n_strings + 1)) return r;
@@ -424,7 +414,7 @@ static int run_device(latok_b200_engine *e, Batch &b)
     Params p;
     memset(&p, 0, sizeof p);
     p.in = b.cur_in; p.n_bytes = b.n_bytes; p.offsets = b.cur_off; p.n_strings = b.n_strings;
-    p.tile_first_str = b.d_first.p; p.ntiles = ntiles; p.nranges = nunits;
+    p.tile_first_str = b.d_first.p; p.ntiles = t5.ntiles; p.nranges = t5.nranges;
     p.splits = b.d_splits.p; p.char_off = b.d_char_off.p; p.spans = b.d_spans.p; p.tok_off = b.d_tok_off.p;
     p.feats = b.d_feats.p;
     p.cap_tokens = (long long)(b.d_spans.cap / 2);
@@ -433,21 +423,18 @@ static int run_device(latok_b200_engine *e, Batch &b)
     p.ticket = &b.d_result.p->ticket; p.ticket_base = 0;
     p.result = b.d_result.p;
     p.table_blob = e->d_table.p; p.tl = e->tl; p.rules = e->rules;
-    int grid = e->n_sm * (shortg ? tokenize5_ctas_per_sm_short(e->tl, e->rules.is_default != 0, feats)
-                                 : tokenize5_ctas_per_sm(e->tl, e->rules.is_default != 0, feats));
-    if ((long long)grid > ntiles) grid = (int)ntiles;
 
     // The string index of this batch is built on the aux stream, so that with back-to-back submits it overlaps the
     // tokenize kernel of the previous batch (the two sets alternate).
     if (b.inputs_on_stream) CU(cudaStreamWaitEvent(e->aux, b.ev_h2d, 0));    // host submit: the offsets arrive on the copy-in stream
     CU(cudaStreamWaitEvent(e->aux, b.ev_kdone, 0));            // this set's previous batch has been tokenized
     CU(cudaMemsetAsync(b.d_result.p, 0, sizeof(Result), e->aux));
-    CU(launch_tile_index(b.cur_off, b.n_strings, b.n_bytes, b.d_first.p, nunits, range5, b.d_result.p, e->aux));
+    CU(launch_tile_index(b.cur_off, b.n_strings, b.n_bytes, b.d_first.p, t5.nranges, t5.range_bytes, b.d_result.p, e->aux));
     CU(cudaEventRecord(b.ev_index, e->aux));
     if (b.inputs_on_stream) CU(cudaStreamWaitEvent(e->stream, b.ev_h2d, 0));
     CU(cudaStreamWaitEvent(e->stream, b.ev_index, 0));
     CU(cudaEventRecord(b.ev_k0, e->stream));
-    CU(shortg ? launch_tokenize5_short(p, grid, e->stream) : launch_tokenize5(p, grid, e->stream));
+    CU(launch_tokenize5(t5, p, e->stream));
     CU(cudaEventRecord(b.ev_k1, e->stream));
     e->launches += 2;
     if (b.what & LATOK_B200_MATRIX) {

@@ -1,4 +1,4 @@
-// latok_device.cuh -- device helpers shared by the kernels (latok_tok5.cu: tokenize; latok_kernels.cu: parse matrix;
+// latok_device.cuh -- device helpers shared by the kernels (latok_tok5.cuh: tokenize; latok_kernels.cu: parse matrix;
 // latok_tokbytes.cu: token byte ranges): PTX wrappers, Unicode class look-up, the context features, the scalar rule
 // evaluation used on rare paths, the look-ahead walk and the decoupled look-back.
 #pragma once
@@ -242,10 +242,7 @@ static __device__ bool walk_ahead(const Params &p, const Tables &t, long long po
 // =====================================================================================================
 // Decoupled look-back (single chain, 16-byte aggregate records, LB_WINDOW predecessors per step)
 // =====================================================================================================
-#ifndef LATOK_LB_PER_LANE
-#define LATOK_LB_PER_LANE 2
-#endif
-constexpr int LB_PER_LANE = LATOK_LB_PER_LANE;
+constexpr int LB_PER_LANE = 2;
 constexpr int LB_WINDOW = 32 * LB_PER_LANE;
 
 __device__ __forceinline__ uint4 ld_rec(const void *p)

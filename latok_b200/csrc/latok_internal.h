@@ -1,4 +1,4 @@
-// Internal structures shared by the kernels (latok_tok5.cu, latok_kernels.cu, latok_tokbytes.cu, latok_vocab.cu) and
+// Internal structures shared by the kernels (latok_tok5.cuh, latok_kernels.cu, latok_tokbytes.cu, latok_vocab.cu) and
 // the C-ABI host layer (latok_capi.cu).
 #pragma once
 #include "_gen/latok_table_types.h"   // latok_stage1_t (8 bits for UCD 11, 16 when a newer UCD needs more than 256 blocks)
@@ -6,22 +6,6 @@
 #include <stdint.h>
 
 namespace latok {
-
-// v5 kernel (latok_tok5.cu): one warp analyses a "range" (V5_RS steps of 1 KB, the last V5_HALO bytes shared with the
-// next range), a tile is the V5_NW ranges of one CTA
-#ifndef LATOK_V5_RS
-#define LATOK_V5_RS 4
-#endif
-#ifndef LATOK_V5_CTAS
-#define LATOK_V5_CTAS 2
-#endif
-constexpr int V5_RS = LATOK_V5_RS;
-constexpr int V5_HALO = 128;
-constexpr int V5_RANGE = V5_RS * 1024 - V5_HALO;
-#ifndef LATOK_V5_NW
-#define LATOK_V5_NW 9
-#endif
-constexpr int V5_NW = LATOK_V5_NW;
 
 constexpr int NFEAT = 25;
 constexpr int MAX_RULE_ROWS = 15;
@@ -86,7 +70,7 @@ struct Params {
     long long n_strings;
     const long long *tile_first_str;  // [ntiles + 1]
     long long ntiles;
-    long long nranges;                // v5: tile_first_str is indexed by range, ntiles counts groups of V5_NW ranges
+    long long nranges;                // tile_first_str is indexed by range, ntiles counts tiles (Tok5Plan)
     int8_t *splits;
     long long *char_off;
     int32_t *spans;
@@ -107,17 +91,17 @@ struct Params {
     RuleSet rules;
 };
 
-// the v5 kernel exists in two geometries (latok_tok5.cu is compiled twice): long strings / short strings (_short)
-int tokenize5_range_bytes();
-int tokenize5_ranges_per_tile();
-int tokenize5_ctas_per_sm(const TableLayout &tl, bool is_default, bool want_feats);
-size_t tokenize5_plane_words(long long nranges);
-cudaError_t launch_tokenize5(const Params &p, int grid, cudaStream_t s);
-int tokenize5_range_bytes_short();
-int tokenize5_ranges_per_tile_short();
-int tokenize5_ctas_per_sm_short(const TableLayout &tl, bool is_default, bool want_feats);
-size_t tokenize5_plane_words_short(long long nranges);
-cudaError_t launch_tokenize5_short(const Params &p, int grid, cudaStream_t s);
+// The tokenize kernel (latok_tok5.cu): one warp analyses a range of the text, a tile is the ranges of one CTA.  The plan
+// picks the kernel's geometry for a batch and sizes its work; the launch runs that geometry.
+struct Tok5Plan {
+    bool short_geometry;
+    int range_bytes;          // bytes from one range's start to the next's (launch_tile_index)
+    long long nranges, ntiles;
+    size_t plane_words;       // token-feature planes (Params::planes)
+    int grid;                 // CTAs: ctas_per_sm x SMs, at most ntiles
+};
+Tok5Plan tokenize5_plan(long long n_bytes, long long n_strings, bool feats, const TableLayout &tl, bool is_default, int n_sm);
+cudaError_t launch_tokenize5(const Tok5Plan &plan, const Params &p, cudaStream_t s);
 cudaError_t launch_tile_index(const long long *offsets, long long n_strings, long long n_bytes,
                               long long *tile_first_str, long long ntiles, int tile_bytes, Result *result, cudaStream_t s);
 cudaError_t launch_block_mask(const int8_t *a1, long long s1, const int8_t *a2, long long s2, long long n,

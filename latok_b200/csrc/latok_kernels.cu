@@ -7,7 +7,7 @@
 //   block_mask_kernel     stand-alone _gen_block_mask
 //   combine_rows_kernel   stand-alone _combine_matrix_rows
 //
-// The tokenize kernel itself (split mask, spans, CSR offsets, token features) is in latok_tok5.cu.
+// The tokenize kernel itself (split mask, spans, CSR offsets, token features) is in latok_tok5.cuh.
 // No tensor cores: nothing here is a dense contraction.
 #include "latok_device.cuh"
 

@@ -101,7 +101,7 @@ def test_tokens_spanning_whole_ranges_and_tiles(engine):
 
 def test_token_feature_rows_in_ordinal_order(engine):
     """Token-feature rows are written in the order of the token ordinals, 32 per trip, staged at their byte phase
-    (latok_tok5.cu, token-feature mode): steps with few, many and more than 512 token ends (the per-lane fallback),
+    (latok_tok5.cuh, token-feature mode): steps with few, many and more than 512 token ends (the per-lane fallback),
     the 25-byte rows at every phase of a 16-byte chunk, tokens longer than 255 characters (uint8 wrap-around of the
     sums, latok.c:342-354), tokens that begin several lane-words / steps / ranges before they end."""
     RANGE, _ = engine.geometry

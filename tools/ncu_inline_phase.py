@@ -1,22 +1,22 @@
 #!/usr/bin/env python3
-"""Executed warp-instructions and stall samples of the v5 tokenize kernel per PHASE and per SOURCE LINE of latok_tok5.cu,
-with inlined helpers (latok_bits.h, latok_device.cuh, CUDA intrinsics headers) charged to the line of latok_tok5.cu
+"""Executed warp-instructions and stall samples of the v5 tokenize kernel per PHASE and per SOURCE LINE of latok_tok5.cuh,
+with inlined helpers (latok_bits.h, latok_device.cuh, CUDA intrinsics headers) charged to the line of latok_tok5.cuh
 that called them.  ncu's own source page charges an instruction to the innermost inlined function only.
 
     python tools/ncu_inline_phase.py <rep.ncu-rep> <kernel-substring> <input bytes> [first-line last-line]
-        kernel-substring  e.g. tokenize5_kernelILb1ELb0 (split mask + spans), ...ILb1ELb1 (with token features);
-                          prefix v5s / v516 picks the short / long geometry
+        kernel-substring  e.g. Lb1ELb0E (default rules: split mask + spans), Lb1ELb1E (with token features)
         LATOK_SHORT=0     the report is of the long geometry (4 KB ranges); default: short (3 KB ranges)
 
-How: the file is compiled to a cubin with the library's flags, `nvdisasm -gi` gives every SASS instruction its chain of
-inlined call sites, and the n-th instruction of the kernel in the disassembly is the n-th row of
-`ncu --page source --print-source sass` (checked: same count, same opcodes).  The source must be the one the profiled
-library was built from."""
+How: the translation unit of that geometry (latok_tok5_short.cu or latok_tok5.cu) is compiled to a cubin with the
+library's flags, `nvdisasm -gi` gives every SASS instruction its chain of inlined call sites, and the n-th instruction of
+the kernel in the disassembly is the n-th row of `ncu --page source --print-source sass` (checked: same count, same
+opcodes).  The source must be the one the profiled library was built from."""
 import collections, csv, os, re, subprocess, sys, tempfile
 from pathlib import Path
 
 ROOT = Path(__file__).resolve().parent.parent
-SRC = ROOT / "latok_b200" / "csrc" / "latok_tok5.cu"
+CSRC = ROOT / "latok_b200" / "csrc"
+SRC = CSRC / "latok_tok5.cuh"
 rep, kern, nbytes = sys.argv[1], sys.argv[2], float(sys.argv[3])
 lohi = (int(sys.argv[4]), int(sys.argv[5])) if len(sys.argv) > 5 else None
 short = os.environ.get("LATOK_SHORT", "1") != "0"
@@ -24,9 +24,9 @@ RS = 3 if short else 4
 NSTEP = nbytes / (RS * 1024 - 128) * RS                   # warp-steps (1 KB each) per launch
 
 tmp = Path(tempfile.mkdtemp())
-defs = ["-DLATOK_V5_SHORT", "-DLATOK_V5_RS=3", "-DLATOK_V5_NW=11"] if short else []
-subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", *defs, "-cubin",
-                "-o", str(tmp / "k.cubin"), str(SRC)], check=True, capture_output=True)
+tu = CSRC / ("latok_tok5_short.cu" if short else "latok_tok5.cu")
+subprocess.run(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-std=c++17", "-lineinfo", "-cubin",
+                "-o", str(tmp / "k.cubin"), str(tu)], check=True, capture_output=True)
 sass = subprocess.run(["nvdisasm", "-gi", "-c", str(tmp / "k.cubin")], check=True, capture_output=True, text=True).stdout.split("\n")
 start = end = None
 for i, l in enumerate(sass):
@@ -61,12 +61,12 @@ src = SRC.read_text().split("\n")
 calls = {i + 1 for i, l in enumerate(src) if re.search(r"\b(analyze|output|finish_tile|begin_load)\(", l) and "auto " not in l}
 by, sm, ops, st = collections.Counter(), collections.Counter(), collections.defaultdict(collections.Counter), collections.defaultdict(collections.Counter)
 for (ch, op), r in zip(recs, data):
-    tag = next((ln for f, ln in reversed(ch) if f == "latok_tok5.cu" and ln not in calls), None)
+    tag = next((ln for f, ln in reversed(ch) if f == "latok_tok5.cuh" and ln not in calls), None)
     e = int(r[iE]); by[tag] += e; sm[tag] += int(r[iS]); ops[tag][op] += e
     for n in stalls:
         v = int(r[sidx[n]] or 0)
         if v: st[n][tag] += v
-markers = [("setup", "template <bool kDefault, bool kFeats>"), ("analysis: head", "auto analyze = [&]"), ("analysis: base planes", "for (int j = 0; j <= RS; ++j) {"),
+markers = [("setup", "template <class Geom, bool kDefault, bool kFeats>"), ("analysis: head", "auto analyze = [&]"), ("analysis: base planes", "for (int j = 0; j <= RS; ++j) {"),
            ("analysis: context + rules + block mask", "context + rules of step j-1"), ("analysis: guess", "PROF5(1);"),
            ("pass C", "pass C: blanked chunks, values, tokens"), ("service warp", "// service warp: tile aggregate"),
            ("output: head + CSR", "auto output = [&]"), ("output: step head", "for (int js = 0; js < RS; ++js) {\n            const uint32_t *t = SA("),
