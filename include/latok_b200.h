@@ -169,7 +169,15 @@ LATOK_B200_API int latok_b200_vocab_export(latok_b200_vocab *v, int64_t cap_keys
  * (NULL: 0).  A key that is empty, repeated, or already in the vocabulary is EINVAL (nothing is added then). */
 LATOK_B200_API int latok_b200_vocab_import(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *bytes,
                                            const int64_t *offsets, int64_t n_keys, const int64_t *counts);
-/* device time of the last encode / import (token byte ranges included; harness) */
+/* Adds every key of src to dst with its src count: a key dst lacks gets the next id (new keys in src's id order), a
+ * key dst has gets src's count added (Counter.update(other)).  src may be on any device; e is dst's engine.
+ * map: int32 [n_keys(src)], the dst id of every src id, in host memory or (on_device != 0) in device memory on dst's
+ * device; NULL skips it.  All or nothing, as for encode.  EINVAL when src == dst or the result would pass 2^31 - 1 keys. */
+LATOK_B200_API int latok_b200_vocab_merge(latok_b200_engine *e, latok_b200_vocab *dst, const latok_b200_vocab *src,
+                                          int32_t *map, int on_device);
+/* Drops every key and count; keeps the table and arena allocations (for scratch vocabularies reused per batch). */
+LATOK_B200_API int latok_b200_vocab_clear(latok_b200_vocab *v);
+/* device time of the last encode / import / merge (token byte ranges and a merge's copy-in included; harness) */
 LATOK_B200_API int latok_b200_vocab_last_ms(latok_b200_vocab *v, float *ms);
 
 /* ---- measurement hooks (harness only) ----------------------------------------------------- */

@@ -71,6 +71,8 @@ def load():
         "latok_b200_vocab_size": (C.c_int, [vp, P(i64), P(i64), P(i64)]),
         "latok_b200_vocab_export": (C.c_int, [vp, i64, i64, vp, vp, vp]),
         "latok_b200_vocab_import": (C.c_int, [vp, vp, vp, vp, i64, vp]),
+        "latok_b200_vocab_merge": (C.c_int, [vp, vp, vp, vp, i32]),
+        "latok_b200_vocab_clear": (C.c_int, [vp]),
         "latok_b200_vocab_last_ms": (C.c_int, [vp, P(C.c_float)]),
     }
     for name, (res, args) in proto.items():

@@ -829,6 +829,7 @@ struct latok_b200_vocab {
     DevBuf<int32_t> rank;                           // per token: first-occurrence flags, then new ids, then the ids
     DevBuf<uint8_t> scan_tmp, imp_bytes;
     DevBuf<longlong2> imp_rng;
+    DevBuf<long long> imp_w;                        // a merge from another device: its counts, then its key offsets
     DevBuf<VocabStatus> st;
     PinBuf<VocabStatus> h_st;
     cudaEvent_t ev[4] = {nullptr, nullptr, nullptr, nullptr};
@@ -918,6 +919,33 @@ static int vocab_commit(latok_b200_vocab *v, const uint8_t *text, const longlong
     return 0;
 }
 
+// One batch into v (encode, import, merge): the keys text[rng[k].x, rng[k].y) (k < n, on v's device) are inserted and
+// committed, then, with `count` or ids, the count kernel writes the id of every key into ids and adds 1 per key, or
+// weight[k] with weights, to its count.  strict: every key must be new (import); otherwise nothing is committed and
+// the call is EINVAL.  Records v->ev[1] (insert done) and v->ev[2] (commit started).
+static int vocab_add(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *text, const longlong2 *rng, long long n,
+                     bool strict, bool count, const long long *weight, int32_t *ids)
+{
+    cudaStream_t s = e->stream;
+    long long n_new = 0, new_bytes = 0;
+    if (int r = vocab_insert(v, text, rng, n, e->n_sm, s, &n_new, &new_bytes)) return r;
+    if (strict && n_new != n) {
+        if (int r = vocab_rebuild(v, v->cap, e->n_sm, s)) return r;
+        CU(cudaStreamSynchronize(s));
+        return fail(LATOK_B200_EINVAL, "duplicate keys: %lld of the %lld keys are new to the vocabulary", n_new, n);
+    }
+    if (int r = vocab_commit(v, text, rng, n, n_new, new_bytes, e->n_sm, s)) return r;
+    e->launches += 5;
+    if (!count && !ids) return 0;
+    VocabParams p = vocab_params(v);
+    if (!count) p.counts = nullptr;
+    p.weight = weight; p.ids = ids;
+    p.text = text; p.rng = rng; p.n = n;
+    CU(launch_vocab(VOCAB_COUNT, p, 0, e->n_sm, s));
+    e->launches += 1;
+    return 0;
+}
+
 static float elapsed(cudaEvent_t a, cudaEvent_t b)
 {
     float ms = 0.f;
@@ -965,6 +993,7 @@ int latok_b200_vocab_destroy(latok_b200_vocab *v)
     cudaSetDevice(v->device);
     v->table.release(); v->first_occ.release(); v->arena.release(); v->key_off.release(); v->counts.release();
     v->slot.release(); v->rank.release(); v->scan_tmp.release(); v->imp_bytes.release(); v->imp_rng.release();
+    v->imp_w.release();
     v->st.release(); v->h_st.release();
     for (cudaEvent_t ev : v->ev) if (ev) cudaEventDestroy(ev);
     delete v;
@@ -993,15 +1022,9 @@ int latok_b200_vocab_encode(latok_b200_engine *e, latok_b200_vocab *v, int add, 
     const longlong2 *rng = reinterpret_cast<const longlong2 *>(e->d_tok_bytes.p);
     VocabParams p;
     if (add) {
-        long long n_new = 0, new_bytes = 0;
-        if (int r = vocab_insert(v, b.cur_in, rng, T, e->n_sm, s, &n_new, &new_bytes)) return r;
-        if (int r = vocab_commit(v, b.cur_in, rng, T, n_new, new_bytes, e->n_sm, s)) return r;
-        p = vocab_params(v);
         p.ids = ids ? (on_device ? ids : v->rank.p) : nullptr;
-        p.text = b.cur_in; p.rng = rng; p.n = T;
-        CU(launch_vocab(VOCAB_COUNT, p, 0, e->n_sm, s));
+        if (int r = vocab_add(e, v, b.cur_in, rng, T, false, true, nullptr, p.ids)) return r;
         CU(cudaEventRecord(v->ev[3], s));
-        e->launches += 6;
     } else {
         p = vocab_params(v);
         p.ids = on_device ? ids : v->rank.p;
@@ -1065,20 +1088,66 @@ int latok_b200_vocab_import(latok_b200_engine *e, latok_b200_vocab *v, const uin
     CU(cudaMemcpyAsync(v->imp_bytes.p, bytes, (size_t)nb, cudaMemcpyHostToDevice, s));
     CU(cudaMemcpyAsync(v->imp_rng.p, rng.data(), (size_t)n_keys * sizeof(longlong2), cudaMemcpyHostToDevice, s));
     CU(cudaEventRecord(v->ev[0], s));
-    long long n_new = 0, new_bytes = 0;
-    if (int r = vocab_insert(v, v->imp_bytes.p, v->imp_rng.p, n_keys, e->n_sm, s, &n_new, &new_bytes)) return r;
-    if (n_new != n_keys) {
-        if (int r = vocab_rebuild(v, v->cap, e->n_sm, s)) return r;
-        CU(cudaStreamSynchronize(s));
-        return fail(LATOK_B200_EINVAL, "duplicate keys: %lld of the %lld keys are new to the vocabulary", n_new, (long long)n_keys);
-    }
     const long long first = v->n_keys;
-    if (int r = vocab_commit(v, v->imp_bytes.p, v->imp_rng.p, n_keys, n_new, new_bytes, e->n_sm, s)) return r;
+    if (int r = vocab_add(e, v, v->imp_bytes.p, v->imp_rng.p, n_keys, true, false, nullptr, nullptr)) return r;
     if (counts) CU(cudaMemcpyAsync(v->counts.p + first, counts, (size_t)n_keys * sizeof(long long), cudaMemcpyHostToDevice, s));
     CU(cudaEventRecord(v->ev[3], s));
     CU(cudaStreamSynchronize(s));
-    e->launches += 5;
     v->last_ms = elapsed(v->ev[0], v->ev[1]) + elapsed(v->ev[2], v->ev[3]);
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_merge(latok_b200_engine *e, latok_b200_vocab *dst, const latok_b200_vocab *src, int32_t *map, int on_device)
+{
+    if (!e || !dst || !src) return fail(LATOK_B200_EINVAL, "engine or vocabulary is NULL");
+    if (dst->device != e->device) return fail(LATOK_B200_EINVAL, "the vocabulary is on device %d, the engine on device %d", dst->device, e->device);
+    if (src == dst) return fail(LATOK_B200_EINVAL, "a vocabulary cannot be merged into itself");
+    if (map && on_device && ((uintptr_t)map & 3u) != 0) return fail(LATOK_B200_EINVAL, "a device map must be 4-byte aligned");
+    dst->last_ms = 0.f;
+    const long long n = src->n_keys;
+    if (!n) return LATOK_B200_OK;
+    if (int r = set_device(e)) return r;
+    cudaStream_t s = e->stream;
+    CU(cudaStreamSynchronize(s));
+    if (int r = dst->imp_rng.ensure((size_t)n)) return r;
+    CU(cudaEventRecord(dst->ev[0], s));
+    // the source's keys, offsets and counts: read in place on the same device, else copied into the staging buffers
+    // (imp_w = counts [n], then key_off [n + 1]) on dst's stream.  cudaMemcpyPeerAsync needs no peer access; the
+    // source is stable while the copies run because every vocabulary call ends synchronised.
+    const uint8_t *text = src->arena.p;
+    const long long *key_off = src->key_off.p, *weight = src->counts.p;
+    if (src->device != dst->device) {
+        if (int r = dst->imp_bytes.ensure((size_t)src->key_bytes)) return r;
+        if (int r = dst->imp_w.ensure(2 * (size_t)n + 1)) return r;
+        CU(cudaMemcpyPeerAsync(dst->imp_bytes.p, dst->device, src->arena.p, src->device, (size_t)src->key_bytes, s));
+        CU(cudaMemcpyPeerAsync(dst->imp_w.p, dst->device, src->counts.p, src->device, (size_t)n * sizeof(long long), s));
+        CU(cudaMemcpyPeerAsync(dst->imp_w.p + n, dst->device, src->key_off.p, src->device, ((size_t)n + 1) * sizeof(long long), s));
+        text = dst->imp_bytes.p; weight = dst->imp_w.p; key_off = dst->imp_w.p + n;
+    }
+    CU(launch_vocab_ranges(key_off, n, dst->imp_rng.p, e->n_sm, s));
+    e->launches += 1;
+    int32_t *ids = map ? (on_device ? map : nullptr) : nullptr;
+    if (map && !on_device) {
+        if (int r = dst->rank.ensure((size_t)n + 1)) return r;
+        ids = dst->rank.p;
+    }
+    if (int r = vocab_add(e, dst, text, dst->imp_rng.p, n, false, true, weight, ids)) return r;
+    CU(cudaEventRecord(dst->ev[3], s));
+    if (map && !on_device) CU(cudaMemcpyAsync(map, ids, (size_t)n * sizeof(int32_t), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    dst->last_ms = elapsed(dst->ev[0], dst->ev[1]) + elapsed(dst->ev[2], dst->ev[3]);
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_clear(latok_b200_vocab *v)
+{
+    if (!v) return fail(LATOK_B200_EINVAL, "vocabulary is NULL");
+    CU(cudaSetDevice(v->device));
+    CU(cudaMemsetAsync(v->table.p, 0, (size_t)v->cap * sizeof(VocabSlot), 0));
+    CU(cudaStreamSynchronize(0));
+    v->n_keys = 0;
+    v->key_bytes = 0;
+    v->last_ms = 0.f;
     return LATOK_B200_OK;
 }
 

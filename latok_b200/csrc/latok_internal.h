@@ -154,11 +154,14 @@ struct VocabParams {
     int32_t *ids;                  // [n] or NULL
     int32_t unk;
     unsigned long long *counts;    // [n_keys] or NULL
+    const long long *weight;       // [n]: count of key k (a merge), or NULL: 1 per token
     VocabStatus *st;
     unsigned long long limit;      // new claims the load limit allows in this launch
 };
 enum VocabPhase { VOCAB_INSERT, VOCAB_LOOKUP, VOCAB_FLAG, VOCAB_LENS, VOCAB_COMMIT, VOCAB_COUNT, VOCAB_REHASH };
 cudaError_t launch_vocab(VocabPhase phase, const VocabParams &p, long long n_new, int n_sm, cudaStream_t s);
+// rng[k] = (key_off[k], key_off[k + 1]) for k < n, on the device (a merge's source keys)
+cudaError_t launch_vocab_ranges(const long long *key_off, long long n, longlong2 *rng, int n_sm, cudaStream_t s);
 cudaError_t vocab_scan(int which, void *tmp, size_t *tmp_bytes, const VocabParams &p, long long n_new, long long key_bytes,
                        cudaStream_t s);
 

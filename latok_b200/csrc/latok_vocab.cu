@@ -19,8 +19,11 @@
 //   (exclusive scan)     arena offsets of the new keys
 //   vocab_commit_kernel  copies the new keys into the arena and rewrites their slots' ref to VOCAB_COMMITTED | id
 //   vocab_count_kernel   ids per token; counts += 1 per token, aggregated within a warp first (__match_any_sync: a Zipf
-//                        stream puts most increments on a handful of slots)
+//                        stream puts most increments on a handful of slots), or += weight[k] per key (merge)
 // Lookup (frozen use) is vocab_insert_kernel without claims: id of the key, or the caller's unk id.
+// Merge (latok_b200_vocab_merge) is one batch whose tokens are the source's keys in id order, weighted by their counts:
+// vocab_ranges_kernel turns the source's key offsets into the batch's ranges on the device, and the count kernel's ids
+// are the map source id -> destination id.
 // Keys of up to VOCAB_LONG bytes take one lane each; longer keys (documents reach 64 KB per string) a whole warp each.
 // Integer / memory-bound kernels; no tensor cores.
 #include "latok_internal.h"
@@ -230,7 +233,8 @@ __global__ void __launch_bounds__(256) vocab_commit_kernel(const VocabParams p)
     }
 }
 
-// ids per token (ids may be NULL) and counts += 1 per token (counts may be NULL)
+// ids per token (ids may be NULL) and counts += 1 per token (counts may be NULL), or counts += weight[k] per token with
+// weights (a merge: its tokens are distinct keys, so there is nothing to aggregate)
 __global__ void __launch_bounds__(256) vocab_count_kernel(const VocabParams p)
 {
     const int lane = threadIdx.x & 31;
@@ -242,7 +246,9 @@ __global__ void __launch_bounds__(256) vocab_count_kernel(const VocabParams p)
             id = (long long)(p.table[p.slot[k]].ref & ~VOCAB_COMMITTED);
             if (p.ids) p.ids[k] = (int32_t)id;
         }
-        if (p.counts) {
+        if (p.weight) {
+            if (k < p.n && p.counts) atomicAdd(&p.counts[id], (unsigned long long)p.weight[k]);
+        } else if (p.counts) {
             const unsigned same = __match_any_sync(0xFFFFFFFFu, id);
             if (k < p.n && lane == __ffs(same) - 1) atomicAdd(&p.counts[id], (unsigned long long)__popc(same));
         }
@@ -265,6 +271,13 @@ __global__ void __launch_bounds__(256) vocab_rehash_kernel(const VocabParams p)
     }, [](long long, bool) {});
 }
 
+// rng[k] = (key_off[k], key_off[k + 1]): the ranges of a merge's source keys in its arena
+__global__ void __launch_bounds__(256) vocab_ranges_kernel(const long long *key_off, long long n, longlong2 *rng)
+{
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x)
+        rng[k] = make_longlong2(key_off[k], key_off[k + 1]);
+}
+
 static unsigned grid_for(long long n, int per_block, int n_sm)
 {
     const long long want = (n + per_block - 1) / per_block, cap = (long long)n_sm * 8;
@@ -282,6 +295,12 @@ cudaError_t launch_vocab(VocabPhase phase, const VocabParams &p, long long n_new
     case VOCAB_COUNT: vocab_count_kernel<<<grid_for(p.n, 256, n_sm), 256, 0, s>>>(p); break;
     case VOCAB_REHASH: if (p.n_keys) vocab_rehash_kernel<<<grid_for(p.n_keys, 256, n_sm), 256, 0, s>>>(p); break;
     }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_vocab_ranges(const long long *key_off, long long n, longlong2 *rng, int n_sm, cudaStream_t s)
+{
+    if (n) vocab_ranges_kernel<<<grid_for(n, 256, n_sm), 256, 0, s>>>(key_off, n, rng);
     return cudaGetLastError();
 }
 

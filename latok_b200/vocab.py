@@ -6,12 +6,16 @@
     v.most_common(10)                    # [(token, count), ...]
     frozen = Vocab.from_tokens([t for t, c in v.most_common() if c >= 5])
     ids, _ = frozen.encode(texts, add=False, unk=-1)
+    m = v.merge(w)                       # Counter.update(w); m[i] = v's id of w's key i (w may be on another GPU)
 
 Keys are the exact token texts (``text[s:e].strip()`` of the tokenizer, no normalisation); ids are dense and follow the
-order of first occurrence, so two vocabularies fed the same batches agree id for id.  A vocabulary lives on one GPU.
+order of first occurrence, so two vocabularies fed the same batches agree id for id.  A vocabulary lives on one GPU;
+merging vocabularies built from consecutive shards of a batch, in shard order, gives the vocabulary one GPU builds
+from the whole batch (latok_b200.sharding.encode_sharded / update_sharded count and encode a batch over several GPUs).
 """
 from __future__ import annotations
 
+import contextlib
 import ctypes as C
 from typing import List, Optional, Sequence, Tuple
 
@@ -29,12 +33,16 @@ class Vocab:
         self.engine = engine or default_engine()
         self._L = self.engine._L
         self.frozen = False
+        self.version = 0             # +1 for every change of keys or counts (replicas of latok_b200.sharding)
+        self._replicas = {}          # device -> (version, Vocab): lookup copies for sharded encodes
         h = C.c_void_p()
         with self.engine._lock:
             _lib.check(self._L.latok_b200_vocab_create(self.engine._h, int(capacity), C.byref(h)))
         self._h = h
 
     def close(self):
+        for _, r in getattr(self, "_replicas", {}).values():
+            r.close()
         if getattr(self, "_h", None):
             self._L.latok_b200_vocab_destroy(self._h)
             self._h = None
@@ -58,6 +66,8 @@ class Vocab:
             else:
                 ptr, on_device = ids.data_ptr(), 1
         _lib.check(self._L.latok_b200_vocab_encode(e._h, self._h, 1 if add else 0, int(unk), n_tokens, ptr, on_device))
+        if add:
+            self.version += 1
 
     def encode_oldest(self, add: bool = True, unk: int = -1, want_ids: bool = True) -> Optional[np.ndarray]:
         """int32 ids of the tokens of the engine's oldest batch in flight (submitted with SPANS), or None without
@@ -112,6 +122,43 @@ class Vocab:
         buf = np.ascontiguousarray(buf, dtype=np.uint8)
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         return self._run(buf, offsets, add, unk, "device" if device else "host")
+
+    def merge(self, other: "Vocab", device: bool = False):
+        """Counter.update(other) on the device: every key of `other` is added with its count, keys new to `self` get
+        the next ids in `other`'s id order.  Returns the map from `other`'s ids to `self`'s: int32 NumPy array of
+        len(other), or (device=True) a CUDA int32 tensor on `self`'s device.  `other` may live on another GPU."""
+        return self._merge(other, "device" if device else "host")
+
+    def _merge(self, other: "Vocab", out: str):
+        if self.frozen:
+            raise RuntimeError("this vocabulary is frozen (Vocab.from_tokens): it cannot take a merge")
+        if other is self:
+            raise ValueError("a vocabulary cannot be merged into itself")
+        # both engines' locks, in one order for every caller: two threads merging in opposite directions cannot deadlock
+        engines = {id(e): e for e in (self.engine, other.engine)}.values()
+        with contextlib.ExitStack() as held:
+            for e in sorted(engines, key=lambda e: (e.device, id(e))):
+                held.enter_context(e._lock)
+            n = len(other)
+            m, ptr, on_device = None, None, 0
+            if out == "device":
+                import torch
+                m = torch.empty(n, dtype=torch.int32, device=f"cuda:{self.engine.device}")
+                ptr, on_device = m.data_ptr(), 1
+            elif out == "host":
+                m = np.empty(n, dtype=np.int32)
+                ptr = m.ctypes.data if n else None
+            _lib.check(self._L.latok_b200_vocab_merge(self.engine._h, self._h, other._h, ptr, on_device))
+            self.version += 1
+            return m
+
+    def clear(self) -> None:
+        """Drop every key and count (the device allocations stay for the next batches)."""
+        if self.frozen:
+            raise RuntimeError("this vocabulary is frozen (Vocab.from_tokens): it cannot be cleared")
+        with self.engine._lock:
+            _lib.check(self._L.latok_b200_vocab_clear(self._h))
+            self.version += 1
 
     # ---- contents --------------------------------------------------------------------------------
     def _size(self):
@@ -174,10 +221,11 @@ class Vocab:
                                                     off.ctypes.data, len(tokens),
                                                     None if cnt is None else cnt.ctypes.data))
         v.frozen = True
+        v.version += 1
         return v
 
     def last_ms(self) -> float:
-        """Device time of the last encode / update / import (token byte ranges included)."""
+        """Device time of the last encode / update / import / merge (token byte ranges and a merge's copy-in included)."""
         ms = C.c_float(0)
         _lib.check(self._L.latok_b200_vocab_last_ms(self._h, C.byref(ms)))
         return ms.value
