@@ -79,7 +79,9 @@ LATOK_B200_API int latok_b200_destroy(latok_b200_engine *e);
  *      Defaults = C_SPLIT / C_MASK / C_SYM of default_tokenizer.py:108-110.
  *      Restriction: the split matrix must contain the row [SPACE_IDX] (every whitespace
  *      character is a split point), which is what makes "drop an all-whitespace span"
- *      equal to the reference's `text[s:e].strip()` test. */
+ *      equal to the reference's `text[s:e].strip()` test.
+ *      A batch is tokenized with the rules in force when it is submitted: set_rules between a submit
+ *      and its fetch (pipeline depth 2) applies to later submits only. */
 LATOK_B200_API int latok_b200_set_rules(latok_b200_engine *e,
                          const int8_t *split, int split_rows, int split_cols,
                          const int8_t *mask, int mask_rows, int mask_cols,

@@ -183,12 +183,14 @@ LATOK_HD void squeeze_planes_log(uint32_t P[NP], uint32_t &F, uint32_t lead)
 }
 
 // ---- block mask, common case (latok.c:218-244 when no whitespace chunk holds more than one mark) -------------
-// CL = characters that close a chunk (space / last character of a string), M = marks (never closers under the
-// default rules), cin = a mark is pending in the chunk that is open at the first character.
+// CL = characters that close a chunk (space / last character of a string), M = marks, cin = a mark is pending in
+// the chunk that is open at the first character.
 // Returns T = (M & ~CL) + ~CL + cin: T & CL are the closers reached with a pending mark ("hot"), M & ~CL & T are
-// marks that found another mark pending in their chunk (then the exact evaluation must be used), and the carry
-// out of bit 31 (cout) says a mark is still pending after the last character.  Positions that hold no character
-// must be 0 in CL and M; they pass the carry on.
+// marks that found another mark pending in their chunk, and the carry out of bit 31 (cout) says a mark is still
+// pending after the last character.  Positions that hold no character must be 0 in CL and M; they pass the carry on.
+// The result is exact unless (M & ~CL & T) | (M & CL) != 0; then the exact evaluation must be used.  A mark on a
+// closer (never under the default rules; custom mask rows can fire on a space or on the last character of a
+// string) is dropped here, while latok.c:218-244 takes it before that closer, which makes the closer hot.
 LATOK_HD uint32_t chunk_carry(uint32_t M, uint32_t CL, uint32_t cin, uint32_t &cout)
 {
     const uint32_t R = ~CL, A = M & R;

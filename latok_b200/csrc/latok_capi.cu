@@ -153,6 +153,7 @@ struct Batch {
     const long long *cur_off = nullptr;
     long long n_strings = 0, n_bytes = 0;
     uint32_t what = 0;
+    RuleSet rules{};                                // the engine's rules at submit (a token-capacity re-run uses them too)
     long long n_chars = 0, n_tokens = 0, walks = 0;
     float kernel_ms = 0.f;
     void release()
@@ -390,7 +391,7 @@ static int run_device(latok_b200_engine *e, Batch &b)
     // The tokenize kernel, in the geometry its plan picks for the batch.  It also gives the character counts and the
     // offsets check of a matrix-only batch.  The parse matrix follows it on the same stream.
     const bool feats = (b.what & LATOK_B200_FEATS) != 0;
-    const Tok5Plan t5 = tokenize5_plan(b.n_bytes, b.n_strings, feats, e->tl, e->rules.is_default != 0, e->n_sm);
+    const Tok5Plan t5 = tokenize5_plan(b.n_bytes, b.n_strings, feats, e->tl, b.rules.is_default != 0, e->n_sm);
     if (int r = b.d_first.ensure((size_t)t5.nranges + 1)) return r;
     // the status word of every aggregate record carries the launch epoch, so records are zeroed only when (re)allocated
     // (agg / inc / osum / planes are shared by the two sets: tokenize kernels run one after the other on one stream)
@@ -422,7 +423,7 @@ static int run_device(latok_b200_engine *e, Batch &b)
     p.agg = e->agg.p; p.inc = e->inc.p; p.osum = e->osum.p; p.planes = e->d_planes.p; p.epoch = e->epoch;
     p.ticket = &b.d_result.p->ticket; p.ticket_base = 0;
     p.result = b.d_result.p;
-    p.table_blob = e->d_table.p; p.tl = e->tl; p.rules = e->rules;
+    p.table_blob = e->d_table.p; p.tl = e->tl; p.rules = b.rules;
 
     // The string index of this batch is built on the aux stream, so that with back-to-back submits it overlaps the
     // tokenize kernel of the previous batch (the two sets alternate).
@@ -521,7 +522,7 @@ int latok_b200_submit(latok_b200_engine *e, const uint8_t *utf8, const int64_t *
         CU(cudaMemcpyAsync(b.d_off.p, src_o, sizeof(long long) * ((size_t)n_strings + 1), cudaMemcpyHostToDevice, e->s_in));
         CU(cudaEventRecord(b.ev_h2d, e->s_in));
         b.cur_in = b.d_in.p; b.cur_off = b.d_off.p;
-        b.n_strings = n_strings; b.n_bytes = n_bytes; b.what = what;
+        b.n_strings = n_strings; b.n_bytes = n_bytes; b.what = what; b.rules = e->rules;
         b.inputs_on_stream = true;
         return run_device(e, b);
     }();
@@ -543,7 +544,7 @@ int latok_b200_submit_device(latok_b200_engine *e, const uint8_t *d_utf8, const 
     Batch &b = *bp;
     b.submitted = false;
     b.cur_in = d_utf8; b.cur_off = (const long long *)d_offsets;
-    b.n_strings = n_strings; b.n_bytes = n_bytes; b.what = what;
+    b.n_strings = n_strings; b.n_bytes = n_bytes; b.what = what; b.rules = e->rules;
     b.inputs_on_stream = false;
     const int rc = run_device(e, b);
     if (rc) drop_last(e);

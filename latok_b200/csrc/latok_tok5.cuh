@@ -580,7 +580,10 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     if (UNLIKELY(!lo_found && !seen_cl)) {
                         const unsigned Gc = __ballot_sync(FULL, CL != 0u);
                         const int fl = Gc ? __ffs(Gc) - 1 : 32;
-                        mb1 += __popc(lane < fl ? Mm : (lane == fl ? (Mm & ((CL & (0u - CL)) - 1u)) : 0u));
+                        // (a mark on a closer comes first: the first closer's own mark counts -- generic rules only, the
+                        // default mask rows never fire on a closer)
+                        const uint32_t upto = kDefault ? (CL & (0u - CL)) - 1u : CL ^ (CL - 1u);
+                        mb1 += __popc(lane < fl ? Mm : (lane == fl ? (Mm & upto) : 0u));
                         seen_cl = Gc != 0u;
                     }
                     uint32_t co;
@@ -589,7 +592,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     const unsigned long long sum = (unsigned long long)(G | Pg) + (unsigned long long)G + (unsigned long long)(xb != 0 ? 1u : 0u);
                     const uint32_t cin = (((uint32_t)sum ^ Pg) >> lane) & 1u;
                     const uint32_t T = chunk_carry(Mm, CL, cin, co);
-                    if (LIKELY(xb < 2 && !__any_sync(FULL, (Mm & ~CL & T) != 0u))) {
+                    // chunk_carry drops a mark on a closer: under generic rules such a step is evaluated mark by mark
+                    const uint32_t exact = (Mm & ~CL & T) | (kDefault ? 0u : (Mm & CL));
+                    if (LIKELY(xb < 2 && !__any_sync(FULL, exact != 0u))) {
                         HOTorM = T & CL;
                         xb = (int)((sum >> 32) & 1u);
                     } else {

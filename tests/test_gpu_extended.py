@@ -89,12 +89,7 @@ def test_tokens_spanning_whole_ranges_and_tiles(engine):
     RANGE, TILE5 = engine.geometry
     # one token that covers 2, 3 and 10 whole ranges (the last one crosses a tile boundary), started and ended at
     # drifting offsets; once with spans only and once with token features (the open-token sums chain, `osum`)
-    texts = []
-    for k in range(40):
-        for nr in (2, 3, 10):
-            n = nr * RANGE + (k * 53) % 257 - 128
-            texts.append("lead " * (k % 7) + "x" * n + " tail word")
-            texts.append("日" * (n // 3) + " z")
+    texts = corpus.tokens_spanning_ranges(RANGE)
     check_batch(engine, texts, 3, label="long tokens, spans")
     check_batch(engine, texts, 7, label="long tokens, token features")
 
@@ -105,22 +100,12 @@ def test_token_feature_rows_in_ordinal_order(engine):
     the 25-byte rows at every phase of a 16-byte chunk, tokens longer than 255 characters (uint8 wrap-around of the
     sums, latok.c:342-354), tokens that begin several lane-words / steps / ranges before they end."""
     RANGE, _ = engine.geometry
-    texts = []
-    for k in range(48):
-        lead = "w " * k                                  # k tokens in front: the rows of what follows start at every phase
-        texts.append(lead + "a,b" * 700)                 # one token end per character: > 512 per 1 KB step (fallback path)
-        texts.append(lead + "!?" * (300 + 7 * k))        # symbols only
-        texts.append(lead + "ab cd, " * (140 + k))       # ordinary density, ~170 rows per step
-        texts.append(lead + ("x" * (250 + k) + " ") * 9) # tokens around the uint8 wrap (250..297 characters)
-        texts.append(lead + "é" * (260 + 3 * k) + " 日本語 " + "y" * (1000 + 37 * k) + " z")
-        texts.append(lead + "tok " * 3 + "q" * (RANGE + 100 * k) + ",end")     # a token that began a range earlier
-        texts.append("z" * k)                            # a few bytes, also the empty string
+    texts = corpus.token_feature_rows(RANGE)
     check_batch(engine, texts, 7, label="token-feature rows")
     # exactly around the list capacity: 505..520 token ends in the first step of a string, then sparse text
-    texts = [(",a" * (250 + j) + " " + "word " * 300) for j in range(0, 12)]
-    check_batch(engine, texts, 7, label="token-feature rows around the list capacity")
+    check_batch(engine, corpus.token_feature_rows_at_capacity(), 7, label="token-feature rows around the list capacity")
     # one token / a handful of tokens per batch (the trip's first and last chunk are the same one)
-    for t in (["a"], ["a b"], ["a b c d e f"], ["", "a", "", "b c"]):
+    for t in corpus.TINY_BATCHES:
         check_batch(engine, t, 7, label=f"token-feature rows, tiny batch {t!r}")
 
 

@@ -12,12 +12,9 @@ from oracle import oracle
 pytestmark = pytest.mark.gpu
 
 ALL = 1 | 2 | 4 | 8
-# bytes owned per unit of work (latok_internal.h): a range (one warp) and a tile (the ranges of one CTA, one look-back
-# record) in both geometries of the tokenize kernel (long strings: 3 968-byte ranges x 9, short strings: 2 944 x 11);
-# tests place interesting things around multiples of each, and around 7 936 bytes, a size that cuts ranges at
-# other phases
-RANGES = (3968, 2944)
-UNITS = (3968, 7936, 9 * 3968, 2944, 11 * 2944)
+# units of work of the two kernel geometries (corpus.py)
+RANGES = corpus.RANGES
+UNITS = corpus.UNITS
 TILE = 7936
 
 
@@ -120,93 +117,44 @@ def test_every_code_point(engine, golden_dir):
     assert bad.size == 0, [hex(int(b)) for b in bad[:10]]
 
 
-def _long_doc(rng, n_chars, profile="ascii"):
-    parts, total = [], 0
-    while total < n_chars:
-        s = corpus.fuzz_string(rng, 200, profile)
-        parts.append(s)
-        parts.append(" " if rng.random() < 0.7 else "\n")
-        total += len(s) + 1
-    return "".join(parts)[:n_chars]
+_long_doc = corpus.long_doc
 
 
 def test_long_documents_cross_tiles(engine):
-    rng = np.random.default_rng(42)
-    sizes = [(70000, "ascii"), (50000, "mixed"), (33000, "marks"), (100, "ascii")]
-    for u in UNITS:
-        sizes += [(u, "ascii"), (u + 1, "ascii"), (u - 1, "ascii"), (2 * u, "ascii"), (3 * u + 5, "mixed")]
-    docs = [_long_doc(rng, int(n), p) for n, p in sizes]
-    check_batch(engine, docs, label="long docs")
+    check_batch(engine, corpus.long_documents(), label="long docs")
 
 
 def test_boundary_alignment_sweep(engine):
     """Slide interesting patterns across the tile boundary one byte at a time."""
-    patterns = ["a@b.c", " #tag ", "x http://t.co/abc y", "fooBar", ".@joe ", "éè 日本 \U0001F600!", "a, b",
-                "  ", "!! ", "e@f,g@h,i@j one,two three,four "]
     for unit in UNITS:
-        texts = []
-        for pat in patterns:
-            for shift in range(-8, 6):
-                pad = unit + shift - 3
-                texts.append("w" * 5 + " " + "z" * (pad - 6) + pat + " tail end")
+        texts = corpus.alignment_sweep(unit)
         check_batch(engine, texts, label=f"alignment sweep {unit} (one string per case)")
         # same but as one long string so the boundary falls inside a string at many different phases
         check_batch(engine, [" ".join(texts[:20])], label=f"alignment sweep {unit} (joined)")
     # the same patterns against the 1 KB steps inside a range and against the 116-byte closer search windows
-    texts = []
-    for pat in patterns:
-        for base in (1024, 2048, 3072, 3968 + 116, 3968 + 128, 4096, 2 * 3968 + 116, 2944 + 116, 2944 + 128, 2 * 2944 + 116):
-            for shift in range(-6, 5):
-                texts.append("q r " + "z" * (base + shift - 8) + " " + pat + " tail end")
-    check_batch(engine, texts, label="alignment sweep (steps / search windows)")
+    check_batch(engine, corpus.alignment_sweep_steps(), label="alignment sweep (steps / search windows)")
 
 
 def test_multibyte_straddling_tiles(engine):
-    for ch in ["é", "日", "\U0001F600", "　", " "]:
+    for ch in corpus.STRADDLE_CHARS:
         n = len(ch.encode("utf-8"))
-        texts = []
-        for unit in UNITS + (1024, 2048, 4096):
-            for shift in range(0, 6):
-                texts.append("a" * (unit - shift) + ch * 40 + " b")
-                texts.append("a b " * ((unit - shift) // 4 - 1) + "a" * ((unit - shift) % 4 + 4) + ch * 40 + " b")
-        check_batch(engine, texts, label=f"straddle {ch!r} ({n} bytes)")
+        check_batch(engine, corpus.multibyte_straddle(ch), label=f"straddle {ch!r} ({n} bytes)")
 
 
 def test_long_space_free_runs_and_walk(engine):
     """Chunks longer than the right halo force the look-ahead walk; marks far ahead must blank
     characters in earlier tiles (latok.c:218-244 has unbounded reach)."""
-    cases = []
-    for TILE, run in ((7936, 300), (7936, 1000), (7936, 7936 - 50), (7936, 7936 + 300), (7936, 2 * 7936 + 77), (7936, 40000),
-                      (3968, 100), (3968, 130), (3968, 3968 + 300), (35712, 200), (35712, 35712 + 5000), (31744, 200), (3968, 70000),
-                      (2944, 100), (2944, 130), (2944, 2944 + 300), (32384, 200), (32384, 32384 + 5000), (2944, 70000)):
-        base = "x y " * ((TILE - 120) // 4)
-        cases.append(base + " " + ",".join(["ab"] * (run // 3)) + " end")                    # no mark: commas split
-        cases.append(base + " " + ",".join(["ab"] * (run // 3)) + ",q@r end")                # mark at the very end
-        cases.append(base + " " + ",".join(["ab"] * (run // 3)) + ",http://x.y/z end")
-        cases.append(base + " #" + ",".join(["ab"] * (run // 3)) + " end,more stuff")        # mark at the start
-        cases.append(base + " " + ",".join(["ab"] * (run // 3)))                             # run reaches end of string
-        cases.append(base + " " + ",".join(["ab"] * (run // 3)) + "@z")                      # mark, then end of string
+    cases = corpus.space_free_runs()
     r = check_batch(engine, cases, label="space-free runs")
     assert r.lookahead_walks > 0
     # multibyte inside the long run
-    check_batch(engine, ["y" * (u - 100) + " " + "日、" * 3000 + "a@b 日 end" for u in UNITS], label="cjk run")
+    check_batch(engine, corpus.cjk_runs(), label="cjk run")
 
 
 def test_backlog_across_tiles(engine):
     """Q2: k marks in one whitespace chunk blank the following k-1 chunks too; make the backlog
     cross tile boundaries and string boundaries (it must reset at each string start)."""
-    many = ",".join(f"a{i}@b" for i in range(40))
-    words = " ".join(f"w{i},x" for i in range(60))
-    texts = []
-    for u in UNITS:
-        texts += ["p" * (u - 200) + " " + many + " " + words, "p" * (u - 30) + " " + many + " " + words,
-                  "p q " * ((u - 200) // 4) + many + " " + words, "p q " * ((u - 40) // 4) + many + " " + words]
-    texts += [
-        many + " " + " ".join(f"w{i},x" for i in range(3000)),
-        ",".join(f"a{i}@b" for i in range(5000)) + " " + " ".join(f"w{i},x" for i in range(6000)),
-        many, words, many + " " + words,
-        many + "   " + words,       # empty chunks also consume backlog
-    ]
+    texts = corpus.backlog_across_tiles()
     check_batch(engine, texts, label="backlog")
 
 
@@ -290,32 +238,17 @@ def test_backlog_handoff_between_ranges(engine):
     settle(): the next range repeats its ordinary analysis with the backlog entering): swept over the range end, with
     hand-offs in consecutive ranges (cascade), across a tile boundary, from a tile's last range into the next tile, and
     with backlogs larger than one."""
-    filler = "lorem ipsum dolor sit amet consectetur "
-    marks = ["aa@bb,cc@dd xx", "aa@bb,cc@dd,ee@ff,gg@hh xx yy zz", "http://a.b/c,x@y,#t d@e.f,g@h uu vv ww",
-             "a@b,c@d,e@f,g@h,i@j,k@l,m@n one two three four five six seven"]
-    texts = []
-    for shift, R in [(sh, R) for R in RANGES for sh in range(0, 64, 3 if R == 3968 else 7)]:
-        for m in marks:
-            parts, pos = [], 0
-            for k in range(1, 21 if R == 3968 else 25):  # one multi-mark chunk near the end of each of 20+ ranges (2 tiles + 2)
-                target = R * k - 20 + shift - len(m) // 2
-                pad = max(target - pos, 1)
-                fill = (filler * (pad // len(filler) + 1))[:pad - 1] + " "
-                parts += [fill, m + " "]
-                pos += len(fill) + len(m) + 1
-            texts.append("".join(parts))
+    texts = corpus.handoff_between_ranges()
     check_batch(engine, texts[:40], ALL, label="hand-off, all outputs")
     check_batch(engine, texts, 3, label="hand-off")
     # the same chunks with no space after them for a long while: the backlog is carried through several ranges
-    long_tail = ["pre fix " + m + " " + ("word,word;word/" * 1200) + " end tail a b c" for m in marks]
-    check_batch(engine, long_tail, 7, label="hand-off into a space-free run")
+    check_batch(engine, corpus.handoff_long_tail(), 7, label="hand-off into a space-free run")
 
 
 def test_token_covering_a_whole_range(engine):
     """A token (here: a whole string without a split point) that begins in one range, covers the next one completely
     and ends within the closer search window of the third: the middle range must write its end.  Strings of 4-byte
     characters a few bytes longer than a range drift through every alignment (found by tools/ucd_check.py)."""
-    texts = [chr(0x20000 + j) * n for j in range(700) for n in (997,)] + [chr(0x4E00 + j) * 1325 for j in range(500)]
-    texts += [chr(0x20000 + j) * n for j in range(300) for n in (993, 1001, 1012)]
+    texts = corpus.token_over_whole_range()
     check_batch(engine, texts, 3, label="token over a whole range")
     check_batch(engine, texts[:400], 7, label="token over a whole range, token features")

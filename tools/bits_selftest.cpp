@@ -1,5 +1,6 @@
 // Host self-test of latok_b200/csrc/latok_bits.h (g++ only, no GPU): the bit-sliced ASCII classifier against the
-// generated class table, the byte->plane transpose, squeeze_planes, chunk_carry and flood_down against scalar loops.
+// generated class table, the byte->plane transpose, squeeze_planes, chunk_carry (and when it must defer to the exact
+// evaluation) and flood_down against scalar loops.
 //   g++ -O1 -std=c++17 -I latok_b200/csrc tools/bits_selftest.cpp -o /tmp/bits_selftest && /tmp/bits_selftest
 #include "latok_bits.h"
 #include "_gen/latok_tables.h"
@@ -53,12 +54,16 @@ int main()
         squeeze_planes_log<3>(R, H, lead);
         if (lead) CHECK(R[0] == wantP[0] && R[1] == wantP[1] && R[2] == wantP[2] && H == wantF, "squeeze (compress form) lead %08X", lead);
     }
-    // chunk_carry / flood_down against the sequential definition (at most one mark per chunk, else just the DUP flag)
+    // chunk_carry / flood_down against the sequential definition (latok.c:218-244: a mark is taken before a closer at
+    // the same position).  Marks may fall on closers (custom mask rows); chunk_carry is exact unless it flags the case
+    // for the exact evaluation: a chunk with two marks pending, or a mark on a closer.
+    int flagged_on_closer = 0;
     for (int rep = 0; rep < 200000; ++rep) {
         const int n = rep % 7 == 0 ? (int)(rng() % 33) : 32;
         const uint32_t nm = bits_low(n);
-        uint32_t CL = rng() & rng() & nm, M = rng() & rng() & rng() & ~CL & nm;
+        uint32_t CL = rng() & rng() & nm, M = rng() & rng() & rng() & nm;
         if (rep % 4 == 0) M &= rng();
+        if (rep % 3 != 0) M &= ~CL | (rng() & rng() & rng());    // mostly off the closers (all of them, under the default rules)
         const uint32_t cin = rng() & 1u, bin = rng() & 1u;
         // sequential
         int x = (int)cin; uint32_t hot = 0; bool dup = false;
@@ -68,9 +73,11 @@ int main()
         }
         uint32_t cout;
         const uint32_t T = chunk_carry(M, CL, cin, cout);
-        const bool dup2 = (M & ~CL & T) != 0u;
-        CHECK(dup == dup2, "dup M %08X CL %08X cin %u", M, CL, cin);
-        if (!dup) {
+        const bool dup2 = (M & ~CL & T) != 0u, flagged = dup2 || (M & CL) != 0u;
+        if ((M & CL) == 0u) CHECK(dup == dup2, "dup M %08X CL %08X cin %u", M, CL, cin);
+        else ++flagged_on_closer;
+        CHECK(!dup || flagged, "two marks pending not flagged: M %08X CL %08X cin %u", M, CL, cin);
+        if (!flagged) {
             CHECK((T & CL) == hot, "hot M %08X CL %08X cin %u: %08X vs %08X", M, CL, cin, T & CL, hot);
             CHECK(cout == (uint32_t)(x >= 1), "cout M %08X CL %08X cin %u", M, CL, cin);
             // flood
@@ -83,6 +90,7 @@ int main()
             CHECK(Z == Z2, "flood hot %08X CL %08X bin %u n %d: %08X vs %08X", hot, CL, bin, n, Z2, Z);
         }
     }
+    CHECK(flagged_on_closer > 10000, "only %d cases with a mark on a closer", flagged_on_closer);
     printf(fails ? "bits selftest: %d FAILURES\n" : "bits selftest ok\n", fails);
     return fails ? 1 : 0;
 }
