@@ -561,8 +561,9 @@ static int size_batch(latok_b200_engine *e, Batch &b)
         if (res.error & 1u) { b.submitted = false; return fail(LATOK_B200_EINTERNAL, "device look-back watchdog tripped"); }
         if (res.error & 8u) {
             b.submitted = false;
-            return fail(LATOK_B200_EINTERNAL, "device consistency check failed: tile %llu G_in %llu K_in %llu n_own %lld ntok %lld c_lo %lld c_hi %lld",
-                        res.prof[8], res.prof[9], res.prof[10], (long long)res.prof[11], (long long)res.prof[12], (long long)res.prof[13], (long long)res.prof[14]);
+            const FaultRec &f = res.fault;
+            return fail(LATOK_B200_EINTERNAL, "device consistency check failed: range %llu G_in %llu K_in %llu n_own %lld ntok %lld c_lo %lld c_hi %lld",
+                        f.range, f.G_in, f.K_in, f.n_own, f.ntok, f.c_lo, f.c_hi);
         }
         if ((res.error & 4u) || (long long)res.n_tokens > (long long)(b.d_spans.cap / 2)) {
             // token buffers too small: grow to the exact count and run the batch again
@@ -573,8 +574,18 @@ static int size_batch(latok_b200_engine *e, Batch &b)
         }
         if (res.error & 16u) { b.submitted = false; return fail(LATOK_B200_EINVAL, "LATOK_B200_SPANS16: a string of the batch has 65 536 or more characters"); }
         if (getenv("LATOK_B200_PRINT_PROF")) {
-            fprintf(stderr, "[latok prof]");
-            for (int i = 0; i < 16; ++i) fprintf(stderr, " %llu", res.prof[i]);
+            const KernelStats &st = res.stats;
+            fprintf(stderr, "[latok prof] repeat_rounds=%llu ranges_repeated=%llu repeats_hot_tail=%llu open_head=%llu open_tail=%llu "
+                            "backlog_out=%llu lookback_restarts=%llu walks=%llu",
+                    st.repeat_rounds, st.ranges_repeated, st.repeats_hot_tail, st.open_head, st.open_tail, st.backlog_out,
+                    st.lookback_restarts, res.walks);
+#ifdef LATOK_PROFILE
+            const ProfClocks &c = res.clocks;
+            fprintf(stderr, " | clocks: window=%llu pass_a=%llu guess=%llu pass_c=%llu prefix_wait=%llu pass_d=%llu resolve=%llu/%llu "
+                            "lb_poll=%llu lb_sum=%llu lb_windows=%llu lb_superseded=%llu lb_repolls=%llu",
+                    c.phase[0], c.phase[1], c.phase[2], c.phase[3], c.phase[4], c.phase[5], c.resolve, c.resolve_calls,
+                    c.lb_poll, c.lb_sum, c.lb_windows, c.lb_superseded, c.lb_repolls);
+#endif
             fprintf(stderr, "\n");
         }
         b.n_chars = (long long)res.n_chars; b.n_tokens = (long long)res.n_tokens; b.walks = (long long)res.walks;

@@ -124,28 +124,14 @@ __device__ __forceinline__ uint32_t make_word(uint32_t pw, uint32_t w, uint32_t 
     return x;
 }
 
-// ---- rule evaluation (combine_matrix_rows 2-D, latok.c:318-341) -------------------------------------
-__device__ __forceinline__ void eval_rules(const RuleSet &c_rules, uint32_t w, uint32_t &cnt, bool &mark, uint32_t &sym)
+// ---- block-mask mark of a character (the mask rows of combine_matrix_rows, latok.c:318-341; default_rules() fills C_MASK)
+// (unrolled: constant row indices read the rows straight from the parameter bank and keep the caller's registers free)
+__device__ __forceinline__ bool rule_mark(const RuleSet &rules, uint32_t w)
 {
-    if (c_rules.is_default) {
-        // C_SPLIT: SPACE + SYMBOL + PREV_SYMBOL + UPPER*NEXT_LOWER + UPPER*PREV_LOWER (default_tokenizer.py:49-55)
-        uint32_t upper = (w >> 4) & 1u;
-        cnt = ((w >> 5) & 1u) + ((w >> 6) & 1u) + ((w >> 20) & 1u) + (upper & (w >> 17)) + (upper & (w >> 16));
-        // C_MASK (default_tokenizer.py:80-91)
-        const uint32_t M0 = (1u << 7) | (1u << 18) | (1u << 13);
-        const uint32_t M1 = (1u << 11) | (1u << 18) | (1u << 21) | (1u << 23);
-        const uint32_t M2 = (1u << 8) | (1u << 14) | (1u << 15);
-        const uint32_t M3 = (1u << 9) | (1u << 22) | (1u << 24) | (1u << 12);
-        mark = ((w & M0) == M0) | ((w & M1) == M1) | ((w & M2) == M2) | ((w & M3) == M3);
-        // C_SYM: SYMBOL*NEXT_SPACE (default_tokenizer.py:100-102)
-        sym = ((w >> 6) & (w >> 19)) & 1u;
-    } else {
-        cnt = 0; sym = 0; uint32_t mk = 0;
-        for (int i = 0; i < c_rules.n_split; ++i) cnt += ((w & c_rules.split[i]) == c_rules.split[i]);
-        for (int i = 0; i < c_rules.n_mask; ++i) mk += ((w & c_rules.mask[i]) == c_rules.mask[i]);
-        for (int i = 0; i < c_rules.n_sym; ++i) sym += ((w & c_rules.sym[i]) == c_rules.sym[i]);
-        mark = mk != 0;
-    }
+    bool mark = false;
+#pragma unroll
+    for (int i = 0; i < MAX_RULE_ROWS; ++i) mark |= i < rules.n_mask && (w & rules.mask[i]) == rules.mask[i];
+    return mark;
 }
 
 // 4 feature bits -> 4 byte counters (bit k -> byte k)
@@ -221,8 +207,7 @@ static __device__ bool walk_ahead(const Params &p, const Tables &t, long long po
         const bool ev = lead && lane < ZONE;
         if (ev) {
             const uint32_t full = make_word(pw, w, nw, aw, false, !has_next, !has_an);
-            uint32_t cnt, sy;
-            eval_rules(p.rules, full, cnt, mk, sy);
+            mk = rule_mark(p.rules, full);
             closer = ((full >> 5) & 1u) || !has_next;
         }
         const unsigned bc = __ballot_sync(0xFFFFFFFFu, ev && closer), bm = __ballot_sync(0xFFFFFFFFu, ev && mk);
@@ -315,7 +300,7 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
                         if (first + j >= 0 && !((rec[j].x >> 2) == p.epoch && (rec[j].x & 3u) != 0u)) { rec[j] = ld_rec(p.agg + (first + j)); pending = true; }
                     if (!pending) break;
 #ifdef LATOK_PROFILE
-                    if (lane == 31) atomicAdd(&p.result->prof[14], 1ull);
+                    if (lane == 31) atomicAdd(&p.result->clocks.lb_repolls, 1ull);
 #endif
                     if (++spins > SPIN_LIMIT || (((spins & 1023u) == 0u) && ld_volatile_u32(&p.result->abort_flag))) {
                         atomicOr(&p.result->error, 1u);
@@ -326,7 +311,7 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
                 }
             }
 #ifdef LATOK_PROFILE
-            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->prof[6], (unsigned long long)(_t - _lt0)); _lt0 = _t; }
+            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->clocks.lb_poll, (unsigned long long)(_t - _lt0)); _lt0 = _t; }
 #endif
             // the newest inclusive record of this lane: fetch its prefix
 #pragma unroll
@@ -354,7 +339,7 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
             const unsigned has_reset = __ballot_sync(0xFFFFFFFFu, rj >= 0);
             const int Lr = has_reset ? 31 - __clz(has_reset) : -1;
 #ifdef LATOK_PROFILE
-            if (lane == 0) { atomicAdd(&p.result->prof[13], 1ull); if (Lr >= 0) atomicAdd(&p.result->prof[8], (unsigned long long)((31 - Lr) * LB_PER_LANE)); }
+            if (lane == 0) { atomicAdd(&p.result->clocks.lb_windows, 1ull); if (Lr >= 0) atomicAdd(&p.result->clocks.lb_superseded, (unsigned long long)((31 - Lr) * LB_PER_LANE)); }
 #endif
             const bool contrib = lane >= Lr;          // lanes older than the newest inclusive element are superseded
             // characters / tokens
@@ -375,7 +360,7 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
             if (!x_set) { x_in = __shfl_sync(0xFFFFFFFFu, lastv, 31); x_set = true; }
             if (!__all_sync(0xFFFFFFFFu, ok)) { out.x = 0; return out; }    // watchdog tripped: error flag is set
 #ifdef LATOK_PROFILE
-            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->prof[7], (unsigned long long)(_t - _lt0)); }
+            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->clocks.lb_sum, (unsigned long long)(_t - _lt0)); }
 #endif
             if (Lr >= 0) {
                 const unsigned long long G0 = __shfl_sync(0xFFFFFFFFu, rG, Lr), B0 = __shfl_sync(0xFFFFFFFFu, rB, Lr);
@@ -396,7 +381,7 @@ static __device__ Prefix lookback(long long tile, const Params &p, int lane)
         // wait for the tile after the offending one to publish its exact inclusive prefix, then walk again
         bool ok2 = true;
         wait_rec(p.agg, viol + 1, p.epoch, 2u, p.result, ok2);
-        if (lane == 0) atomicAdd(&p.result->prof[15], 1ull);
+        if (lane == 0) atomicAdd(&p.result->stats.lookback_restarts, 1ull);
         if (!ok2) return out;
     }
 }

@@ -53,13 +53,42 @@ struct __align__(16) IncRec {
 // token-feature mode only: feature sums of the token still open at the end of a tile
 struct __align__(16) OpenSums { unsigned has_split; unsigned pad[3]; unsigned sums[8]; };
 
+// Statistics of the tokenize kernel's rare paths, counted in every build (LATOK_B200_PRINT_PROF prints them)
+struct KernelStats {
+    unsigned long long repeat_rounds;       // rounds of repeated analyses (resolve())
+    unsigned long long ranges_repeated;     // ranges analysed again
+    unsigned long long repeats_hot_tail;    // ... of those, because the guess about a hot tail was wrong
+    unsigned long long open_head;           // analyses of ranges that begin inside a chunk
+    unsigned long long open_tail;           // ... that end inside one
+    unsigned long long backlog_out;         // ... that leave a block-mask backlog
+    unsigned long long lookback_restarts;   // look-back walks started again behind a tile that needs a real backlog
+};
+// The range whose prefix failed the consistency check of pass D (error bit 3)
+struct FaultRec {
+    unsigned long long range, G_in, K_in;
+    long long n_own, ntok, c_lo, c_hi;
+};
+// LATOK_PROFILE builds: summed clock64() deltas and event counts (lane 0 / 31 of the warps that measure them)
+struct ProfClocks {
+    unsigned long long phase[6];            // compute warps: ticket + window wait, pass A, hot-tail guess, pass C, prefix wait, pass D
+    unsigned long long resolve;             // service warp: resolve() with the backlog from the look-back
+    unsigned long long resolve_calls;
+    unsigned long long lb_poll;             // look-back: waiting for a window of records
+    unsigned long long lb_sum;              // ... summing it
+    unsigned long long lb_windows;          // windows walked
+    unsigned long long lb_superseded;       // records skipped behind an inclusive prefix
+    unsigned long long lb_repolls;          // polling rounds over records not yet published
+};
+
 struct Result {
     unsigned long long n_chars;
     unsigned long long n_tokens;
     unsigned long long walks;
     unsigned long long ticket;   // dynamic tile counter (zeroed with the rest of the struct before each launch)
-    unsigned long long prof[16]; // LATOK_PROFILE builds: summed clock64() deltas per phase (thread 0 of every CTA)
-    unsigned int error;      // bit 0: watchdog, bit 1: offsets not monotone, bit 2: token capacity exceeded
+    KernelStats stats;
+    FaultRec fault;
+    ProfClocks clocks;
+    unsigned int error;      // bit 0: watchdog, bit 1: offsets not monotone, bit 2: token capacity exceeded, bit 3: inconsistent prefix (fault)
     unsigned int abort_flag;
 };
 

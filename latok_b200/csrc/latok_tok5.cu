@@ -26,11 +26,12 @@ static Tok5Plan plan_geometry(bool short_geometry, long long n_bytes, bool feats
 
 Tok5Plan tokenize5_plan(long long n_bytes, long long n_strings, bool feats, const TableLayout &tl, bool is_default, int n_sm)
 {
-    // By the average string length of the batch: short strings get the short geometry.  Token features always run in the
-    // long one.  LATOK_B200_GEOMETRY=short|long overrides both (read on every call).
+    // By the average string length of the batch: short strings get the short geometry; LATOK_B200_GEOMETRY=short|long
+    // overrides that (read on every call).  Token features always run in the long geometry, the only one built with them:
+    // that instantiation lives on registers (25 planes per lane), and 96 of them beat 24 warps per SM.
     bool shortg = n_bytes < 4096LL * (n_strings > 0 ? n_strings : 1);
-    if (feats) shortg = false;      // the token-feature instantiation lives on registers (25 planes per lane): 96 beat 24 warps per SM
     if (const char *g = getenv("LATOK_B200_GEOMETRY")) shortg = g[0] == 's';
+    if (feats) shortg = false;
     return shortg ? plan_geometry<v5::ShortGeometry>(true, n_bytes, feats, tl, is_default, n_sm)
                   : plan_geometry<v5::LongGeometry>(false, n_bytes, feats, tl, is_default, n_sm);
 }

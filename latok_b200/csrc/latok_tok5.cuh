@@ -31,8 +31,10 @@
 // result depends on something it assumed differently is analysed again (the ORDINARY analysis, with the real values) by
 // the service warp itself, at once: the warp that owns the range is busy with its next tile by then.
 // The warps run one tile ahead of the look-back: analysis of tile k+1, then pass D of tile k, whose state waits in
-// place of its input bytes (two window buffers per warp).  Tickets are taken by the first warp that is ready for the
-// next tile, so ticket order follows start order and predecessors publish first.
+// place of its input bytes (two window buffers per warp; Parked owns that layout).  What the analysis of a range found
+// goes to one RangeRec per (slot, range) in Ctl, which the service warp, the prefix of every warp and pass D read.
+// Tickets are taken by the first warp that is ready for the next tile, so ticket order follows start order and
+// predecessors publish first.
 //
 // No tensor cores: nothing here is a dense contraction; the bound is HBM bandwidth.
 #pragma once
@@ -52,7 +54,6 @@ constexpr int TCAP = 320;                // tokens staged per step; steps with m
 constexpr int TSTAGE = (TCAP + 2) * 8;
 constexpr int FLIST = 512;               // token-feature mode: token ends per step that are written in the order of their ordinals
 constexpr int FSTAGE = 832;              // ... row stage: up to 15 bytes left of the trip before + 32 * 25 bytes, in 16-byte chunks
-constexpr int TWG = 12;                  // generic rules: words per lane-word in the (separate) state buffers
 enum { BAR_AGG = 1, BAR_PRE = 3 };
 static_assert(HALO % 32 == 0, "geometry");
 static_assert(TSTAGE >= STEP + 64, "the token stage doubles as the byte stage of partly owned split-mask chunks");
@@ -61,9 +62,10 @@ static_assert(TSTAGE >= 1024 + FSTAGE && FSTAGE >= 15 + 32 * NFEAT + 8 && FSTAGE
 // The kernel exists in two geometries; the host picks one per batch (tokenize5_plan, latok_tok5.cu).  Long strings: 4 KB
 // ranges, 9 compute warps per CTA -- fewer range boundaries inside space-free runs.  Short strings: 3 KB ranges, 11
 // compute warps per CTA at 80 registers -- more warps in flight, which is what the instruction-bound regular path gains
-// from.
-template <int RS_, int NW_>
+// from.  Token features run in the long geometry only (the 25 planes per lane want its 96 registers).
+template <int RS_, int NW_, bool FEATS_>
 struct Geometry {
+    static constexpr bool FEATS = FEATS_;    // the token-feature instantiation exists
     static constexpr int NW = NW_;           // compute warps per CTA (warp 0 is the service warp)
     static constexpr int NTH = (NW + 1) * 32;
     static constexpr int RS = RS_;           // steps per range
@@ -73,28 +75,116 @@ struct Geometry {
     static constexpr int CTAS = 2;           // CTAs per SM the default-rules instantiation is compiled for
     static_assert(RANGE % 16 == 0, "geometry");
 };
-using LongGeometry = Geometry<4, 9>;
-using ShortGeometry = Geometry<3, 11>;
+using LongGeometry = Geometry<4, 9, true>;
+using ShortGeometry = Geometry<3, 11, false>;
 
-struct WAgg { int n_own, ntok, lft, v, flags, u, mb1, pad; };   // flags: 1 have, 2 closed, 4 lo_found, 8 holds a closer, 16 guessed a hot tail
 struct Slot { unsigned long long G, K, base; int pad[2]; };
-struct RInfo { int c_lo, c_hi, n_own, ntok, flags, pad[3]; };    // flags: 1 have, 2 closed, 4 lo_found, 8 last_range
+// What the analysis of a range posts: the characters it owns [c_lo, c_hi) (range-relative; n_own = c_hi - c_lo), the tokens
+// counted in them, its last owned string start (lft, relative to c_lo; -1: none), the block-mask backlog it leaves (v) and --
+// for a range that begins inside a chunk -- how it transforms a backlog: x -> max(x + u, v), mb1 marks in front of its
+// first closer (resolve()).  One record per (slot, range of the tile); the owner of range i is compute warp i.
+struct RangeRec {
+    enum : int {
+        HAVE = 1,            // the range holds data
+        CLOSED = 2,          // it ends at a chunk closer
+        LO_FOUND = 4,        // it begins at a chunk closer (else u and mb1 are set)
+        HOLDS_CLOSER = 8,    // it owns a chunk closer
+        GUESSED_HOT = 16,    // (a range that ends inside a chunk) its first analysis assumed that chunk closed hot
+    };
+    int c_lo, c_hi, n_own, ntok, lft, v, u, mb1, flags;
+};
 template <class Geom>
 struct Ctl {
     int tile_id[2], tk_cnt[2], tk_flag[2];
     int pad0[4];
     Slot slot[2];
-    WAgg wagg[2][Geom::NW];
-    RInfo rinfo[Geom::NW][2];
+    RangeRec rec[2][Geom::NW];
     int tokstep[Geom::NW][2][Geom::RS];  // tokens per step
     int nsa[Geom::NW][2][Geom::RS];      // first split after the step (range-relative character index, -1: none)
 };
 
-// Per lane-word, between the passes, 8 words live IN PLACE of the lane-word's 32 input bytes (default rules):
-//   after pass A : CNT0 CNT1 CNT2 SYM | S  M/HOT  F  packed        after pass C : V0 V1 V2 E | S  lead  F  packed
-// (generic rules: TWG words in a separate buffer: CNT[4] SYM[4] S M/HOT F packed -> V[5] E - - S lead F packed);
-// the string-start map of the window (bit = byte) turns into the lane-word's lead-byte mask once it has been read and
-// moves into the state in pass C.
+// The state of one lane-word while it waits between the passes:
+//   after pass A : CNT[NC] SYM[NY] | S HOT  F packed
+//   after pass C : V[NV]   E       | S lead F packed
+// Pass C rewrites V, E, lead and packed and leaves S and F as pass A stored them: pass D reads them.  The slot of the hot
+// closers takes the lane-word's lead-byte mask: the window's string-start map (bit = byte), whose slot has become that
+// mask in pass A, is rebuilt by the analysis of the next window before pass D reads it.
+// Default rules: 8 words IN PLACE of the lane-word's 32 input bytes (pass A parks a step after it has read the next one),
+// as two 16-byte halves 512 bytes apart inside the step's 1 KB (word w at js*256 + (w >> 2)*128 + ln*4 + (w & 3)), so the
+// 128-bit accesses of a quarter warp fall into 32 different banks (a 32-byte lane stride makes them collide in pairs).
+// Generic rules: WORDS words in a row, in a buffer of their own (plan()).
+template <bool kDefault>
+struct Parked {
+    static constexpr int NC = kDefault ? 3 : 4;     // split-count planes
+    static constexpr int NY = kDefault ? 1 : 4;     // sym-count planes
+    static constexpr int NV = kDefault ? 3 : 5;     // split-value planes
+    static constexpr int WORDS = kDefault ? 8 : 12;
+    static_assert(!kDefault || WORDS * 4 == 32, "the in-place state takes the lane-word's 32 bytes");
+    static_assert(NC + NY <= WORDS - 4 && NV + 1 <= WORDS - 4, "layout");
+    uint32_t *t;
+    __device__ __forceinline__ Parked(uint32_t *base, int js, int ln) : t(kDefault ? base + js * 256 + ln * 4 : base + (js * 32 + ln) * WORDS) {}
+    // the words of step js, once read, as scratch: at least 1 KB
+    __device__ __forceinline__ static uint16_t *scratch(uint32_t *base, int js) { return reinterpret_cast<uint16_t *>(Parked(base, js, 0).t); }
+    __device__ __forceinline__ uint32_t s() const { return w(W_S); }
+    __device__ __forceinline__ uint32_t f() const { return w(W_F); }
+    __device__ __forceinline__ uint32_t packed() const { return w(W_K); }
+    __device__ __forceinline__ uint32_t e() const { return w(W_E); }          // after pass C
+    __device__ __forceinline__ uint32_t lead() const { return w(W_H); }       // after pass C
+
+    __device__ __forceinline__ void store_a(const uint32_t (&cnt)[NC], const uint32_t (&sym)[NY], uint32_t S, uint32_t hot, uint32_t F, uint32_t pk) const
+    {
+        if (kDefault) {
+            *reinterpret_cast<uint4 *>(t) = make_uint4(cnt[0], cnt[1], cnt[2], sym[0]);
+            *reinterpret_cast<uint4 *>(t + 128) = make_uint4(S, hot, F, pk);
+        } else {
+#pragma unroll
+            for (int q = 0; q < NC; ++q) t[q] = cnt[q];
+#pragma unroll
+            for (int q = 0; q < NY; ++q) t[NC + q] = sym[q];
+            t[W_S] = S; t[W_H] = hot; t[W_F] = F; t[W_K] = pk;
+        }
+    }
+    __device__ __forceinline__ void load_a(uint32_t (&cnt)[NC], uint32_t (&sym)[NY], uint32_t &S, uint32_t &hot, uint32_t &F, uint32_t &pk) const
+    {
+        if (kDefault) {
+            const uint4 a = *reinterpret_cast<const uint4 *>(t), b = *reinterpret_cast<const uint4 *>(t + 128);
+            cnt[0] = a.x; cnt[1] = a.y; cnt[2] = a.z; sym[0] = a.w; S = b.x; hot = b.y; F = b.z; pk = b.w;
+        } else {
+#pragma unroll
+            for (int q = 0; q < NC; ++q) cnt[q] = t[q];
+#pragma unroll
+            for (int q = 0; q < NY; ++q) sym[q] = t[NC + q];
+            S = t[W_S]; hot = t[W_H]; F = t[W_F]; pk = t[W_K];
+        }
+    }
+    __device__ __forceinline__ void store_c(const uint32_t (&v)[NV], uint32_t E, uint32_t lead, uint32_t pk) const
+    {
+        if (kDefault) *reinterpret_cast<uint4 *>(t) = make_uint4(v[0], v[1], v[2], E);
+        else {
+#pragma unroll
+            for (int q = 0; q < NV; ++q) t[q] = v[q];
+            t[W_E] = E;
+        }
+        w(W_H) = lead; w(W_K) = pk;
+    }
+    __device__ __forceinline__ void load_c(uint32_t (&v)[NV], uint32_t &E, uint32_t &S, uint32_t &F, uint32_t &pk) const
+    {
+        if (kDefault) {
+            const uint4 a = *reinterpret_cast<const uint4 *>(t), b = *reinterpret_cast<const uint4 *>(t + 128);
+            v[0] = a.x; v[1] = a.y; v[2] = a.z; E = a.w; S = b.x; F = b.z; pk = b.w;
+        } else {
+#pragma unroll
+            for (int q = 0; q < NV; ++q) v[q] = t[q];
+            E = t[W_E]; S = t[W_S]; F = t[W_F]; pk = t[W_K];
+        }
+    }
+
+  private:
+    static constexpr int W_E = NV, W_S = WORDS - 4, W_H = WORDS - 3, W_F = WORDS - 2, W_K = WORDS - 1;
+    __device__ __forceinline__ uint32_t &w(int i) const { return t[kDefault && i >= 4 ? 124 + i : i]; }
+};
+static_assert(FLIST * 2 <= STEP, "token-feature mode: the token-end list lives in a step's parked state");
+
 struct Plan {
     int tables, ctl, mbar, sbm0, warp0, x[2], sst, tst, sbm, temp[2], per_warp, total;
 };
@@ -112,14 +202,15 @@ __host__ __device__ inline Plan plan(const TableLayout &tl, bool is_default)
     s.sst = take(SSTAGE);
     s.tst = take(TSTAGE);
     s.sbm = take(Geom::RS * 32 * 4);
-    for (int b = 0; b < 2; ++b) s.temp[b] = is_default ? s.x[b] + LPAD : take(Geom::RS * TWG * 32 * 4);
+    for (int b = 0; b < 2; ++b)                 // parked state (default rules: in place of the window's bytes)
+        s.temp[b] = is_default ? s.x[b] + LPAD : take(Geom::RS * 32 * Parked<false>::WORDS * 4);
     s.per_warp = o - s.warp0;
     s.total = s.warp0 + Geom::NW * s.per_warp;
     return s;
 }
 
 #ifdef LATOK_PROFILE
-#define PROF5(i) do { if (lane == 0) { long long _t = clock64(); atomicAdd(&p.result->prof[i], (unsigned long long)(_t - _prof_t)); _prof_t = _t; } } while (0)
+#define PROF5(i) do { if (lane == 0) { long long _t = clock64(); atomicAdd(&p.result->clocks.phase[i], (unsigned long long)(_t - _prof_t)); _prof_t = _t; } } while (0)
 #else
 #define PROF5(i) do { } while (0)
 #endif
@@ -144,11 +235,8 @@ template <class Geom, bool kDefault, bool kFeats>
 __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize5_kernel(const Params p)
 {
     constexpr int NW = Geom::NW, NTH = Geom::NTH, RS = Geom::RS, WIN = Geom::WIN, RANGE = Geom::RANGE, XBYTES = Geom::XBYTES;
-    constexpr int NC = kDefault ? 3 : 4;      // split-count planes
-    constexpr int NY = kDefault ? 1 : 4;      // sym-count planes
-    constexpr int NV = kDefault ? 3 : 5;      // split-value planes
-    constexpr int TWD = kDefault ? 8 : TWG;   // state words per lane-word
-    constexpr int I_S = kDefault ? 4 : 8, I_H = kDefault ? 5 : 9, I_F = kDefault ? 6 : 10, I_K = kDefault ? 7 : 11, I_E = kDefault ? 3 : 5;
+    using PS = Parked<kDefault>;
+    constexpr int NC = PS::NC, NY = PS::NY, NV = PS::NV;
     extern __shared__ __align__(128) unsigned char smem[];
     const Plan sp = plan<Geom>(p.tl, kDefault);
     uint8_t *tableS = smem + sp.tables;
@@ -183,26 +271,19 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
     // =================================================================================================
     // compute warps
     // =================================================================================================
-    // `tw` = the compute warp whose buffers are worked on: the warp itself, or -- when the service warp repeats the
-    // analysis of a range (resolve()) -- the warp that owns that range
-    int tw = cw;
-    auto wbase_of = [&]() -> unsigned char * { return smem + sp.warp0 + tw * sp.per_warp; };
+    // the buffers of compute warp `w`: a compute warp works on its own; the service warp, when it repeats the analysis of a
+    // range (resolve()), on those of the warp that owns the range
+    auto wbase_of = [&](int w) -> unsigned char * { return smem + sp.warp0 + w * sp.per_warp; };
     unsigned char *wbase = smem + sp.warp0 + (cw < 0 ? 0 : cw) * sp.per_warp;      // (own buffers: output path of the compute warps)
     uint8_t *sst = wbase + (sp.sst - sp.warp0);
     int2 *tst = reinterpret_cast<int2 *>(wbase + (sp.tst - sp.warp0));
-    auto Xof = [&](int b) -> uint8_t * { return wbase_of() + (sp.x[b] - sp.warp0); };
+    auto Xof = [&](int w, int b) -> uint8_t * { return wbase_of(w) + (sp.x[b] - sp.warp0); };
     // string-start map / lead masks of the window under analysis (the service warp has a scratch of its own: the owner
     // of the range is busy with its next tile)
-    auto sbm_of = [&]() -> uint32_t * {
-        return reinterpret_cast<uint32_t *>(warp == 0 ? smem + sp.sbm0 : wbase_of() + (sp.sbm - sp.warp0));
+    auto sbm_of = [&](int w) -> uint32_t * {
+        return reinterpret_cast<uint32_t *>(warp == 0 ? smem + sp.sbm0 : wbase_of(w) + (sp.sbm - sp.warp0));
     };
-    auto tempof = [&](int b) -> uint32_t * { return reinterpret_cast<uint32_t *>(wbase_of() + (sp.temp[b] - sp.warp0)); };
-    // State words of lane-word (js, ln).  Default rules: the two 16-byte halves of a lane-word's 8 words lie 512 bytes
-    // apart inside the step's 1 KB (word w at js*256 + (w >> 2)*128 + ln*4 + (w & 3)), so the 128-bit accesses of a
-    // quarter warp fall into 32 different banks (a 32-byte lane stride makes them collide in pairs); generic rules: TWG
-    // words in a row.
-    auto SA = [&](uint32_t *base, int js, int ln) -> uint32_t * { return kDefault ? base + js * 256 + ln * 4 : base + (js * 32 + ln) * TWD; };
-    auto SW = [&](int w) -> int { return kDefault ? (w < 4 ? w : 124 + w) : w; };        // offset of word w from SA()
+    auto tempof = [&](int w, int b) -> uint32_t * { return reinterpret_cast<uint32_t *>(wbase_of(w) + (sp.temp[b] - sp.warp0)); };
     const uint32_t *lutv = reinterpret_cast<const uint32_t *>(tableS);
 #ifdef LATOK_PROFILE
     long long _prof_t = clock64();
@@ -213,7 +294,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
     // ---- window load: TMA bulk copy of the 16-byte aligned interior, plain loads for the ragged end
     auto begin_load = [&](long long r, int b) -> bool {
         if (r >= p.nranges) return false;
-        uint8_t *X = Xof(b);
+        uint8_t *X = Xof(cw, b);
         const long long wl = r * (long long)RANGE - LPAD;          // global position of X[0]
         const long long lo = wl < 0 ? 0 : wl;
         long long hi = wl + XBYTES;
@@ -234,8 +315,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         }
         return tma_bytes > 0;
     };
-    auto plain_load = [&](long long r, int b) {          // repeated analysis: fetch the window again
-        uint8_t *X = Xof(b);
+    auto plain_load = [&](long long r, int w, int b) {          // repeated analysis: fetch the window again
+        uint8_t *X = Xof(w, b);
         const long long wl = r * (long long)RANGE - LPAD;
         for (int i = lane * 16; i < XBYTES; i += 512) {
             const long long g = wl + i;
@@ -288,9 +369,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
     // ---- string-start map of a window (bit = byte position), from the offsets of the strings that begin in it.  Needs
     // nothing of the window itself: the compute warps build it while the window is still on its way (the two dependent
     // global loads overlap the TMA copy).
-    auto build_map = [&](const long long r) {
+    auto build_map = [&](const long long r, const int w) {
         if (r >= p.nranges) return;
-        uint32_t *sbmS = sbm_of();
+        uint32_t *sbmS = sbm_of(w);
         const long long w0 = r * (long long)RANGE;
 #pragma unroll
         for (int j = 0; j < RS; ++j) sbmS[j * 32 + lane] = 0;
@@ -304,46 +385,39 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         }
         __syncwarp();
     };
-    // results of the analysis that are posted right away (the rest goes to ctl.rinfo for pass D)
-    int a_n_own = 0, a_ntok = 0, a_lft = -1, a_v = 0, a_u = 0, a_mb1 = 0, a_flags = 0; bool a_guess = false;
 
     // ================================================================================================= analysis
-    // x_init: block-mask backlog entering the range; far_init: the chunk open at the end of the range (a range that does
-    // not end at a chunk closer) will be closed hot.  The first analysis of every range assumes that nothing enters and
-    // (far_init = -1) that an open last chunk WILL be closed hot; the service warp orders a repeat with the real values
-    // where that changes the result (resolve()).
-    auto analyze = [&](const long long r, const int buf, const int x_init, const int far_init) {
+    // Analyses range r in buffer `buf` of compute warp `w` and returns its record.  x_init: block-mask backlog entering the
+    // range; far_init: the chunk open at the end of the range (a range that does not end at a chunk closer) will be closed
+    // hot.  The first analysis of every range assumes that nothing enters and (far_init = -1) that an open last chunk WILL
+    // be closed hot; the service warp orders a repeat with the real values where that changes the result (resolve()).
+    auto analyze = [&](const long long r, const int buf, const int w, const int x_init, const int far_init) -> RangeRec {
         const long long w0 = r * (long long)RANGE;
         const bool have = r < p.nranges, last_range = r == p.nranges - 1;
-        uint8_t *X = Xof(buf);
-        uint32_t *tempS = tempof(buf);
-        uint32_t *sbmS = sbm_of();
+        uint8_t *X = Xof(w, buf);
+        uint32_t *tempS = tempof(w, buf);
+        uint32_t *sbmS = sbm_of(w);
         int c_lo = 0, c_hi = CINF, n_own = 0, ntok_range = 0, lft = -1, v_out = 0;
-        bool closed = true, lo_found = true;
+        bool closed = true, lo_found = true, guessed_hot = false;
         // backlog transfer summary of the owned characters: marks - closers, a string boundary (= reset), marks in front of
         // the first closer, whether there is a closer at all
         int d_mc = 0, mb1 = 0; uint32_t rs_any = 0; bool seen_cl = false;
-        a_guess = false;
-        auto finish = [&]() {
-            a_n_own = n_own; a_ntok = ntok_range; a_lft = lft >= 0 ? lft - c_lo : -1; a_v = v_out;
-            a_flags = (have ? 1 : 0) | (closed ? 2 : 0) | (lo_found ? 4 : 0) | (seen_cl ? 8 : 0) | (a_guess ? 16 : 0);
-            a_u = 0; a_mb1 = 0;
+        auto finish = [&]() -> RangeRec {
+            RangeRec a;
+            a.c_lo = c_lo; a.c_hi = c_hi; a.n_own = n_own; a.ntok = ntok_range; a.lft = lft >= 0 ? lft - c_lo : -1; a.v = v_out;
+            a.flags = (have ? RangeRec::HAVE : 0) | (closed ? RangeRec::CLOSED : 0) | (lo_found ? RangeRec::LO_FOUND : 0) |
+                      (seen_cl ? RangeRec::HOLDS_CLOSER : 0) | (guessed_hot ? RangeRec::GUESSED_HOT : 0);
+            a.u = 0; a.mb1 = 0;
             if (have && !lo_found) {               // (the summary exists)
-                a_u = __any_sync(FULL, rs_any != 0u) ? NEG : __reduce_add_sync(FULL, d_mc);
-                a_mb1 = min(__reduce_add_sync(FULL, mb1), 1 << 20);
+                a.u = __any_sync(FULL, rs_any != 0u) ? NEG : __reduce_add_sync(FULL, d_mc);
+                a.mb1 = min(__reduce_add_sync(FULL, mb1), 1 << 20);
             }
-            if (lane == 0) {
-                RInfo &ri = ctl.rinfo[tw][buf];
-                ri.c_lo = c_lo; ri.c_hi = c_hi; ri.n_own = n_own; ri.ntok = ntok_range;
-                ri.flags = (have ? 1 : 0) | (closed ? 2 : 0) | (lo_found ? 4 : 0) | (last_range ? 8 : 0);
-            }
-            __syncwarp();
+            return a;
         };
         if (!have) {
             c_hi = 0;
             v_out = x_init;
-            finish();
-            return;
+            return finish();
         }
         // ---- the character in front of the window: prev-context of the window's first character.  Matters only when the
         // range owns that character, i.e. no closer is found in the head window (then the range begins inside a chunk), and
@@ -604,21 +678,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                         xb = __shfl_sync(FULL, out, 31);
                     }
                 }
-                // ---- park the step for pass C (in place of its input bytes; step js+1 has been read already)
-                {
-                    uint32_t *t = SA(tempS, js, lane);
-                    const uint32_t pk = pack_ncp(n, c0, (int)((LB >> 3) & 1u)) | ((XF & 1u) << 31);
-                    if (kDefault) {
-                        *reinterpret_cast<uint4 *>(t) = make_uint4(CNT[0], CNT[1], CNT[2], SYC[0]);
-                        *reinterpret_cast<uint4 *>(t + 128) = make_uint4(Sraw, HOTorM, Fm, pk);
-                    } else {
-#pragma unroll
-                        for (int q = 0; q < NC; ++q) t[q] = CNT[q];
-#pragma unroll
-                        for (int q = 0; q < NY; ++q) t[4 + q] = SYC[q];
-                        t[I_S] = Sraw; t[I_H] = HOTorM; t[I_F] = Fm; t[I_K] = pk;
-                    }
-                }
+                // ---- park the step for pass C (step js+1 has been read already)
+                PS(tempS, js, lane).store_a(CNT, SYC, Sraw, HOTorM, Fm, pack_ncp(n, c0, (int)((LB >> 3) & 1u)) | ((XF & 1u) << 31));
             }
 #pragma unroll
             for (int f = 0; f < NBASE; ++f) Pp[f] = Pc[f];
@@ -630,9 +691,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         if (n_own < 0) n_own = 0;
         v_out = xb;
         if (lane == 0) {                           // (statistics)
-            if (xb != 0) atomicAdd(&p.result->prof[14], 1ull);
-            if (!lo_found) atomicAdd(&p.result->prof[12], 1ull);
-            if (!closed) atomicAdd(&p.result->prof[13], 1ull);
+            if (xb != 0) atomicAdd(&p.result->stats.backlog_out, 1ull);
+            if (!lo_found) atomicAdd(&p.result->stats.open_head, 1ull);
+            if (!closed) atomicAdd(&p.result->stats.open_tail, 1ull);
         }
         __syncwarp();
         // character ends its string: the next character (possibly in the next lane-word) starts one
@@ -655,10 +716,10 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 int open_len = n_own;
 #pragma unroll 1
                 for (int js = RS - 1; js >= 0; --js) {
-                    const uint32_t *t = SA(tempS, js, lane);
-                    const uint32_t pk = t[SW(I_K)];
+                    const PS t(tempS, js, lane);
+                    const uint32_t pk = t.packed();
                     const int n = pk_n(pk), c0 = pk_c0(pk);
-                    const uint32_t CLo = (t[SW(I_S)] | L_of(t[SW(I_F)], pk)) & range_mask(c0, c_lo, c_hi) & real_mask(js, n);
+                    const uint32_t CLo = (t.s() | L_of(t.f(), pk)) & range_mask(c0, c_lo, c_hi) & real_mask(js, n);
                     const unsigned hb = __ballot_sync(FULL, CLo != 0u);
                     if (hb) {
                         const int pos = __shfl_sync(FULL, c0 + 31 - (int)__clz(CLo), 31 - __clz(hb));
@@ -669,7 +730,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 far_guess = open_len >= 512;
             }
         }
-        a_guess = far_init < 0 ? far_guess : (far_init != 0);
+        guessed_hot = far_init < 0 ? far_guess : (far_init != 0);
         PROF5(2);
         // ---------------------------------------------------------------- pass C: blanked chunks, values, tokens
         {
@@ -678,18 +739,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
             int lft_max = -1;
 #pragma unroll 1
             for (int js = RS - 1; js >= 0; --js) {
-                uint32_t *t = SA(tempS, js, lane);
+                const PS t(tempS, js, lane);
                 uint32_t CNT[NC], SYC[NY], Sraw, HOT, Fm, pk;
-                if (kDefault) {
-                    const uint4 a = *reinterpret_cast<const uint4 *>(t), b4 = *reinterpret_cast<const uint4 *>(t + 128);
-                    CNT[0] = a.x; CNT[1] = a.y; CNT[2] = a.z; SYC[0] = a.w; Sraw = b4.x; HOT = b4.y; Fm = b4.z; pk = b4.w;
-                } else {
-#pragma unroll
-                    for (int q = 0; q < NC; ++q) CNT[q] = t[q];
-#pragma unroll
-                    for (int q = 0; q < NY; ++q) SYC[q] = t[4 + q];
-                    Sraw = t[I_S]; HOT = t[I_H]; Fm = t[I_F]; pk = t[I_K];
-                }
+                t.load_a(CNT, SYC, Sraw, HOT, Fm, pk);
                 const int n = pk_n(pk), c0 = pk_c0(pk);
                 const uint32_t REAL = real_mask(js, n);
                 const uint32_t OWN = range_mask(c0, c_lo, c_hi) & REAL;
@@ -739,26 +791,18 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 const uint32_t SPq = SPLIT & mask_lt(n) & range_mask(c0, c_lo, closed ? c_hi + 1 : c_hi);
                 const unsigned hs = __ballot_sync(FULL, SPq != 0u);
                 const int firstsp = __shfl_sync(FULL, c0 + __ffs(SPq) - 1, hs ? __ffs(hs) - 1 : 0);
-                if (lane == 0) { ctl.tokstep[tw][buf][js] = tot; ctl.nsa[tw][buf][js] = nsa_carry; }
+                if (lane == 0) { ctl.tokstep[w][buf][js] = tot; ctl.nsa[w][buf][js] = nsa_carry; }
                 if (hs) nsa_carry = firstsp;
                 const uint32_t FO = Fm & OWN;
                 if (FO) lft_max = max(lft_max, c0 + 31 - __clz(FO));
-                // state for pass D, in place
-                const uint32_t pk2 = (pk & 0xC007FFFFu) | ((uint32_t)(ts - mytok) << 19);
-                const uint32_t leadw = sbmS[js * 32 + lane];      // the window's map is rebuilt by the next analysis: keep the mask here
-                if (kDefault) {
-                    *reinterpret_cast<uint4 *>(t) = make_uint4(V[0], V[1], V[2], E);
-                    t[SW(I_H)] = leadw; t[SW(I_K)] = pk2;
-                } else {
-#pragma unroll
-                    for (int q = 0; q < NV; ++q) t[q] = V[q];
-                    t[I_E] = E; t[I_H] = leadw; t[I_K] = pk2;
-                }
+                // state for pass D (the window's map is rebuilt by the next analysis: the lead mask moves into the state)
+                t.store_c(V, E, sbmS[js * 32 + lane], (pk & 0xC007FFFFu) | ((uint32_t)(ts - mytok) << 19));
             }
             lft = __reduce_max_sync(FULL, lft_max);
         }
-        finish();
+        const RangeRec a = finish();
         PROF5(3);
+        return a;
     };
 
     // =================================================================================================
@@ -769,14 +813,14 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
             const int s = k & 1;
             int n = 0, ntok = 0, lft_rel = -1;
             // lane i < NW: what range i posted with its FIRST analysis (nothing entering): backlog left (sf0), flags,
-            // and -- only for ranges that begin inside a chunk (flag 4 clear) -- marks - closers (su; NEG: a string
+            // and -- only for ranges that begin inside a chunk (LO_FOUND clear) -- marks - closers (su; NEG: a string
             // boundary resets the backlog) and the marks in front of the first closer (smb1) ...
-            int su = 0, sf0 = 0, smb1 = 0, sflags = 2 | 4;
+            int su = 0, sf0 = 0, smb1 = 0, sflags = RangeRec::CLOSED | RangeRec::LO_FOUND;
             // ... what it has been analysed with so far, and the backlog it left the last time
             int x_used = 0, far_used = 0, v_last = 0;
-            // tile totals from what the ranges have posted (ctl.wagg)
+            // tile totals from what the ranges have posted (ctl.rec)
             auto sum_up = [&](bool first) {
-                const WAgg a = ctl.wagg[s][lane < NW ? lane : 0];
+                const RangeRec a = ctl.rec[s][lane < NW ? lane : 0];
                 const int mn = lane < NW ? a.n_own : 0, mk = lane < NW ? a.ntok : 0;
                 int pn = mn;                                   // inclusive prefix of characters over the ranges
 #pragma unroll
@@ -789,7 +833,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 lft_rel = hl ? lv : -1;
                 if (first && lane < NW) {
                     su = a.u; sf0 = a.v; smb1 = a.mb1; sflags = a.flags; v_last = a.v;
-                    far_used = (a.flags & 16) ? 1 : 0;      // (what a range that ends inside a chunk guessed in its first analysis)
+                    far_used = (a.flags & RangeRec::GUESSED_HOT) ? 1 : 0;
                 }
             };
             // Backlog entering / hot tail of every range, given the backlog `x_tile` that enters the tile.  A range whose
@@ -802,7 +846,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
             // Returns the backlog leaving the tile.
             auto resolve = [&](int x_tile) -> int {
                 // nothing enters, nothing is left, every range ends at a closer: almost every tile
-                if (x_tile == 0 && !__any_sync(FULL, lane < NW && (sflags & 1) != 0 && (sf0 != 0 || (sflags & 2) == 0 || x_used != 0)))
+                if (x_tile == 0 && !__any_sync(FULL, lane < NW && (sflags & RangeRec::HAVE) != 0 &&
+                                                          (sf0 != 0 || (sflags & RangeRec::CLOSED) == 0 || x_used != 0)))
                     return 0;
                 const long long tile_w = ld_vs32(&ctl.tile_id[s]);
                 int x_out = x_tile;
@@ -815,8 +860,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                         const int xu = __shfl_sync(FULL, x_used, i), vl = __shfl_sync(FULL, v_last, i);
                         if (lane == i) { xin = x; kin = known; }
                         if (known) {
-                            if ((fl & 1) == 0) { /* no data: passes the backlog on */ }
-                            else if ((fl & 4) == 0) x = max(x + ui, fi);
+                            if ((fl & RangeRec::HAVE) == 0) { /* no data: passes the backlog on */ }
+                            else if ((fl & RangeRec::LO_FOUND) == 0) x = max(x + ui, fi);
                             else if (x == 0) x = fi;
                             else if (x == xu) x = vl;                 // it has been analysed with exactly this backlog
                             else known = false;
@@ -825,13 +870,14 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     }
                     x_out = x;
                     const bool all_known = known;
-                    const bool have = lane < NW && (sflags & 1) != 0;
-                    const bool open = have && (sflags & 2) == 0;           // the range ends inside a chunk
+                    const bool have = lane < NW && (sflags & RangeRec::HAVE) != 0;
+                    const bool open = have && (sflags & RangeRec::CLOSED) == 0;           // the range ends inside a chunk
                     int far = far_used;
                     bool walk = false;
                     {
-                        const unsigned Bm = __ballot_sync(FULL, lane < NW && smb1 > 0), Bc = __ballot_sync(FULL, lane < NW && (sflags & 8) != 0);
-                        const unsigned Bn = __ballot_sync(FULL, lane < NW && (sflags & 1) == 0);
+                        const unsigned Bm = __ballot_sync(FULL, lane < NW && smb1 > 0);
+                        const unsigned Bc = __ballot_sync(FULL, lane < NW && (sflags & RangeRec::HOLDS_CLOSER) != 0);
+                        const unsigned Bn = __ballot_sync(FULL, lane < NW && (sflags & RangeRec::HAVE) == 0);
                         if (open && kend) {
                             far = 0;
                             if (xend > 0) far = 1;
@@ -851,7 +897,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     // the backlog that enters matters where there is a closer to meet it (a range without a summary -- it begins
                     // at a closer -- is assumed to hold one); a range that lies inside one chunk only needs to know whether
                     // that chunk will be closed hot
-                    const bool x_matters = (sflags & 4) != 0 || (sflags & 8) != 0;
+                    const bool x_matters = (sflags & (RangeRec::LO_FOUND | RangeRec::HOLDS_CLOSER)) != 0;
                     const bool need = have && kin && ((xin != x_used && x_matters) || far != far_used);
                     unsigned todo = __ballot_sync(FULL, need);
                     if (!todo) {
@@ -861,24 +907,22 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     {   // (statistics: repeat rounds, ranges repeated, of those because of the hot-tail guess)
                         const unsigned fb = __ballot_sync(FULL, need && far != far_used);
                         if (lane == 0) {
-                            atomicAdd(&p.result->prof[9], 1ull); atomicAdd(&p.result->prof[8], (unsigned long long)__popc(todo));
-                            atomicAdd(&p.result->prof[7], (unsigned long long)__popc(fb));
+                            atomicAdd(&p.result->stats.repeat_rounds, 1ull); atomicAdd(&p.result->stats.ranges_repeated, (unsigned long long)__popc(todo));
+                            atomicAdd(&p.result->stats.repeats_hot_tail, (unsigned long long)__popc(fb));
                         }
                     }
                     if (need) { x_used = xin; far_used = far; }
                     while (todo) {
                         const int i = __ffs(todo) - 1; todo &= todo - 1;
                         const int xi = __shfl_sync(FULL, xin, i), fi = __shfl_sync(FULL, far, i);
-                        tw = i;
                         const long long r = tile_w * NW + i;
-                        plain_load(r, s);
-                        build_map(r);
-                        analyze(r, s, xi, fi);
-                        if (lane == 0) {                       // (flags and summary stand: they do not depend on what enters)
-                            WAgg &a = ctl.wagg[s][i];
-                            a.n_own = a_n_own; a.ntok = a_ntok; a.lft = a_lft; a.v = a_v;
+                        plain_load(r, i, s);
+                        build_map(r, i);
+                        const RangeRec a = analyze(r, s, i, xi, fi);
+                        if (lane == 0) {                       // (the rest does not depend on what enters the range)
+                            ctl.rec[s][i].ntok = a.ntok; ctl.rec[s][i].v = a.v;
                         }
-                        if (lane == i) v_last = a_v;
+                        if (lane == i) v_last = a.v;
                     }
                     __threadfence_block();
                     __syncwarp();
@@ -894,7 +938,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
             // A tile that begins inside a chunk (a long space-free run is passing through) most likely does get one: it
             // publishes nothing before it knows (its successors would have to wait for its inclusive prefix anyway) and
             // settles once, with the backlog that really enters.
-            const bool begins_inside = tile > 0 && (__shfl_sync(FULL, sflags, 0) & 5) == 1;
+            const bool begins_inside = tile > 0 && (__shfl_sync(FULL, sflags, 0) & (RangeRec::HAVE | RangeRec::LO_FOUND)) == RangeRec::HAVE;
             int v = 0;
             if (!begins_inside) {
                 v = resolve(0);
@@ -913,7 +957,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
 #endif
                 v = resolve(pre.x);
 #ifdef LATOK_PROFILE
-                if (lane == 0) { atomicAdd(&p.result->prof[10], (unsigned long long)(clock64() - _s1)); atomicAdd(&p.result->prof[11], 1ull); }
+                if (lane == 0) { atomicAdd(&p.result->clocks.resolve, (unsigned long long)(clock64() - _s1)); atomicAdd(&p.result->clocks.resolve_calls, 1ull); }
 #endif
             }
             if (lane == 0) {
@@ -942,20 +986,23 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
 
     // ================================================================================================= output
     auto output = [&](const long long r, const int buf, unsigned long long G_in, unsigned long long K_in, unsigned long long base_in) {
-        const RInfo ri = ctl.rinfo[cw][buf];
-        const bool have = (ri.flags & 1) != 0, closed = (ri.flags & 2) != 0, lo_found = (ri.flags & 4) != 0, last_range = (ri.flags & 8) != 0;
+        const RangeRec ri = ctl.rec[buf][cw];
+        const bool have = (ri.flags & RangeRec::HAVE) != 0, closed = (ri.flags & RangeRec::CLOSED) != 0;
+        const bool lo_found = (ri.flags & RangeRec::LO_FOUND) != 0;
+        // (the last range is tested as r == p.nranges - 1 where it matters: r stays live anyway, a bool held across pass D
+        // costs the token-feature instantiation spills)
         if (!have) return;
         const int c_lo = ri.c_lo, c_hi = ri.c_hi, n_own = ri.n_own, ntok_range = ri.ntok;
         const long long w0 = r * (long long)RANGE;
         const long long rem64 = p.n_bytes - w0;
         const int nb_win = rem64 > (long long)(WIN + 64) ? WIN + 64 : (int)rem64;
-        const uint32_t *tempS = tempof(buf);
+        uint32_t *tempS = tempof(cw, buf);
         if (K_in + (unsigned long long)ntok_range > (unsigned long long)p.cap_tokens && lane == 0) atomicOr(&p.result->error, 4u);
         if (G_in + (unsigned long long)n_own > (unsigned long long)p.n_bytes || K_in + (unsigned long long)ntok_range > (unsigned long long)p.n_bytes + 1ull) {
             if (lane == 0 && atomicOr(&p.result->error, 8u) == 0u) {
-                p.result->prof[8] = (unsigned long long)r; p.result->prof[9] = G_in; p.result->prof[10] = K_in;
-                p.result->prof[11] = (unsigned long long)(long long)n_own; p.result->prof[12] = (unsigned long long)(long long)ntok_range;
-                p.result->prof[13] = (unsigned long long)(long long)c_lo; p.result->prof[14] = (unsigned long long)(long long)c_hi;
+                FaultRec &f = p.result->fault;
+                f.range = (unsigned long long)r; f.G_in = G_in; f.K_in = K_in;
+                f.n_own = n_own; f.ntok = ntok_range; f.c_lo = c_lo; f.c_hi = c_hi;
             }
             return;
         }
@@ -991,11 +1038,11 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 if (in) {
                     const int wb = int(o - w0);
                     const int js = wb >> 10, tl = (wb >> 5) & 31;
-                    const uint32_t *t = SA(const_cast<uint32_t *>(tempS), js, tl);
-                    const uint32_t l_pk = t[SW(I_K)], l_E = t[SW(I_E)], l_lead = t[SW(I_H)];
+                    const PS t(tempS, js, tl);
+                    const uint32_t l_pk = t.packed(), l_E = t.e(), l_lead = t.lead();
                     const int l_c0 = pk_c0(l_pk);
                     const int c = l_c0 + __popc(l_lead & mask_lt_nn(wb & 31));
-                    const bool mine = last_range ? (c >= c_lo) : (c >= c_lo && c < c_hi);
+                    const bool mine = r == p.nranges - 1 ? (c >= c_lo) : (c >= c_lo && c < c_hi);
                     if (mine) {
                         int kb = 0;
                         for (int q2 = 0; q2 < js; ++q2) kb += ctl.tokstep[cw][buf][q2];
@@ -1008,16 +1055,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         }
 #pragma unroll 1
         for (int js = 0; js < RS; ++js) {
-            const uint32_t *t = SA(const_cast<uint32_t *>(tempS), js, lane);
             uint32_t V[NV], E, Sraw, Fm, pk;
-            if (kDefault) {
-                const uint4 a = *reinterpret_cast<const uint4 *>(t), b4 = *reinterpret_cast<const uint4 *>(t + 128);
-                V[0] = a.x; V[1] = a.y; V[2] = a.z; E = a.w; Sraw = b4.x; Fm = b4.z; pk = b4.w;
-            } else {
-#pragma unroll
-                for (int q = 0; q < NV; ++q) V[q] = t[q];
-                E = t[I_E]; Sraw = t[I_S]; Fm = t[I_F]; pk = t[I_K];
-            }
+            PS(tempS, js, lane).load_c(V, E, Sraw, Fm, pk);
             const int n = pk_n(pk), c0 = pk_c0(pk), tp = pk_tp(pk);
             const int wrel = nb_win - (js * STEP + lane * 32);          // data bytes from this lane-word on
             const bool has_term = (unsigned)wrel < 32u;
@@ -1205,7 +1244,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     const uint32_t PSr = (Sraw << 1) | pk_ps(pk);
                     // (a range that ends at a closer also answers for the character after it: the next range begins at a
                     // closer then and does not come here -- a token that covers this whole range may end exactly there)
-                    const uint32_t END = SPLIT & ~PSr & mask_lt(n) & range_mask(c0, c_lo, (last_range || closed) ? c_hi + 1 : c_hi);
+                    const uint32_t END = SPLIT & ~PSr & mask_lt(n) & range_mask(c0, c_lo, (r == p.nranges - 1 || closed) ? c_hi + 1 : c_hi);
                     if (END) {
                         const int i = __ffs(END) - 1;
                         if (ktok + tp + __popc(E & mask_lt(i)) == 0) {
@@ -1302,7 +1341,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                         // (the lane-words of a warp hold between none and a dozen token ends: a loop of every lane over its own
                         // ones runs as long as the busiest lane, and its rows would leave the warp as scattered words).
                         // (1) every lane lists its token ends: lane-word, position, position of the split the token began at
-                        uint16_t *list = reinterpret_cast<uint16_t *>(SA(const_cast<uint32_t *>(tempS), js, 0));   // (the step's state has been read)
+                        uint16_t *list = PS::scratch(tempS, js);         // (the step's state has been read)
                         {
                             uint32_t e = ev; int idx = kr_first - kr0;
                             while (e) {
@@ -1447,7 +1486,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 st_rec(o, make_uint4(fc_hit ? 1u : 0u, p.epoch, 0u, 0u));
             }
         }
-        if (last_range && lane == 0) {
+        if (r == p.nranges - 1 && lane == 0) {
             p.result->n_chars = G_in + (unsigned long long)n_own;
             p.result->n_tokens = K_in + (unsigned long long)ntok_range;
         }
@@ -1475,10 +1514,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         }
         return __shfl_sync(FULL, t, 0);
     };
-    auto post = [&](int s) {
+    auto post = [&](int s, const RangeRec &a) {
         if (lane == 0) {
-            WAgg &a = ctl.wagg[s][cw];
-            a.n_own = a_n_own; a.ntok = a_ntok; a.lft = a_lft; a.v = a_v; a.flags = a_flags; a.u = a_u; a.mb1 = a_mb1;
+            ctl.rec[s][cw] = a;
             __threadfence_block();
         }
         __syncwarp();
@@ -1501,7 +1539,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         unsigned long long G_in, K_in, base_in;
         {
             const Slot sl = ctl.slot[s];
-            const WAgg a = ctl.wagg[s][lane < NW ? lane : 0];
+            const RangeRec a = ctl.rec[s][lane < NW ? lane : 0];
             const bool before = lane < cw;
             const int pn = __reduce_add_sync(FULL, before ? a.n_own : 0), pkk = __reduce_add_sync(FULL, before ? a.ntok : 0);
             int pnx = lane < NW ? a.n_own : 0;            // exclusive prefix of characters per range
@@ -1527,12 +1565,11 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
     for (int k = 0;; ++k) {
         const int s = k & 1;
         if (tile_cur < ntiles_i) {
-            build_map((long long)tile_cur * NW + cw);
+            build_map((long long)tile_cur * NW + cw, cw);
             if (s == 0 ? pending[0] : pending[1]) wait_window(s, phase_bits);
             __syncwarp();
             PROF5(0);
-            analyze((long long)tile_cur * NW + cw, s, 0, -1);
-            post(s);
+            post(s, analyze((long long)tile_cur * NW + cw, s, cw, 0, -1));
         } else {
             nb_arrive(BAR_AGG + s, NTH);                 // tells the service warp that the tickets have run out
         }
@@ -1575,16 +1612,20 @@ static int ctas_one(const TableLayout &tl)
 template <class Geom>
 int ctas_per_sm(const TableLayout &tl, bool is_default, bool want_feats)
 {
-    if (is_default) return want_feats ? ctas_one<Geom, true, true>(tl) : ctas_one<Geom, true, false>(tl);
-    return want_feats ? ctas_one<Geom, false, true>(tl) : ctas_one<Geom, false, false>(tl);
+    if constexpr (Geom::FEATS) {
+        if (want_feats) return is_default ? ctas_one<Geom, true, true>(tl) : ctas_one<Geom, false, true>(tl);
+    } else if (want_feats) return 0;                          // no such instantiation (tokenize5_plan never asks for it)
+    return is_default ? ctas_one<Geom, true, false>(tl) : ctas_one<Geom, false, false>(tl);
 }
 
 template <class Geom>
 cudaError_t launch(const Params &p, int grid, cudaStream_t s)
 {
     const bool feats = (p.what & 4u) != 0u;
-    if (p.rules.is_default) return feats ? launch_one<Geom, true, true>(p, grid, s) : launch_one<Geom, true, false>(p, grid, s);
-    return feats ? launch_one<Geom, false, true>(p, grid, s) : launch_one<Geom, false, false>(p, grid, s);
+    if constexpr (Geom::FEATS) {
+        if (feats) return p.rules.is_default ? launch_one<Geom, true, true>(p, grid, s) : launch_one<Geom, false, true>(p, grid, s);
+    } else if (feats) return cudaErrorInvalidValue;
+    return p.rules.is_default ? launch_one<Geom, true, false>(p, grid, s) : launch_one<Geom, false, false>(p, grid, s);
 }
 
 extern template int ctas_per_sm<LongGeometry>(const TableLayout &, bool, bool);

@@ -21,7 +21,8 @@ TILE = 7936
 @pytest.fixture(scope="module", params=["auto", "long", "short"])
 def engine(request):
     """Every test of this module runs three times: with the geometry the library picks for the batch (by average string
-    length), and with each of the two forced (LATOK_B200_GEOMETRY is read at every submit)."""
+    length), and with each of the two forced (LATOK_B200_GEOMETRY is read at every submit).  A batch with token features
+    runs in the long geometry whatever is forced: the short one is not built with them."""
     import os
     from latok_b200.engine import Engine
     old = os.environ.pop("LATOK_B200_GEOMETRY", None)

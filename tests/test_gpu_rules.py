@@ -74,7 +74,8 @@ CLOSER_ROWS = {
 @pytest.fixture(scope="module", params=["long", "short"])
 def engine(request):
     """Every test of this module runs with each geometry of the kernel forced (LATOK_B200_GEOMETRY is read at every
-    submit); the sweeps use that geometry's range and tile sizes."""
+    submit); the sweeps use that geometry's range and tile sizes.  A batch with token features runs in the long geometry
+    whatever is forced: the short one is not built with them."""
     from latok_b200.engine import Engine
     old = os.environ.pop("LATOK_B200_GEOMETRY", None)
     os.environ["LATOK_B200_GEOMETRY"] = request.param

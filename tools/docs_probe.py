@@ -2,9 +2,10 @@
 """Cost of the irregular tiles of the long-document corpus (development aid; run under gpurun):
 clean documents, then the same with k documents given a 32 KB space-free run / a 300-byte multi-mark stretch.
    LATOK_B200_PRINT_PROF=1 python tools/docs_probe.py
-The [latok prof] line printed per launch holds the kernel's statistics counters: [7] ranges repeated because the guess
-about a hot tail was wrong, [8] ranges repeated, [9] repeat rounds, [12] analyses of ranges that begin inside a chunk,
-[13] ... that end inside one, [14] ranges that leave a backlog, [15] look-back restarts."""
+The [latok prof] line printed per launch holds the kernel's statistics counters (Result::stats): repeat_rounds,
+ranges_repeated, repeats_hot_tail (ranges repeated because the guess about a hot tail was wrong), open_head / open_tail
+(analyses of ranges that begin / end inside a chunk), backlog_out (ranges that leave a backlog), lookback_restarts, and the
+look-ahead walks; a LATOK_PROFILE build adds the phase clocks (Result::clocks)."""
 import sys; sys.path.insert(0, '.'); sys.path.insert(1, 'tests')
 import numpy as np, ctypes as C
 from latok_b200 import _lib
