@@ -19,8 +19,8 @@ LIB = PKG / "liblatok_b200.so"
 # compiled in parallel, each once; latok_tok5.cu and latok_tok5_short.cu hold the tokenize kernel's two geometries
 SOURCES = [CSRC / "latok_kernels.cu", CSRC / "latok_tok5.cu", CSRC / "latok_tok5_short.cu", CSRC / "latok_tokbytes.cu",
            CSRC / "latok_vocab.cu", CSRC / "latok_capi.cu", CSRC / "latok_reader.cpp"]
-HEADERS = [CSRC / "latok_internal.h", CSRC / "latok_bits.h", CSRC / "latok_device.cuh", CSRC / "latok_tok5.cuh",
-           ROOT / "include" / "latok_b200.h"]
+HEADERS = [CSRC / "latok_internal.h", CSRC / "latok_bits.h", CSRC / "latok_device.cuh", CSRC / "latok_chain.cuh",
+           CSRC / "latok_tok5.cuh", ROOT / "include" / "latok_b200.h"]
 GEN = CSRC / "_gen" / "latok_tables.h"
 RANGES = PKG / "data" / "ucd11_latok_classes.txt"
 

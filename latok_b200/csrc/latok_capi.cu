@@ -393,7 +393,7 @@ static int run_device(latok_b200_engine *e, Batch &b)
     const bool feats = (b.what & LATOK_B200_FEATS) != 0;
     const Tok5Plan t5 = tokenize5_plan(b.n_bytes, b.n_strings, feats, e->tl, b.rules.is_default != 0, e->n_sm);
     if (int r = b.d_first.ensure((size_t)t5.nranges + 1)) return r;
-    // the status word of every aggregate record carries the launch epoch, so records are zeroed only when (re)allocated
+    // aggregate and open-sums records carry the launch epoch, so they are zeroed only when (re)allocated and when it wraps
     // (agg / inc / osum / planes are shared by the two sets: tokenize kernels run one after the other on one stream)
     if ((size_t)t5.ntiles > e->agg.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->agg.ensure((size_t)t5.ntiles, true)) return r; }
     if ((size_t)t5.ntiles > e->inc.cap) { CU(cudaStreamSynchronize(e->stream)); if (int r = e->inc.ensure((size_t)t5.ntiles)) return r; }
@@ -407,9 +407,10 @@ static int run_device(latok_b200_engine *e, Batch &b)
     if (b.what & LATOK_B200_MATRIX) { if (int r = b.d_matrix.ensure(((size_t)b.n_bytes + 64) * NFEAT)) return r; }
     if (b.what & LATOK_B200_SPANS16) { if (int r = b.d_spans16.ensure(b.d_spans.cap / 2)) return r; }
 
-    e->epoch = (e->epoch + 1) & 0x3FFFFFFFu;
-    if (e->epoch == 0) {  // wrapped: clear stale status words
+    e->epoch = (e->epoch + 1) & EPOCH_MASK;
+    if (e->epoch == 0) {  // wrapped: clear every epoch-stamped record, so that no record of an earlier launch can match
         CU(cudaMemsetAsync(e->agg.p, 0, e->agg.cap * sizeof(AggRec), e->stream));
+        if (e->osum.cap) CU(cudaMemsetAsync(e->osum.p, 0, e->osum.cap * sizeof(OpenSums), e->stream));
         e->epoch = 1;
     }
     Params p;

@@ -1,6 +1,7 @@
-// latok_device.cuh -- device helpers shared by the kernels (latok_tok5.cuh: tokenize; latok_kernels.cu: parse matrix;
-// latok_tokbytes.cu: token byte ranges): PTX wrappers, Unicode class look-up, the context features, the scalar rule
-// evaluation used on rare paths, the look-ahead walk and the decoupled look-back.
+// latok_device.cuh -- device helpers of the kernels (latok_tok5.cuh: tokenize; latok_kernels.cu: parse matrix;
+// latok_tokbytes.cu: token byte ranges): PTX wrappers, Unicode class look-up, the context features, the block-mask mark
+// test and the backlog functions.  What crosses between the CTAs of the tokenize kernel (the look-back chain) is that
+// kernel's own, in latok_chain.cuh; its look-ahead walk is in latok_tok5.cuh.
 #pragma once
 #include "latok_internal.h"
 #include "latok_bits.h"
@@ -8,7 +9,6 @@
 namespace latok {
 
 constexpr int NEG = -(1 << 28);           // "-infinity" of the (max,+) backlog functions
-constexpr unsigned SPIN_LIMIT = 1u << 23; // watchdog for look-back spins
 
 // ---- small helpers ------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t mask_lt(int k) { return __funnelshift_lc(0xFFFFFFFFu, 0u, (unsigned)max(k, 0)); }  // low k bits (k clamped to 0..32)
@@ -136,255 +136,6 @@ __device__ __forceinline__ bool rule_mark(const RuleSet &rules, uint32_t w)
 
 // 4 feature bits -> 4 byte counters (bit k -> byte k)
 __device__ __forceinline__ uint32_t spread4(uint32_t nib) { return (nib * 0x00204081u) & 0x01010101u; }
-
-// ---- look-ahead walk (rare): the whitespace chunk open at the end of a tile did not close inside
-// the right halo.  Warp 0 scans forward from global byte `pos0` until the chunk closes (a SPACE
-// character or the end of the string) and reports whether a mark occurs up to and including the
-// closing character.  Exact but slow; it exists so that arbitrarily long space-free runs stay
-// bit-exact (latok.c:218-244 has unbounded reach).
-static __device__ bool walk_ahead(const Params &p, const Tables &t, long long pos0, int lane)
-{
-    const uint8_t *in = p.in;
-    // end of the string that contains pos0: first offset > pos0 (32 probes per round)
-    long long e;
-    {
-        long long lo = 0, hi = p.n_strings;              // the answer is in [lo, hi]; offsets[n_strings] = n_bytes > pos0
-        while (lo < hi) {
-            const long long step = (hi - lo + 31) / 32;
-            const long long c = lo + step * lane;
-            const bool gt = c >= hi || p.offsets[c] > pos0;       // monotone over the lanes
-            const unsigned b = __ballot_sync(0xFFFFFFFFu, gt);
-            if (b == 0u) lo = lo + 31 * step + 1;
-            else {
-                const int f = __ffs(b) - 1;
-                const long long nh = lo + step * f;
-                if (f > 0) lo = lo + step * (f - 1) + 1;
-                hi = nh < hi ? nh : hi;
-            }
-        }
-        e = p.offsets[lo];
-    }
-    struct G { const uint8_t *in; long long q, n; __device__ uint32_t operator[](int k) const { long long a = q + k; return a < n ? (uint32_t)in[a] : 0u; } };
-    // the character in front of pos0 (we are strictly inside the string, so it exists)
-    uint32_t prev_w;
-    {
-        long long pp = pos0 - 1;
-        for (int k = 0; k < 8 && pp > 0 && (in[pp] & 0xC0u) == 0x80u; ++k) --pp;
-        prev_w = classify_at(G{in, pp, p.n_bytes}, t);
-    }
-    // 32 bytes per trip, one byte per lane; the rules are evaluated for the characters that begin in the first ZONE
-    // bytes (their next and after-next characters begin inside the 32 bytes), then the window moves on by ZONE
-    constexpr int ZONE = 24, AHEAD = 4;
-    bool any = false;
-    for (long long q0 = pos0; q0 < e; q0 += AHEAD * ZONE) {
-      // the bytes of AHEAD windows are fetched together (the walk runs into text nobody has touched yet: DRAM latency)
-      uint32_t bytes[AHEAD];
-#pragma unroll
-      for (int g = 0; g < AHEAD; ++g) {
-          const long long pos = q0 + g * ZONE + lane;
-          bytes[g] = pos < e ? (uint32_t)in[pos] : 0x80u;
-      }
-#pragma unroll
-      for (int g = 0; g < AHEAD; ++g) {
-        const long long q = q0 + g * ZONE;
-        if (q >= e) break;
-        const long long pos = q + lane;
-        const bool inb = pos < e;
-        const uint32_t byte = bytes[g];
-        const bool lead = inb && (byte & 0xC0u) != 0x80u;
-        const unsigned leads = __ballot_sync(0xFFFFFFFFu, lead);
-        uint32_t w = 0;
-        if (lead) w = byte < 0x80u ? (uint32_t)t.ascii_feat[byte] : classify_at(G{in, pos, p.n_bytes}, t);
-        const unsigned above = lane == 31 ? 0u : (leads & (0xFFFFFFFFu << (lane + 1)));
-        const unsigned above2 = above & (above - 1u);
-        const unsigned below = leads & ((1u << lane) - 1u);
-        const uint32_t nw = __shfl_sync(0xFFFFFFFFu, w, above ? __ffs(above) - 1 : 0);
-        const uint32_t aw = __shfl_sync(0xFFFFFFFFu, w, above2 ? __ffs(above2) - 1 : 0);
-        uint32_t pw = __shfl_sync(0xFFFFFFFFu, w, below ? 31 - __clz(below) : 0);
-        if (!below) pw = prev_w;
-        const bool has_next = above != 0u, has_an = above2 != 0u;
-        bool closer = false, mk = false;
-        const bool ev = lead && lane < ZONE;
-        if (ev) {
-            const uint32_t full = make_word(pw, w, nw, aw, false, !has_next, !has_an);
-            mk = rule_mark(p.rules, full);
-            closer = ((full >> 5) & 1u) || !has_next;
-        }
-        const unsigned bc = __ballot_sync(0xFFFFFFFFu, ev && closer), bm = __ballot_sync(0xFFFFFFFFu, ev && mk);
-        if (bc) {
-            const int first = __ffs(bc) - 1;
-            return any || (bm & (first == 31 ? 0xFFFFFFFFu : ((2u << first) - 1u))) != 0u;
-        }
-        any = any || bm != 0u;
-        if (any) return true;
-        const unsigned zone = leads & ((1u << ZONE) - 1u);
-        if (zone) prev_w = __shfl_sync(0xFFFFFFFFu, w, 31 - __clz(zone));
-      }
-    }
-    return any;
-}
-
-// =====================================================================================================
-// Decoupled look-back (single chain, 16-byte aggregate records, LB_WINDOW predecessors per step)
-// =====================================================================================================
-constexpr int LB_PER_LANE = 2;
-constexpr int LB_WINDOW = 32 * LB_PER_LANE;
-
-__device__ __forceinline__ uint4 ld_rec(const void *p)
-{
-    uint4 r;
-    asm volatile("ld.relaxed.gpu.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-    return r;
-}
-__device__ __forceinline__ void st_rec(void *p, uint4 v)
-{
-    asm volatile("st.relaxed.gpu.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
-struct Prefix { unsigned long long G, base, K; int x; };
-
-// spin until tile `idx` has published at least `min_state` for this launch; returns the record
-__device__ __forceinline__ uint4 wait_rec(const AggRec *agg, long long idx, unsigned epoch, unsigned min_state, Result *result, bool &ok)
-{
-    uint4 r;
-    unsigned spins = 0;
-    for (;;) {
-        r = ld_rec(agg + idx);
-        if ((r.x >> 2) == epoch && (r.x & 3u) >= min_state) break;
-        if (++spins > SPIN_LIMIT || (((spins & 1023u) == 0u) && ld_volatile_u32(&result->abort_flag))) {
-            atomicOr(&result->error, 1u);
-            st_volatile_u32(&result->abort_flag, 1u);
-            ok = false;
-            break;
-        }
-    }
-    return r;
-}
-
-// Exclusive prefix of `tile` (warp 0, all lanes).  Walks back LB_WINDOW tiles at a time until it meets an
-// inclusive prefix.  An aggregate is only valid for a tile that no block-mask backlog enters, i.e. when the
-// inclusive prefix it is chained to carries no backlog and every aggregate between them leaves none
-// (backlog-out for backlog-in 0 is stored in the record).  If that does not hold (rare: a whitespace chunk
-// with several marks, or a chunk longer than the halo) the walk waits for the inclusive prefix of the tile
-// right after the offending one -- that tile recomputes with its real backlog -- and starts over.
-static __device__ Prefix lookback(long long tile, const Params &p, int lane)
-{
-    Prefix out;
-    out.G = 0; out.base = 0; out.K = 0; out.x = 0;
-    if (tile == 0) return out;
-    for (int restart = 0;; ++restart) {
-        unsigned long long sum_n = 0, sum_k = 0;     // characters / tokens of the consumed aggregates
-        unsigned long long lf_part = 0; bool lf_found = false;
-        long long viol = -1;                         // newest tile whose successor's aggregate must not be used
-        int x_in = 0; bool x_set = false;
-        bool ok = true, done = false;
-        for (long long newest = tile - 1; !done; newest -= LB_WINDOW) {
-            // lane l covers tiles first .. first + LB_PER_LANE - 1 (older lanes = older tiles)
-            const long long first = newest - (long long)(31 - lane) * LB_PER_LANE - (LB_PER_LANE - 1);
-            int rj = -1;                              // newest inclusive element of this lane
-            unsigned long long rG = 0, rB = 0, rK = 0; int rx = 0;
-            unsigned ln = 0, lk = 0, llf = 0; bool lhas = false; long long lviol = -1; int lastv = 0;
-#ifdef LATOK_PROFILE
-            long long _lt0 = clock64();
-#endif
-            // all records of this lane in flight at once; re-poll only the ones not yet published
-            uint4 rec[LB_PER_LANE];
-#pragma unroll
-            for (int j = 0; j < LB_PER_LANE; ++j) { rec[j] = make_uint4(0, 0, 0, 0); if (first + j >= 0) rec[j] = ld_rec(p.agg + (first + j)); }
-            {
-                unsigned spins = 0;
-                for (;;) {
-                    bool pending = false;
-#pragma unroll
-                    for (int j = 0; j < LB_PER_LANE; ++j)
-                        if (first + j >= 0 && !((rec[j].x >> 2) == p.epoch && (rec[j].x & 3u) != 0u)) { rec[j] = ld_rec(p.agg + (first + j)); pending = true; }
-                    if (!pending) break;
-#ifdef LATOK_PROFILE
-                    if (lane == 31) atomicAdd(&p.result->clocks.lb_repolls, 1ull);
-#endif
-                    if (++spins > SPIN_LIMIT || (((spins & 1023u) == 0u) && ld_volatile_u32(&p.result->abort_flag))) {
-                        atomicOr(&p.result->error, 1u);
-                        st_volatile_u32(&p.result->abort_flag, 1u);
-                        ok = false;
-                        break;
-                    }
-                }
-            }
-#ifdef LATOK_PROFILE
-            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->clocks.lb_poll, (unsigned long long)(_t - _lt0)); _lt0 = _t; }
-#endif
-            // the newest inclusive record of this lane: fetch its prefix
-#pragma unroll
-            for (int j = 0; j < LB_PER_LANE; ++j) if (first + j >= 0 && (rec[j].x & 3u) == 2u) rj = j;
-            if (rj >= 0) {
-                __threadfence();
-                const IncRec *ir = p.inc + (first + rj);
-                const uint4 a = ld_rec(ir), b = ld_rec(reinterpret_cast<const uint4 *>(ir) + 1);
-                rG = a.x | ((unsigned long long)a.y << 32); rB = a.z | ((unsigned long long)a.w << 32);
-                rK = b.x | ((unsigned long long)b.y << 32); rx = (int)b.z;
-            }
-#pragma unroll
-            for (int j = 0; j < LB_PER_LANE; ++j) {
-                const long long idx = first + j;
-                if (idx < -1) continue;
-                if (idx == -1) { if (rj < 0) { rj = j; rG = rB = rK = 0; rx = 0; } continue; }
-                if (j <= rj) continue;                          // superseded by (or is) the inclusive record
-                const uint4 r = rec[j];
-                const unsigned n = r.y & 0xFFFFu, lf1 = r.y >> 16, k = r.z & 0xFFFFu; const int v = (int)(r.z >> 16);
-                if (lf1) { llf = ln + (lf1 - 1u); lhas = true; }
-                ln += n; lk += k;
-                if (v != 0 && idx != tile - 1) lviol = idx;      // its successor needs a real backlog
-                if (idx == tile - 1) lastv = v;
-            }
-            const unsigned has_reset = __ballot_sync(0xFFFFFFFFu, rj >= 0);
-            const int Lr = has_reset ? 31 - __clz(has_reset) : -1;
-#ifdef LATOK_PROFILE
-            if (lane == 0) { atomicAdd(&p.result->clocks.lb_windows, 1ull); if (Lr >= 0) atomicAdd(&p.result->clocks.lb_superseded, (unsigned long long)((31 - Lr) * LB_PER_LANE)); }
-#endif
-            const bool contrib = lane >= Lr;          // lanes older than the newest inclusive element are superseded
-            // characters / tokens
-            const unsigned wn = __reduce_add_sync(0xFFFFFFFFu, contrib ? ln : 0u), wk = __reduce_add_sync(0xFFFFFFFFu, contrib ? lk : 0u);
-            // newest string start among the consumed aggregates of this window
-            const unsigned hasm = __ballot_sync(0xFFFFFFFFu, contrib && lhas);
-            if (!lf_found && hasm) {
-                const int H = 31 - __clz(hasm);
-                const unsigned older = __reduce_add_sync(0xFFFFFFFFu, (contrib && lane < H) ? ln : 0u);
-                lf_part = (unsigned long long)older + __shfl_sync(0xFFFFFFFFu, llf, H);
-                lf_found = true;
-            } else if (lf_found) lf_part += wn;       // this whole window lies before the string start found earlier
-            sum_n += wn; sum_k += wk;
-            // newest offending tile of this window (64-bit max through two 32-bit reductions on the offset from `newest`)
-            const int voff = (contrib && lviol >= 0) ? (int)(newest - lviol) : 0x7FFFFFFF;   // smaller offset = newer
-            const int vmin = __reduce_min_sync(0xFFFFFFFFu, voff);
-            if (vmin != 0x7FFFFFFF && viol < 0) viol = newest - vmin;
-            if (!x_set) { x_in = __shfl_sync(0xFFFFFFFFu, lastv, 31); x_set = true; }
-            if (!__all_sync(0xFFFFFFFFu, ok)) { out.x = 0; return out; }    // watchdog tripped: error flag is set
-#ifdef LATOK_PROFILE
-            if (lane == 31) { long long _t = clock64(); atomicAdd(&p.result->clocks.lb_sum, (unsigned long long)(_t - _lt0)); }
-#endif
-            if (Lr >= 0) {
-                const unsigned long long G0 = __shfl_sync(0xFFFFFFFFu, rG, Lr), B0 = __shfl_sync(0xFFFFFFFFu, rB, Lr);
-                const unsigned long long K0 = __shfl_sync(0xFFFFFFFFu, rK, Lr);
-                const int x0 = __shfl_sync(0xFFFFFFFFu, rx, Lr);
-                const bool consumed_any = sum_n != 0 || sum_k != 0 || __shfl_sync(0xFFFFFFFFu, rj, Lr) != LB_PER_LANE - 1 || Lr != 31 || newest != tile - 1;
-                if (x0 != 0 && consumed_any && viol < 0) {
-                    // the inclusive prefix carries a backlog into the first consumed aggregate
-                    const long long ridx = newest - (long long)(31 - Lr) * LB_PER_LANE - (LB_PER_LANE - 1) + __shfl_sync(0xFFFFFFFFu, rj, Lr);
-                    viol = ridx;
-                }
-                out.G = G0 + sum_n; out.K = K0 + sum_k; out.base = lf_found ? G0 + lf_part : B0;
-                out.x = consumed_any ? x_in : x0;
-                done = true;
-            }
-        }
-        if (viol < 0) return out;
-        // wait for the tile after the offending one to publish its exact inclusive prefix, then walk again
-        bool ok2 = true;
-        wait_rec(p.agg, viol + 1, p.epoch, 2u, p.result, ok2);
-        if (lane == 0) atomicAdd(&p.result->stats.lookback_restarts, 1ull);
-        if (!ok2) return out;
-    }
-}
 
 __device__ __forceinline__ void nb_sync(int id, int cnt) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(cnt) : "memory"); }
 __device__ __forceinline__ void nb_arrive(int id, int cnt) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(cnt) : "memory"); }

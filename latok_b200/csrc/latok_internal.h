@@ -32,16 +32,19 @@ struct RuleSet {
     uint32_t sym[MAX_RULE_ROWS + 1];
 };
 
-// ---- decoupled look-back state (ONE chain) ----------------------------------------------------
+// ---- records that cross between the CTAs of the tokenize kernel (ONE look-back chain) ----------
 // Every tile publishes a 16-byte aggregate as soon as it has finished computing (state 1), computed
 // under the assumption that no block-mask backlog enters the tile (true for almost every tile), and
 // later its inclusive prefix (state 2).  A reader reconstructs the backlog entering each aggregate it
 // consumes; if that is non-zero it waits for that tile's inclusive prefix instead.
+// The device reads and writes these records only through the codec of latok_chain.cuh.  AggRec and OpenSums carry the
+// launch epoch (Params::epoch), so the host zeroes them only when they are allocated and when the epoch wraps.
+constexpr unsigned EPOCH_MASK = (1u << 30) - 1;   // launch epochs wrap at 2^30: AggRec::status keeps two bits for the state
 struct __align__(16) AggRec {
-    unsigned status;   // (epoch << 2) | state
-    unsigned n_lf;     // characters in the tile | (tile-relative index of the last string start + 1) << 16
-    unsigned ntok_v;   // tokens counted in the tile (backlog-in = 0) | backlog-out for backlog-in = 0 << 16
-    int u;             // backlog transfer function x -> max(x + u, v); NEG if the tile holds a string start
+    unsigned status;   // epoch << 2 | state (1: aggregate, 2: the inclusive prefix in IncRec too; another epoch: none yet)
+    unsigned n_lft;    // characters in the tile | (tile-relative index of its last string start + 1; 0: none) << 16
+    unsigned ntok_v;   // tokens in the tile | backlog it leaves << 16, both for no backlog entering it
+    unsigned pad;
 };
 struct __align__(16) IncRec {
     unsigned long long G;     // characters before the end of the tile
@@ -50,8 +53,14 @@ struct __align__(16) IncRec {
     int x;                    // backlog leaving the tile
     int pad;
 };
-// token-feature mode only: feature sums of the token still open at the end of a tile
-struct __align__(16) OpenSums { unsigned has_split; unsigned pad[3]; unsigned sums[8]; };
+// token-feature mode only, one per range: feature sums of the token still open at the end of the range
+struct __align__(16) OpenSums {
+    unsigned has_split;       // that token holds a split
+    unsigned epoch;           // the launch that published the record
+    unsigned pad[2];
+    unsigned sums[8];         // four uint8 sums per word, 25 features (sums[7] is 0)
+};
+static_assert(sizeof(AggRec) == 16 && sizeof(IncRec) == 32 && sizeof(OpenSums) == 48, "chain records are whole 16-byte words");
 
 // Statistics of the tokenize kernel's rare paths, counted in every build (LATOK_B200_PRINT_PROF prints them)
 struct KernelStats {

@@ -38,7 +38,7 @@
 //
 // No tensor cores: nothing here is a dense contraction; the bound is HBM bandwidth.
 #pragma once
-#include "latok_device.cuh"
+#include "latok_chain.cuh"
 
 namespace latok {
 namespace v5 {
@@ -74,11 +74,11 @@ struct Geometry {
     static constexpr int XBYTES = LPAD + WIN + 16;
     static constexpr int CTAS = 2;           // CTAs per SM the default-rules instantiation is compiled for
     static_assert(RANGE % 16 == 0, "geometry");
+    static_assert((NW - 1) * RANGE + WIN < 65536, "what a tile owns lies in its NW windows: its sums fit the 16-bit fields of AggRec");
 };
 using LongGeometry = Geometry<4, 9, true>;
 using ShortGeometry = Geometry<3, 11, false>;
 
-struct Slot { unsigned long long G, K, base; int pad[2]; };
 // What the analysis of a range posts: the characters it owns [c_lo, c_hi) (range-relative; n_own = c_hi - c_lo), the tokens
 // counted in them, its last owned string start (lft, relative to c_lo; -1: none), the block-mask backlog it leaves (v) and --
 // for a range that begins inside a chunk -- how it transforms a backlog: x -> max(x + u, v), mb1 marks in front of its
@@ -97,7 +97,7 @@ template <class Geom>
 struct Ctl {
     int tile_id[2], tk_cnt[2], tk_flag[2];
     int pad0[4];
-    Slot slot[2];
+    Prefix slot[2];                      // the prefix in front of the tile, handed down by the service warp (x unused)
     RangeRec rec[2][Geom::NW];
     int tokstep[Geom::NW][2][Geom::RS];  // tokens per step
     int nsa[Geom::NW][2][Geom::RS];      // first split after the step (range-relative character index, -1: none)
@@ -230,6 +230,109 @@ __device__ __forceinline__ uint32_t pk_ps(uint32_t k) { return (k >> 30) & 1u; }
 __device__ __forceinline__ int bfind32(uint32_t x) { int r; asm("bfind.u32 %0, %1;" : "=r"(r) : "r"(x)); return r; }   // index of the highest set bit (-1: none)
 __device__ __forceinline__ int ld_vs32(const int *p) { int v; asm volatile("ld.volatile.shared.s32 %0, [%1];" : "=r"(v) : "r"(smem_u32(p))); return v; }
 __device__ __forceinline__ void st_vs32(int *p, int v) { asm volatile("st.volatile.shared.s32 [%0], %1;" ::"r"(smem_u32(p)), "r"(v) : "memory"); }
+
+// What ranges [0, end) of a tile add to the prefix, from their records (warp-wide, end <= NW): the service warp sums the
+// whole tile, a compute warp the ranges in front of its own
+template <int NW>
+__device__ __forceinline__ TileSum sum_ranges(const RangeRec (&rec)[NW], int end, int lane)
+{
+    const RangeRec a = rec[lane < NW ? lane : 0];
+    const bool in = lane < end;
+    const int mn = in ? a.n_own : 0;
+    int pn = mn;                                   // inclusive prefix of characters over the ranges
+#pragma unroll
+    for (int d = 1; d < NW; d <<= 1) { const int t = __shfl_up_sync(FULL, pn, d); if (lane >= d) pn += t; }
+    const unsigned hl = __ballot_sync(FULL, in && a.lft >= 0);
+    const int lv = __shfl_sync(FULL, pn - mn + a.lft, hl ? 31 - __clz(hl) : 0);
+    return TileSum{__reduce_add_sync(FULL, mn), __reduce_add_sync(FULL, in ? a.ntok : 0), hl ? lv : -1};
+}
+
+// ---- look-ahead walk (rare): the whitespace chunk open at the end of a tile did not close inside
+// the right halo.  Warp 0 scans forward from global byte `pos0` until the chunk closes (a SPACE
+// character or the end of the string) and reports whether a mark occurs up to and including the
+// closing character.  Exact but slow; it exists so that arbitrarily long space-free runs stay
+// bit-exact (latok.c:218-244 has unbounded reach).
+static __device__ bool walk_ahead(const Params &p, const Tables &t, long long pos0, int lane)
+{
+    const uint8_t *in = p.in;
+    // end of the string that contains pos0: first offset > pos0 (32 probes per round)
+    long long e;
+    {
+        long long lo = 0, hi = p.n_strings;              // the answer is in [lo, hi]; offsets[n_strings] = n_bytes > pos0
+        while (lo < hi) {
+            const long long step = (hi - lo + 31) / 32;
+            const long long c = lo + step * lane;
+            const bool gt = c >= hi || p.offsets[c] > pos0;       // monotone over the lanes
+            const unsigned b = __ballot_sync(0xFFFFFFFFu, gt);
+            if (b == 0u) lo = lo + 31 * step + 1;
+            else {
+                const int f = __ffs(b) - 1;
+                const long long nh = lo + step * f;
+                if (f > 0) lo = lo + step * (f - 1) + 1;
+                hi = nh < hi ? nh : hi;
+            }
+        }
+        e = p.offsets[lo];
+    }
+    struct G { const uint8_t *in; long long q, n; __device__ uint32_t operator[](int k) const { long long a = q + k; return a < n ? (uint32_t)in[a] : 0u; } };
+    // the character in front of pos0 (we are strictly inside the string, so it exists)
+    uint32_t prev_w;
+    {
+        long long pp = pos0 - 1;
+        for (int k = 0; k < 8 && pp > 0 && (in[pp] & 0xC0u) == 0x80u; ++k) --pp;
+        prev_w = classify_at(G{in, pp, p.n_bytes}, t);
+    }
+    // 32 bytes per trip, one byte per lane; the rules are evaluated for the characters that begin in the first ZONE
+    // bytes (their next and after-next characters begin inside the 32 bytes), then the window moves on by ZONE
+    constexpr int ZONE = 24, AHEAD = 4;
+    bool any = false;
+    for (long long q0 = pos0; q0 < e; q0 += AHEAD * ZONE) {
+      // the bytes of AHEAD windows are fetched together (the walk runs into text nobody has touched yet: DRAM latency)
+      uint32_t bytes[AHEAD];
+#pragma unroll
+      for (int g = 0; g < AHEAD; ++g) {
+          const long long pos = q0 + g * ZONE + lane;
+          bytes[g] = pos < e ? (uint32_t)in[pos] : 0x80u;
+      }
+#pragma unroll
+      for (int g = 0; g < AHEAD; ++g) {
+        const long long q = q0 + g * ZONE;
+        if (q >= e) break;
+        const long long pos = q + lane;
+        const bool inb = pos < e;
+        const uint32_t byte = bytes[g];
+        const bool lead = inb && (byte & 0xC0u) != 0x80u;
+        const unsigned leads = __ballot_sync(0xFFFFFFFFu, lead);
+        uint32_t w = 0;
+        if (lead) w = byte < 0x80u ? (uint32_t)t.ascii_feat[byte] : classify_at(G{in, pos, p.n_bytes}, t);
+        const unsigned above = lane == 31 ? 0u : (leads & (0xFFFFFFFFu << (lane + 1)));
+        const unsigned above2 = above & (above - 1u);
+        const unsigned below = leads & ((1u << lane) - 1u);
+        const uint32_t nw = __shfl_sync(0xFFFFFFFFu, w, above ? __ffs(above) - 1 : 0);
+        const uint32_t aw = __shfl_sync(0xFFFFFFFFu, w, above2 ? __ffs(above2) - 1 : 0);
+        uint32_t pw = __shfl_sync(0xFFFFFFFFu, w, below ? 31 - __clz(below) : 0);
+        if (!below) pw = prev_w;
+        const bool has_next = above != 0u, has_an = above2 != 0u;
+        bool closer = false, mk = false;
+        const bool ev = lead && lane < ZONE;
+        if (ev) {
+            const uint32_t full = make_word(pw, w, nw, aw, false, !has_next, !has_an);
+            mk = rule_mark(p.rules, full);
+            closer = ((full >> 5) & 1u) || !has_next;
+        }
+        const unsigned bc = __ballot_sync(0xFFFFFFFFu, ev && closer), bm = __ballot_sync(0xFFFFFFFFu, ev && mk);
+        if (bc) {
+            const int first = __ffs(bc) - 1;
+            return any || (bm & (first == 31 ? 0xFFFFFFFFu : ((2u << first) - 1u))) != 0u;
+        }
+        any = any || bm != 0u;
+        if (any) return true;
+        const unsigned zone = leads & ((1u << ZONE) - 1u);
+        if (zone) prev_w = __shfl_sync(0xFFFFFFFFu, w, 31 - __clz(zone));
+      }
+    }
+    return any;
+}
 
 template <class Geom, bool kDefault, bool kFeats>
 __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize5_kernel(const Params p)
@@ -811,31 +914,13 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
     if (warp == 0) {
         for (int k = 0;; ++k) {
             const int s = k & 1;
-            int n = 0, ntok = 0, lft_rel = -1;
+            TileSum sum;                                       // tile totals from what the ranges have posted (ctl.rec)
             // lane i < NW: what range i posted with its FIRST analysis (nothing entering): backlog left (sf0), flags,
             // and -- only for ranges that begin inside a chunk (LO_FOUND clear) -- marks - closers (su; NEG: a string
             // boundary resets the backlog) and the marks in front of the first closer (smb1) ...
             int su = 0, sf0 = 0, smb1 = 0, sflags = RangeRec::CLOSED | RangeRec::LO_FOUND;
             // ... what it has been analysed with so far, and the backlog it left the last time
             int x_used = 0, far_used = 0, v_last = 0;
-            // tile totals from what the ranges have posted (ctl.rec)
-            auto sum_up = [&](bool first) {
-                const RangeRec a = ctl.rec[s][lane < NW ? lane : 0];
-                const int mn = lane < NW ? a.n_own : 0, mk = lane < NW ? a.ntok : 0;
-                int pn = mn;                                   // inclusive prefix of characters over the ranges
-#pragma unroll
-                for (int d = 1; d < NW; d <<= 1) { const int t = __shfl_up_sync(FULL, pn, d); if (lane >= d) pn += t; }
-                n = __shfl_sync(FULL, pn, NW - 1);
-                ntok = __reduce_add_sync(FULL, mk);
-                const unsigned hl = __ballot_sync(FULL, lane < NW && a.lft >= 0);
-                const int src = hl ? 31 - __clz(hl) : 0;
-                const int lv = __shfl_sync(FULL, pn - mn + a.lft, src);
-                lft_rel = hl ? lv : -1;
-                if (first && lane < NW) {
-                    su = a.u; sf0 = a.v; smb1 = a.mb1; sflags = a.flags; v_last = a.v;
-                    far_used = (a.flags & RangeRec::GUESSED_HOT) ? 1 : 0;
-                }
-            };
             // Backlog entering / hot tail of every range, given the backlog `x_tile` that enters the tile.  A range whose
             // result depends on something other than what it was analysed with is analysed AGAIN -- by this warp, at once:
             // the warp that owns the range is busy with its next tile and would only get to it ~10 us later, with the whole
@@ -926,12 +1011,17 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                     }
                     __threadfence_block();
                     __syncwarp();
-                    sum_up(false);
+                    sum = sum_ranges(ctl.rec[s], NW, lane);
                 }
                 return x_out;
             };
             nb_sync(BAR_AGG + s, NTH);               // every range of the tile has been analysed and posted
-            sum_up(true);
+            sum = sum_ranges(ctl.rec[s], NW, lane);
+            if (lane < NW) {
+                const RangeRec a = ctl.rec[s][lane];
+                su = a.u; sf0 = a.v; smb1 = a.mb1; sflags = a.flags; v_last = a.v;
+                far_used = (a.flags & RangeRec::GUESSED_HOT) ? 1 : 0;
+            }
             const long long tile = ld_vs32(&ctl.tile_id[s]);
             if (tile >= p.ntiles) break;
             // The aggregate is published under the assumption that no backlog enters the tile (true for almost every tile).
@@ -942,13 +1032,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
             int v = 0;
             if (!begins_inside) {
                 v = resolve(0);
-                if (lane == 0) {
-                    uint4 r;
-                    r.x = (p.epoch << 2) | 1u;
-                    r.y = (unsigned)n | ((lft_rel >= 0 ? (unsigned)(lft_rel + 1) : 0u) << 16);
-                    r.z = (unsigned)ntok | ((unsigned)v << 16); r.w = 0;
-                    st_rec(p.agg + tile, r);
-                }
+                if (lane == 0) publish_agg(p.agg + tile, p.epoch, AGG_AGGREGATE, sum, v);
             }
             const Prefix pre = lookback(tile, p, lane);
             if (begins_inside || pre.x != 0) {
@@ -961,21 +1045,13 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
 #endif
             }
             if (lane == 0) {
-                IncRec *ir = p.inc + tile;
-                uint4 a, bq;
-                const unsigned long long Gn = pre.G + (unsigned long long)n, Kn = pre.K + (unsigned long long)ntok;
-                const unsigned long long Bn = lft_rel >= 0 ? pre.G + (unsigned long long)lft_rel : pre.base;
-                a.x = (unsigned)Gn; a.y = (unsigned)(Gn >> 32); a.z = (unsigned)Bn; a.w = (unsigned)(Bn >> 32);
-                bq.x = (unsigned)Kn; bq.y = (unsigned)(Kn >> 32); bq.z = (unsigned)v; bq.w = 0;
-                st_rec(ir, a); st_rec(reinterpret_cast<uint4 *>(ir) + 1, bq);
+                Prefix inc = advance(pre, sum);
+                inc.x = v;
+                publish_inc(p.inc + tile, inc);
                 __threadfence();
-                uint4 r;
-                r.x = (p.epoch << 2) | 2u;
-                r.y = (unsigned)n | ((lft_rel >= 0 ? (unsigned)(lft_rel + 1) : 0u) << 16);
-                r.z = (unsigned)ntok | ((unsigned)v << 16); r.w = 0;
-                st_rec(p.agg + tile, r);
-                Slot &sl = ctl.slot[s];
-                sl.G = pre.G; sl.K = pre.K; sl.base = pre.base;
+                publish_agg(p.agg + tile, p.epoch, AGG_INCLUSIVE, sum, v);
+                Prefix &sl = ctl.slot[s];            // (not x: storing it costs the short geometry a spill)
+                sl.G = pre.G; sl.base = pre.base; sl.K = pre.K;
                 __threadfence_block();
             }
             __syncwarp();
@@ -1313,17 +1389,9 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                         hit = fc_hit;
                     }
                     for (long long rr = r - 1; !hit && rr >= 0; --rr) {            // ranges that do not begin at a closer only
-                        const uint4 *o = reinterpret_cast<const uint4 *>(p.osum + rr);
-                        uint4 h;
-                        unsigned spins = 0;
-                        for (;;) {
-                            h = ld_rec(o);
-                            if (h.y == p.epoch) break;
-                            if (++spins > SPIN_LIMIT) { atomicOr(&p.result->error, 1u); break; }
-                        }
-                        __threadfence();
-                        add8(acc, ld_rec(o + 1), ld_rec(o + 2));
-                        hit = h.x != 0u;
+                        const Open o = wait_open(p.osum + rr, p.epoch, p.result);
+                        add8(acc, o.lo, o.hi);
+                        hit = o.has_split;
                     }
                 };
                 {
@@ -1478,13 +1546,7 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         }
         if (kFeats) {
             // the token open at the end of the range, for ranges that do not begin at a chunk closer
-            if (lane == 0) {
-                uint4 *o = reinterpret_cast<uint4 *>(p.osum + r);
-                st_rec(o + 1, make_uint4(fc[0], fc[1], fc[2], fc[3]));
-                st_rec(o + 2, make_uint4(fc[4], fc[5], fc[6], 0u));
-                __threadfence();
-                st_rec(o, make_uint4(fc_hit ? 1u : 0u, p.epoch, 0u, 0u));
-            }
+            if (lane == 0) publish_open(p.osum + r, p.epoch, fc_hit, fc);
         }
         if (r == p.nranges - 1 && lane == 0) {
             p.result->n_chars = G_in + (unsigned long long)n_own;
@@ -1507,8 +1569,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
                 __threadfence_block();
                 st_vs32(&ctl.tk_flag[s], k + 1);
             } else {
-                unsigned spins = 0;
-                while (ld_vs32(&ctl.tk_flag[s]) != k + 1) { if (++spins > (1u << 26)) { atomicOr(&p.result->error, 1u); break; } }
+                Watchdog wd{SPIN_TICKET, false};
+                while (ld_vs32(&ctl.tk_flag[s]) != k + 1 && !wd.expired(p.result)) {}
                 t = ld_vs32(&ctl.tile_id[s]);
             }
         }
@@ -1523,10 +1585,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         nb_arrive(BAR_AGG + s, NTH);
     };
     auto wait_window = [&](int b, unsigned &phase_bits) {
-        unsigned spins = 0;
-        while (!mbar_try_wait(mbar + 2 * cw + b, (phase_bits >> b) & 1u)) {
-            if (++spins > (1u << 24)) { if (lane == 0) atomicOr(&p.result->error, 1u); break; }   // watchdog: never hang the device
-        }
+        Watchdog wd{SPIN_WINDOW, false};
+        while (!mbar_try_wait(mbar + 2 * cw + b, (phase_bits >> b) & 1u) && !wd.expired(p.result)) {}
         phase_bits ^= 1u << b;
     };
     // write out tile `tile` (iteration kk): wait for its prefix, then pass D
@@ -1536,25 +1596,8 @@ __global__ void __launch_bounds__(Geom::NTH, kDefault ? Geom::CTAS : 1) tokenize
         nb_sync(BAR_PRE + s, NTH);
         PROF5(4);
         // own prefix: the tile's plus the ranges before this one
-        unsigned long long G_in, K_in, base_in;
-        {
-            const Slot sl = ctl.slot[s];
-            const RangeRec a = ctl.rec[s][lane < NW ? lane : 0];
-            const bool before = lane < cw;
-            const int pn = __reduce_add_sync(FULL, before ? a.n_own : 0), pkk = __reduce_add_sync(FULL, before ? a.ntok : 0);
-            int pnx = lane < NW ? a.n_own : 0;            // exclusive prefix of characters per range
-            {
-                int inc = pnx;
-#pragma unroll
-                for (int d = 1; d < NW; d <<= 1) { const int t = __shfl_up_sync(FULL, inc, d); if (lane >= d) inc += t; }
-                pnx = inc - pnx;
-            }
-            const unsigned hl = __ballot_sync(FULL, before && a.lft >= 0);
-            const int lv = __shfl_sync(FULL, pnx + a.lft, hl ? 31 - __clz(hl) : 0);
-            G_in = sl.G + (unsigned long long)pn; K_in = sl.K + (unsigned long long)pkk;
-            base_in = hl ? sl.G + (unsigned long long)lv : sl.base;
-        }
-        output(r, s, G_in, K_in, base_in);
+        const Prefix in = advance(ctl.slot[s], sum_ranges(ctl.rec[s], cw, lane));
+        output(r, s, in.G, in.K, in.base);
         PROF5(5);
     };
 
