@@ -147,7 +147,8 @@ struct Batch {
     cudaEvent_t ev_h2d = nullptr;                   // inputs have arrived on the device (copy-in stream)
     cudaEvent_t ev_index = nullptr;                 // string index built (aux stream)
     cudaEvent_t ev_k0 = nullptr, ev_k1 = nullptr;   // around the tokenize kernel (timing)
-    cudaEvent_t ev_kdone = nullptr;                 // last device work that touches this set (compute stream)
+    cudaEvent_t ev_kernels = nullptr;               // the batch's kernels are done (compute stream)
+    cudaEvent_t ev_kdone = nullptr;                 // last device work that touches this set (result stream or compute stream)
     bool submitted = false, sized = false, inputs_on_stream = false;
     const uint8_t *cur_in = nullptr;
     const long long *cur_off = nullptr;
@@ -161,7 +162,7 @@ struct Batch {
         d_in.release(); d_off.release(); d_first.release(); d_char_off.release(); d_tok_off.release();
         d_splits.release(); d_feats.release(); d_matrix.release(); d_spans.release(); d_spans16.release();
         d_result.release(); h_result.release(); h_in.release(); h_off.release();
-        for (cudaEvent_t *ev : {&ev_h2d, &ev_index, &ev_k0, &ev_k1, &ev_kdone}) { if (*ev) cudaEventDestroy(*ev); *ev = nullptr; }
+        for (cudaEvent_t *ev : {&ev_h2d, &ev_index, &ev_k0, &ev_k1, &ev_kernels, &ev_kdone}) { if (*ev) cudaEventDestroy(*ev); *ev = nullptr; }
     }
 };
 
@@ -169,8 +170,9 @@ struct latok_b200_engine {
     int device = 0;
     int n_sm = 0;
     // compute: kernels; aux: string index of the next batch while the previous one is tokenized;
-    // s_in / s_out: host -> device and device -> host copies (PCIe is full duplex: the three overlap)
-    cudaStream_t stream = nullptr, aux = nullptr, s_in = nullptr, s_out = nullptr;
+    // s_in / s_out: host -> device and device -> host copies (PCIe is full duplex: the three overlap); s_res: the result
+    // counters of a batch to the host, off the compute stream, where the copy would hold back the next batch's kernels
+    cudaStream_t stream = nullptr, aux = nullptr, s_in = nullptr, s_out = nullptr, s_res = nullptr;
     cudaEvent_t ev_t0 = nullptr, ev_t1 = nullptr, ev_b0 = nullptr, ev_b1 = nullptr;
     TableLayout tl{};
     RuleSet rules{};
@@ -280,14 +282,14 @@ int latok_b200_create(int device, size_t max_batch_bytes, int64_t max_strings, l
     int rc = [&]() -> int {
         CU(cudaSetDevice(device));
         CU(cudaDeviceGetAttribute(&e->n_sm, cudaDevAttrMultiProcessorCount, device));
-        for (cudaStream_t *st : {&e->stream, &e->aux, &e->s_in, &e->s_out}) CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
+        for (cudaStream_t *st : {&e->stream, &e->aux, &e->s_in, &e->s_out, &e->s_res}) CU(cudaStreamCreateWithFlags(st, cudaStreamNonBlocking));
         CU(cudaEventCreate(&e->ev_t0)); CU(cudaEventCreate(&e->ev_t1));
         CU(cudaEventCreate(&e->ev_b0)); CU(cudaEventCreate(&e->ev_b1));
         if (int r = build_table(e)) return r;
         e->rules = default_rules();
         for (Batch &b : e->set) {
             CU(cudaEventCreate(&b.ev_k0)); CU(cudaEventCreate(&b.ev_k1));
-            for (cudaEvent_t *ev : {&b.ev_h2d, &b.ev_index, &b.ev_kdone}) CU(cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
+            for (cudaEvent_t *ev : {&b.ev_h2d, &b.ev_index, &b.ev_kernels, &b.ev_kdone}) CU(cudaEventCreateWithFlags(ev, cudaEventDisableTiming));
             if (int r = b.d_result.ensure(1, true)) return r;
             if (int r = b.h_result.ensure(1)) return r;
         }
@@ -315,13 +317,13 @@ int latok_b200_destroy(latok_b200_engine *e)
 {
     if (!e) return LATOK_B200_OK;
     cudaSetDevice(e->device);
-    for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out}) if (st) cudaStreamSynchronize(st);
+    for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out, e->s_res}) if (st) cudaStreamSynchronize(st);
     e->d_table.release(); e->d_scratch.release(); e->d_scratch2.release(); e->d_scratch3.release();
     e->agg.release(); e->inc.release(); e->osum.release(); e->d_planes.release();
     e->d_tok_bytes.release(); e->d_blk_local.release(); e->d_group_tot.release(); e->d_group_pref.release(); e->d_starts.release();
     for (Batch &b : e->set) b.release();
     for (cudaEvent_t ev : {e->ev_t0, e->ev_t1, e->ev_b0, e->ev_b1}) if (ev) cudaEventDestroy(ev);
-    for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out}) if (st) cudaStreamDestroy(st);
+    for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out, e->s_res}) if (st) cudaStreamDestroy(st);
     delete e;
     return LATOK_B200_OK;
 }
@@ -451,8 +453,10 @@ static int run_device(latok_b200_engine *e, Batch &b)
         CU(cudaGetLastError());
         e->launches += 1;
     }
-    CU(cudaMemcpyAsync(b.h_result.p, b.d_result.p, sizeof(Result), cudaMemcpyDeviceToHost, e->stream));
-    CU(cudaEventRecord(b.ev_kdone, e->stream));
+    CU(cudaEventRecord(b.ev_kernels, e->stream));
+    CU(cudaStreamWaitEvent(e->s_res, b.ev_kernels, 0));
+    CU(cudaMemcpyAsync(b.h_result.p, b.d_result.p, sizeof(Result), cudaMemcpyDeviceToHost, e->s_res));
+    CU(cudaEventRecord(b.ev_kdone, e->s_res));
     b.submitted = true;
     b.sized = false;
     return LATOK_B200_OK;

@@ -94,10 +94,19 @@ cudaError_t launch_parse_matrix(const uint8_t *in, long long n_bytes, const long
 }
 
 // =====================================================================================================
+// x / d for 0 <= x < 2^63 without a 64-bit division (a long software sequence on the GPU): m = floor((2^64 - 1) / d)
+// puts the high half of x * m at the quotient or one below it, and the remainder tells which.
+__device__ __forceinline__ long long div_by(long long x, int d, unsigned long long m)
+{
+    unsigned long long q = __umul64hi((unsigned long long)x, m);
+    if ((unsigned long long)x - q * (unsigned)d >= (unsigned)d) ++q;
+    return (long long)q;
+}
+
 // tile_first_str[t] = first string whose byte offset is >= t * TILE  (t = 0 .. ntiles; [ntiles] = S + 1).
-// Also validates the offsets array.
+// Also validates the offsets array.  tile_m = floor((2^64 - 1) / TILE) (div_by).
 __global__ void tile_index_kernel(const long long *offsets, long long n_strings, long long n_bytes,
-                                  long long *first_str, long long ntiles, int TILE, Result *result)
+                                  long long *first_str, long long ntiles, int TILE, unsigned long long tile_m, Result *result)
 {
     const long long s = blockIdx.x * (long long)blockDim.x + threadIdx.x;
     const int lane = threadIdx.x & 31;
@@ -108,8 +117,8 @@ __global__ void tile_index_kernel(const long long *offsets, long long n_strings,
         bool bad = cur < 0 || cur > n_bytes || cur < prev || (s == 0 && cur != 0) || (s == n_strings && cur != n_bytes);
         if (bad) atomicOr(&result->error, 2u);
         else {
-            t_begin = prev < 0 ? 0 : prev / TILE + 1;
-            t_end = cur / TILE;
+            t_begin = prev < 0 ? 0 : div_by(prev, TILE, tile_m) + 1;
+            t_end = div_by(cur, TILE, tile_m);
             if (t_end > ntiles - 1) t_end = ntiles - 1;
         }
         if (s == n_strings) first_str[ntiles] = n_strings + 1;
@@ -133,7 +142,8 @@ cudaError_t launch_tile_index(const long long *offsets, long long n_strings, lon
     const int bs = 256;
     const long long n = n_strings + 1;
     const unsigned grid = (unsigned)((n + bs - 1) / bs);
-    tile_index_kernel<<<grid, bs, 0, s>>>(offsets, n_strings, n_bytes, tile_first_str, ntiles, tile_bytes, result);
+    tile_index_kernel<<<grid, bs, 0, s>>>(offsets, n_strings, n_bytes, tile_first_str, ntiles, tile_bytes,
+                                          ~0ull / (unsigned)tile_bytes, result);
     return cudaGetLastError();
 }
 
