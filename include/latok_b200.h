@@ -147,7 +147,9 @@ LATOK_B200_API int latok_b200_device_results(latok_b200_engine *e, const int8_t 
  * in the order of first occurrence (within a batch: token order).  A batch commits all at once or not at all.
  * Device memory held: the hash table (16 + 8 bytes per slot, at least 2 slots per key, power-of-two capacity, grown
  * 4x when the load passes one half), the key arena (key bytes + 16 bytes per key: offsets and counts) and 8 bytes per
- * token of the largest batch; encode also uses the engine's 16 bytes per token for the token byte ranges.
+ * token of the largest batch; encode also uses the engine's 16 bytes per token for the token byte ranges.  wordpiece
+ * uses those 16 bytes per token too, and the engine holds 12 bytes per token of the largest batch (piece counts and
+ * offsets, one-piece ids) and 4 bytes per piece of the largest call.
  * LATOK_B200_VOCAB_HASH_BITS=n (read at creation; tests only) keeps n bits of the hash to force collisions. */
 typedef struct latok_b200_vocab latok_b200_vocab;
 /* An empty vocabulary on e's device, sized for expected_keys keys (more grow the table). */
@@ -179,7 +181,22 @@ LATOK_B200_API int latok_b200_vocab_merge(latok_b200_engine *e, latok_b200_vocab
                                           int32_t *map, int on_device);
 /* Drops every key and count; keeps the table and arena allocations (for scratch vocabularies reused per batch). */
 LATOK_B200_API int latok_b200_vocab_clear(latok_b200_vocab *v);
-/* device time of the last encode / import / merge (token byte ranges and a merge's copy-in included; harness) */
+/* WordPiece pieces of the tokens of the engine's (oldest) batch in flight (needs LATOK_B200_SPANS and the text in place,
+ * as for vocab_encode).  Every token is split greedily, longest match first: the longest prefix of the token that is a
+ * key, then the longest continuation that is a key when prefixed with prefix[0, prefix_len), and so on; candidate ends
+ * fall on character boundaries only.  A token of more than max_chars characters (code points), or one with a position
+ * no key matches, is the single piece unk_id (BERT's WordpieceTokenizer, HF tokenizers' WordPiece).  The vocabulary
+ * is only read.  word_offsets: int64 [T+1], token k has the pieces [word_offsets[k], word_offsets[k+1]), in host memory
+ * or, with on_device != 0, in device memory, room for cap_tokens tokens; NULL skips it.  *n_pieces = P.  The pieces stay
+ * in the engine until the next submit / release / wordpiece call.  EINVAL for a vocabulary on another device,
+ * prefix_len outside [0, 64], max_chars outside [1, 1024] or cap_tokens < T (nothing is written); ESTATE without SPANS. */
+LATOK_B200_API int latok_b200_vocab_wordpiece(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *prefix, int prefix_len,
+                                              int max_chars, int32_t unk_id, int64_t cap_tokens, int64_t *word_offsets,
+                                              int64_t *n_pieces, int on_device);
+/* the ids of the last wordpiece call: int32 [P], host or device (4-byte aligned), room for cap_pieces (EINVAL when P is
+ * larger); ESTATE when there are no pieces to fetch */
+LATOK_B200_API int latok_b200_vocab_wordpiece_fetch(latok_b200_engine *e, int64_t cap_pieces, int32_t *ids, int on_device);
+/* device time of the last encode / import / merge / wordpiece (token byte ranges and a merge's copy-in included; harness) */
 LATOK_B200_API int latok_b200_vocab_last_ms(latok_b200_vocab *v, float *ms);
 
 /* ---- measurement hooks (harness only) ----------------------------------------------------- */

@@ -74,6 +74,8 @@ def load():
         "latok_b200_vocab_merge": (C.c_int, [vp, vp, vp, vp, i32]),
         "latok_b200_vocab_clear": (C.c_int, [vp]),
         "latok_b200_vocab_last_ms": (C.c_int, [vp, P(C.c_float)]),
+        "latok_b200_vocab_wordpiece": (C.c_int, [vp, vp, vp, i32, i32, C.c_int32, i64, vp, P(i64), i32]),
+        "latok_b200_vocab_wordpiece_fetch": (C.c_int, [vp, i64, vp, i32]),
     }
     for name, (res, args) in proto.items():
         fn = getattr(L, name)

@@ -185,6 +185,13 @@ struct latok_b200_engine {
     DevBuf<unsigned> d_blk_local, d_group_tot;      // characters in front of every 32-byte word (launch_char_prefix)
     DevBuf<unsigned long long> d_group_pref;
     DevBuf<uint32_t> d_starts;                      // string-start bitmap of the parse matrix
+    // WordPiece pieces (latok_b200_vocab_wordpiece): per token its piece count, then its first piece, and the id of a
+    // one-piece word; the ids of the last call (wp_n of them, -1: none to fetch); the continuation prefix
+    DevBuf<long long> d_wp_off;
+    DevBuf<int32_t> d_wp_first, d_wp_ids;
+    DevBuf<uint8_t> d_wp_pre;
+    PinBuf<long long> h_wp_n;
+    long long wp_n = -1;
     float last_token_bytes_ms = 0.f;
     unsigned epoch = 0;
     long long launches = 0;
@@ -321,6 +328,7 @@ int latok_b200_destroy(latok_b200_engine *e)
     e->d_table.release(); e->d_scratch.release(); e->d_scratch2.release(); e->d_scratch3.release();
     e->agg.release(); e->inc.release(); e->osum.release(); e->d_planes.release();
     e->d_tok_bytes.release(); e->d_blk_local.release(); e->d_group_tot.release(); e->d_group_pref.release(); e->d_starts.release();
+    e->d_wp_off.release(); e->d_wp_first.release(); e->d_wp_ids.release(); e->d_wp_pre.release(); e->h_wp_n.release();
     for (Batch &b : e->set) b.release();
     for (cudaEvent_t ev : {e->ev_t0, e->ev_t1, e->ev_b0, e->ev_b1}) if (ev) cudaEventDestroy(ev);
     for (cudaStream_t st : {e->stream, e->aux, e->s_in, e->s_out, e->s_res}) if (st) cudaStreamDestroy(st);
@@ -333,6 +341,7 @@ int latok_b200_set_pipeline_depth(latok_b200_engine *e, int depth)
     if (!e) return fail(LATOK_B200_EINVAL, "engine is NULL");
     if (depth != 1 && depth != 2) return fail(LATOK_B200_EINVAL, "pipeline depth must be 1 or 2");
     e->nq = 0;                   // batches in flight are dropped (their device work still completes)
+    e->wp_n = -1;
     e->depth = depth;
     return LATOK_B200_OK;
 }
@@ -474,6 +483,7 @@ static int take_set(latok_b200_engine *e, Batch **out)
 {
     if (e->depth == 1) e->nq = 0;
     if (e->nq >= e->depth) return fail(LATOK_B200_ESTATE, "%d batches are in flight: fetch and release the oldest one first", e->nq);
+    e->wp_n = -1;                                   // the pieces of a wordpiece call live until the next submit
     const int s = e->last ^ 1;
     e->last = s;
     e->q[e->nq++] = s;
@@ -655,6 +665,7 @@ int latok_b200_release(latok_b200_engine *e)
     if (!e->nq) return fail(LATOK_B200_ESTATE, "no batch in flight");
     e->q[0] = e->q[1];
     --e->nq;
+    e->wp_n = -1;
     return LATOK_B200_OK;
 }
 
@@ -1055,6 +1066,81 @@ int latok_b200_vocab_encode(latok_b200_engine *e, latok_b200_vocab *v, int add, 
     CU(cudaEventRecord(b.ev_kdone, s));          // the set's inputs are in use until here
     CU(cudaStreamSynchronize(s));
     v->last_ms = elapsed(v->ev[0], v->ev[1]) + (add ? elapsed(v->ev[2], v->ev[3]) : 0.f);
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_wordpiece(latok_b200_engine *e, latok_b200_vocab *v, const uint8_t *prefix, int prefix_len,
+                               int max_chars, int32_t unk_id, int64_t cap_tokens, int64_t *word_offsets, int64_t *n_pieces,
+                               int on_device)
+{
+    if (!v) return fail(LATOK_B200_EINVAL, "vocabulary is NULL");
+    if (!n_pieces) return fail(LATOK_B200_EINVAL, "n_pieces is NULL");
+    FRONT(e, b);
+    if (v->device != e->device) return fail(LATOK_B200_EINVAL, "the vocabulary is on device %d, the engine on device %d", v->device, e->device);
+    if (prefix_len < 0 || prefix_len > 64) return fail(LATOK_B200_EINVAL, "prefix_len = %d, must be in [0, 64]", prefix_len);
+    if (prefix_len && !prefix) return fail(LATOK_B200_EINVAL, "prefix is NULL");
+    if (max_chars < 1 || max_chars > 1024) return fail(LATOK_B200_EINVAL, "max_chars = %d, must be in [1, 1024]", max_chars);
+    e->wp_n = -1;
+    if (int r = size_batch(e, b)) return r;
+    if (!(b.what & LATOK_B200_SPANS)) return fail(LATOK_B200_ESTATE, "spans were not requested at submit");
+    const long long T = b.n_tokens;
+    if (word_offsets && cap_tokens < T) return fail(LATOK_B200_EINVAL, "cap_tokens = %lld, the batch has %lld tokens", (long long)cap_tokens, T);
+    v->last_ms = 0.f;
+    if (int r = e->d_tok_bytes.ensure(2 * (size_t)T + 2)) return r;
+    if (int r = e->d_wp_off.ensure((size_t)T + 1)) return r;
+    if (int r = e->d_wp_first.ensure((size_t)T + 1)) return r;
+    if (int r = e->d_wp_pre.ensure(64)) return r;
+    if (int r = e->h_wp_n.ensure(1)) return r;
+    cudaStream_t s = e->stream;
+    CU(cudaStreamWaitEvent(s, b.ev_kdone, 0));
+    CU(cudaEventRecord(v->ev[0], s));
+    if (T)
+        if (int r = enqueue_token_bytes(e, b, e->d_tok_bytes.p)) return r;
+    VocabParams p = vocab_params(v);
+    p.text = b.cur_in; p.rng = reinterpret_cast<const longlong2 *>(e->d_tok_bytes.p); p.n = T;
+    p.unk = unk_id; p.pre = e->d_wp_pre.p; p.plen = prefix_len; p.max_chars = max_chars;
+    p.wp_off = e->d_wp_off.p; p.wp_first = e->d_wp_first.p;
+    if (prefix_len) CU(cudaMemcpyAsync(e->d_wp_pre.p, prefix, (size_t)prefix_len, cudaMemcpyHostToDevice, s));
+    CU(cudaMemsetAsync(v->st.p, 0, sizeof(VocabStatus), s));
+    CU(launch_vocab(VOCAB_MAX_KEY, p, 0, e->n_sm, s));
+    CU(launch_vocab(VOCAB_WP_COUNT, p, 0, e->n_sm, s));
+    size_t need = 0;
+    CU(vocab_scan(2, nullptr, &need, p, 0, 0, s));
+    if (need > v->scan_tmp.cap) { CU(cudaStreamSynchronize(s)); if (int r = v->scan_tmp.ensure(need)) return r; }
+    CU(vocab_scan(2, v->scan_tmp.p, &need, p, 0, 0, s));
+    CU(cudaEventRecord(v->ev[1], s));
+    CU(cudaMemcpyAsync(e->h_wp_n.p, e->d_wp_off.p + T, sizeof(long long), cudaMemcpyDeviceToHost, s));
+    CU(cudaStreamSynchronize(s));
+    const long long P = *e->h_wp_n.p;
+    if (int r = e->d_wp_ids.ensure((size_t)P + 1)) return r;
+    CU(cudaEventRecord(v->ev[2], s));
+    p.ids = e->d_wp_ids.p;
+    CU(launch_vocab(VOCAB_WP_WRITE, p, 0, e->n_sm, s));
+    CU(cudaEventRecord(v->ev[3], s));
+    e->launches += 4;
+    if (word_offsets)
+        CU(cudaMemcpyAsync(word_offsets, e->d_wp_off.p, ((size_t)T + 1) * sizeof(long long),
+                           on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, s));
+    CU(cudaEventRecord(b.ev_kdone, s));          // the set's inputs are in use until here
+    CU(cudaStreamSynchronize(s));
+    v->last_ms = elapsed(v->ev[0], v->ev[1]) + elapsed(v->ev[2], v->ev[3]);
+    e->wp_n = P;
+    *n_pieces = P;
+    return LATOK_B200_OK;
+}
+
+int latok_b200_vocab_wordpiece_fetch(latok_b200_engine *e, int64_t cap_pieces, int32_t *ids, int on_device)
+{
+    if (!e) return fail(LATOK_B200_EINVAL, "engine is NULL");
+    if (e->wp_n < 0) return fail(LATOK_B200_ESTATE, "no wordpiece pieces to fetch (call latok_b200_vocab_wordpiece first)");
+    if (cap_pieces < e->wp_n) return fail(LATOK_B200_EINVAL, "cap_pieces = %lld, the call has %lld pieces", (long long)cap_pieces, e->wp_n);
+    if (!e->wp_n) return LATOK_B200_OK;
+    if (!ids) return fail(LATOK_B200_EINVAL, "ids is NULL");
+    if (on_device && ((uintptr_t)ids & 3u) != 0) return fail(LATOK_B200_EINVAL, "a device ids array must be 4-byte aligned");
+    if (int r = set_device(e)) return r;
+    CU(cudaMemcpyAsync(ids, e->d_wp_ids.p, (size_t)e->wp_n * sizeof(int32_t),
+                       on_device ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, e->stream));
+    CU(cudaStreamSynchronize(e->stream));
     return LATOK_B200_OK;
 }
 

@@ -175,6 +175,7 @@ struct VocabStatus {
     unsigned long long new_bytes;
     unsigned overflow;             // load limit passed or a probe sequence without a slot: the batch is run again
     unsigned pad;
+    unsigned long long max_key;    // bytes of the longest key (WordPiece)
 };
 struct VocabParams {
     VocabSlot *table;
@@ -195,8 +196,15 @@ struct VocabParams {
     const long long *weight;       // [n]: count of key k (a merge), or NULL: 1 per token
     VocabStatus *st;
     unsigned long long limit;      // new claims the load limit allows in this launch
+    // WordPiece (ids = the pieces, [P]; unk = the id of an unknown word)
+    const uint8_t *pre;            // continuation prefix, pre[0, plen), in device memory
+    int plen;
+    int max_chars;                 // a word of more characters is unk
+    long long *wp_off;             // [n + 1]: pieces per word, then (after the scan) the first piece of every word
+    int32_t *wp_first;             // [n]: the id of a one-piece word
 };
-enum VocabPhase { VOCAB_INSERT, VOCAB_LOOKUP, VOCAB_FLAG, VOCAB_LENS, VOCAB_COMMIT, VOCAB_COUNT, VOCAB_REHASH };
+enum VocabPhase { VOCAB_INSERT, VOCAB_LOOKUP, VOCAB_FLAG, VOCAB_LENS, VOCAB_COMMIT, VOCAB_COUNT, VOCAB_REHASH, VOCAB_MAX_KEY,
+                  VOCAB_WP_COUNT, VOCAB_WP_WRITE };
 cudaError_t launch_vocab(VocabPhase phase, const VocabParams &p, long long n_new, int n_sm, cudaStream_t s);
 // rng[k] = (key_off[k], key_off[k + 1]) for k < n, on the device (a merge's source keys)
 cudaError_t launch_vocab_ranges(const long long *key_off, long long n, longlong2 *rng, int n_sm, cudaStream_t s);

@@ -24,6 +24,10 @@
 // Merge (latok_b200_vocab_merge) is one batch whose tokens are the source's keys in id order, weighted by their counts:
 // vocab_ranges_kernel turns the source's key offsets into the batch's ranges on the device, and the count kernel's ids
 // are the map source id -> destination id.
+// WordPiece (latok_b200_vocab_wordpiece) only reads the table: vocab_max_key_kernel finds the longest key,
+// vocab_wp_count_kernel splits every token greedily, longest piece first (one lane per token; a candidate piece is a Key
+// "prefix + text range", hashed as a running sum while its end moves), a scan of the piece counts gives the word
+// offsets, and vocab_wp_write_kernel writes the ids, searching again only for tokens of several pieces.
 // Keys of up to VOCAB_LONG bytes take one lane each; longer keys (documents reach 64 KB per string) a whole warp each.
 // Integer / memory-bound kernels; no tensor cores.
 #include "latok_internal.h"
@@ -44,9 +48,9 @@ __device__ __forceinline__ unsigned long long fmix64(unsigned long long k)
     return k;
 }
 
-// bytes [p, p + 8) of a key that ends at e, little endian, zero at and beyond e (p < e).  Reads only the aligned 8-byte
-// words that hold a byte of the key, so a key at the very end of an allocation is read in bounds.
-__device__ __forceinline__ unsigned long long key_word(const uint8_t *base, long long p, long long e)
+// bytes [p, p + 8) of a byte range that ends at e, little endian, zero at and beyond e (p < e).  Reads only the aligned
+// 8-byte words that hold a byte of the range, so a range at the very end of an allocation is read in bounds.
+__device__ __forceinline__ unsigned long long range_word(const uint8_t *base, long long p, long long e)
 {
     const long long a = p & ~7LL;
     const int sh = (int)(p & 7);
@@ -57,28 +61,59 @@ __device__ __forceinline__ unsigned long long key_word(const uint8_t *base, long
     return w;
 }
 
-// sum over the key's 8-byte words of a mix keyed by the word index, finalised with the length: a warp adds its lanes'
-// partial sums in any order and gets the value one lane computes.  hmask truncates it (LATOK_B200_VOCAB_HASH_BITS).
-template <bool WARP>
-__device__ __forceinline__ unsigned long long key_hash(const uint8_t *base, long long b, long long e, unsigned long long hmask, int lane)
+// A key: the bytes pre[0, plen) followed by base[b, e).  A token, a claimed key and an arena key have plen = 0; a
+// WordPiece candidate is the continuation prefix followed by a piece of a token (plen = 0 for a word's first piece).
+struct Key {
+    const uint8_t *pre;
+    long long plen;
+    const uint8_t *base;
+    long long b, e;
+    __device__ long long len() const { return plen + e - b; }
+};
+__device__ __forceinline__ Key plain_key(const uint8_t *base, long long b, long long e) { return Key{nullptr, 0, base, b, e}; }
+
+// bytes [q, q + 8) of key k, little endian, zero at and beyond its end (0 <= q < k.len())
+__device__ __forceinline__ unsigned long long key_word(const Key &k, long long q)
 {
-    unsigned long long s = 0;
-    const long long nw = (e - b + 7) >> 3;
-    for (long long i = WARP ? lane : 0; i < nw; i += WARP ? 32 : 1)
-        s += fmix64(key_word(base, b + 8 * i, e) ^ (0x9E3779B97F4A7C15ULL * (unsigned long long)(i + 1)));
-    if (WARP)
-        for (int d = 16; d; d >>= 1) s += __shfl_xor_sync(0xFFFFFFFFu, s, d);
-    const unsigned long long h = fmix64(s ^ (0xD6E8FEB86659FD93ULL * (unsigned long long)(e - b))) & hmask;
+    if (q >= k.plen) return range_word(k.base, k.b + q - k.plen, k.e);
+    unsigned long long w = range_word(k.pre, q, k.plen);
+    const long long room = k.plen - q;
+    if (room < 8 && k.b < k.e) w |= range_word(k.base, k.b, k.e) << (8 * room);
+    return w;
+}
+
+// The hash of a key is the sum over its 8-byte words of a mix keyed by the word index (word_term), finalised with the
+// length (hash_final): a warp adds its lanes' partial sums in any order and gets the value one lane computes, and a
+// WordPiece search keeps the sum of a candidate's whole words while the candidate shrinks.  hmask truncates it
+// (LATOK_B200_VOCAB_HASH_BITS).
+__device__ __forceinline__ unsigned long long word_term(unsigned long long w, long long i)
+{
+    return fmix64(w ^ (0x9E3779B97F4A7C15ULL * (unsigned long long)(i + 1)));
+}
+__device__ __forceinline__ unsigned long long hash_final(unsigned long long s, long long len, unsigned long long hmask)
+{
+    const unsigned long long h = fmix64(s ^ (0xD6E8FEB86659FD93ULL * (unsigned long long)len)) & hmask;
     return h ? h : 1ULL;
 }
 
 template <bool WARP>
-__device__ __forceinline__ bool key_equal(const uint8_t *a, long long ab, const uint8_t *b, long long bb, long long len, int lane)
+__device__ __forceinline__ unsigned long long key_hash(const Key &k, unsigned long long hmask, int lane)
+{
+    unsigned long long s = 0;
+    const long long nw = (k.len() + 7) >> 3;
+    for (long long i = WARP ? lane : 0; i < nw; i += WARP ? 32 : 1) s += word_term(key_word(k, 8 * i), i);
+    if (WARP)
+        for (int d = 16; d; d >>= 1) s += __shfl_xor_sync(0xFFFFFFFFu, s, d);
+    return hash_final(s, k.len(), hmask);
+}
+
+// a == b for two keys of length len
+template <bool WARP>
+__device__ __forceinline__ bool key_equal(const Key &a, const Key &b, long long len, int lane)
 {
     bool eq = true;
     const long long nw = (len + 7) >> 3;
-    for (long long i = WARP ? lane : 0; eq && i < nw; i += WARP ? 32 : 1)
-        eq = key_word(a, ab + 8 * i, ab + len) == key_word(b, bb + 8 * i, bb + len);
+    for (long long i = WARP ? lane : 0; eq && i < nw; i += WARP ? 32 : 1) eq = key_word(a, 8 * i) == key_word(b, 8 * i);
     return WARP ? __all_sync(0xFFFFFFFFu, eq) : eq;
 }
 
@@ -106,13 +141,13 @@ __device__ __forceinline__ void each_key(long long n, Range range, Visit visit, 
 
 __device__ __forceinline__ void set_overflow(VocabStatus *st) { atomicExch(&st->overflow, 1u); }
 
-// the slot of key k = text[r.x, r.y): claimed if absent (add), -1 if absent (lookup) or no slot could be had (overflow
-// flag set).  *committed_id: the key's id when it was committed before this launch, else -1.
+// the slot of `key` (hash h = key_hash(key)), token k of the launch: claimed if absent (add), -1 if absent (lookup) or
+// no slot could be had (overflow flag set).  *committed_id: the key's id when it was committed before this launch, else -1.
 template <bool WARP>
-__device__ long long probe(const VocabParams &p, long long k, longlong2 r, bool add, int lane, long long *committed_id)
+__device__ long long probe(const VocabParams &p, long long k, const Key &key, unsigned long long h, bool add, int lane,
+                           long long *committed_id)
 {
-    const long long len = r.y - r.x;
-    const unsigned long long h = key_hash<WARP>(p.text, r.x, r.y, p.hmask, lane);
+    const long long len = key.len();
     unsigned long long s = h & p.mask;
     for (unsigned long long i = 0; i <= p.mask; ++i, s = (s + 1) & p.mask) {
         VocabSlot v = p.table[s];
@@ -137,16 +172,25 @@ __device__ long long probe(const VocabParams &p, long long k, longlong2 r, bool 
         bool eq;
         if (v.ref & VOCAB_COMMITTED) {
             const long long id = (long long)(v.ref & ~VOCAB_COMMITTED), kb = p.key_off[id];
-            eq = p.key_off[id + 1] - kb == len && key_equal<WARP>(p.text, r.x, p.arena, kb, len, lane);
+            eq = p.key_off[id + 1] - kb == len && key_equal<WARP>(key, plain_key(p.arena, kb, kb + len), len, lane);
             if (eq) { *committed_id = id; return (long long)s; }
         } else {
             const longlong2 o = p.rng[v.ref - 1];
-            eq = o.y - o.x == len && key_equal<WARP>(p.text, r.x, p.text, o.x, len, lane);
+            eq = o.y - o.x == len && key_equal<WARP>(key, plain_key(p.text, o.x, o.y), len, lane);
             if (eq) { *committed_id = -1; return (long long)s; }
         }
     }
     if (add && (!WARP || lane == 0)) set_overflow(p.st);
     return -1;
+}
+
+// the slot of token k = text[r.x, r.y), as probe
+template <bool WARP>
+__device__ __forceinline__ long long probe_token(const VocabParams &p, long long k, longlong2 r, bool add, int lane,
+                                                 long long *committed_id)
+{
+    const Key key = plain_key(p.text, r.x, r.y);
+    return probe<WARP>(p, k, key, key_hash<WARP>(key, p.hmask, lane), add, lane, committed_id);
 }
 
 // first_occ[slot] = min token index over the keys of slots claimed in this launch: one atomicMin per group of lanes
@@ -158,7 +202,7 @@ __global__ void __launch_bounds__(256) vocab_insert_kernel(const VocabParams p)
     each_key(p.n, [&](long long k) { return p.rng[k]; },
              [&](auto warp, long long k, longlong2 r, int lane, int owner) {
         long long id = -1;
-        const long long s = probe<decltype(warp)::value>(p, k, r, true, lane, &id);
+        const long long s = probe_token<decltype(warp)::value>(p, k, r, true, lane, &id);
         if (lane == owner) my_s = s >= 0 && id < 0 ? s : -1;
         if (lane == 0 || !decltype(warp)::value) p.slot[k] = s < 0 ? 0u : (uint32_t)s;
     }, [&](long long k, bool live) {
@@ -175,7 +219,7 @@ __global__ void __launch_bounds__(256) vocab_lookup_kernel(const VocabParams p)
 {
     each_key(p.n, [&](long long k) { return p.rng[k]; }, [&](auto warp, long long k, longlong2 r, int lane, int) {
         long long id = -1;
-        const long long s = probe<decltype(warp)::value>(p, k, r, false, lane, &id);
+        const long long s = probe_token<decltype(warp)::value>(p, k, r, false, lane, &id);
         if (lane == 0 || !decltype(warp)::value) p.ids[k] = s >= 0 && id >= 0 ? (int32_t)id : p.unk;
     }, [](long long, bool) {});
 }
@@ -260,7 +304,7 @@ __global__ void __launch_bounds__(256) vocab_rehash_kernel(const VocabParams p)
 {
     each_key(p.n_keys, [&](long long id) { return make_longlong2(p.key_off[id], p.key_off[id + 1]); },
              [&](auto warp, long long id, longlong2 r, int lane, int) {
-        const unsigned long long h = key_hash<decltype(warp)::value>(p.arena, r.x, r.y, p.hmask, lane);
+        const unsigned long long h = key_hash<decltype(warp)::value>(plain_key(p.arena, r.x, r.y), p.hmask, lane);
         if (decltype(warp)::value && lane != 0) return;
         unsigned long long s = h & p.mask;
         VocabSlot mine; mine.hash = h; mine.ref = VOCAB_COMMITTED | (unsigned long long)id;
@@ -276,6 +320,88 @@ __global__ void __launch_bounds__(256) vocab_ranges_kernel(const long long *key_
 {
     for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < n; k += (long long)gridDim.x * blockDim.x)
         rng[k] = make_longlong2(key_off[k], key_off[k + 1]);
+}
+
+// ---- WordPiece: the pieces of every token (latok_b200_vocab_wordpiece) ---------------------------------------------
+// st->max_key = the longest key of the vocabulary (no candidate longer than it can match)
+__global__ void __launch_bounds__(256) vocab_max_key_kernel(const VocabParams p)
+{
+    long long m = 0;
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < p.n_keys; k += (long long)gridDim.x * blockDim.x)
+        m = max(m, p.key_off[k + 1] - p.key_off[k]);
+    for (int d = 16; d; d >>= 1) m = max(m, __shfl_xor_sync(0xFFFFFFFFu, m, d));
+    if ((threadIdx.x & 31) == 0 && m) atomicMax(&p.st->max_key, (unsigned long long)m);
+}
+
+// more than max_chars characters in text[b, e)?  Counts only as far as max_chars + 1 characters.
+__device__ __forceinline__ bool wp_too_long(const uint8_t *text, long long b, long long e, long long max_chars)
+{
+    long long chars = 0;
+    for (long long q = b; q < e && chars <= max_chars; q += 8) {
+        const unsigned long long w = range_word(text, q, e);          // zero bytes past e: not continuation bytes
+        chars += min(8LL, e - q) - __popcll(w & ~(w << 1) & 0x8080808080808080ULL);
+    }
+    return chars > max_chars;
+}
+
+// Greedy longest-match-first split of the word text[b, e): emit(id) for every piece in order; the number of pieces, or
+// 0 when some start has no piece (the word is then unk).  At every start the candidate ends go down from the longest
+// key the vocabulary holds and stop at the first character boundary whose key (the prefix after the first piece, then
+// text[start, end)) is a key.  The hash of a candidate is the sum of the terms of its whole 8-byte words, kept while
+// `end` moves (a word's term leaves the sum when the word stops being whole), plus the term of its partial last word.
+template <class Emit>
+__device__ __forceinline__ long long wp_search(const VocabParams &p, long long b, long long e, long long max_key, Emit emit)
+{
+    long long n = 0;
+    for (long long start = b; start < e;) {
+        Key key{p.pre, start > b ? (long long)p.plen : 0, p.text, start, min(e, start + max_key - (start > b ? p.plen : 0))};
+        if (key.e <= start) return 0;
+        unsigned long long whole = 0;
+        for (long long i = 0; i < key.len() >> 3; ++i) whole += word_term(key_word(key, 8 * i), i);
+        long long id = -1;
+        for (; key.e > start; --key.e) {
+            const long long len = key.len();
+            if (key.e == e || (__ldg(p.text + key.e) & 0xC0) != 0x80) {
+                const unsigned long long part = len & 7 ? word_term(key_word(key, len & ~7LL), len >> 3) : 0ULL;
+                if (probe<false>(p, 0, key, hash_final(whole + part, len, p.hmask), false, 0, &id) < 0) id = -1;
+                if (id >= 0) break;
+            }
+            if (!(len & 7)) whole -= word_term(key_word(key, len - 8), (len >> 3) - 1);
+        }
+        if (id < 0) return 0;
+        emit(n++, (int32_t)id);
+        start = key.e;
+    }
+    return n;
+}
+
+// wp_off[k] = pieces of token k (1 for an unk word), wp_first[k] = the id of a one-piece word; wp_off[n] = 0 (the
+// scan's total lands there)
+__global__ void __launch_bounds__(256, 2) vocab_wp_count_kernel(const VocabParams p)
+{
+    const long long max_key = (long long)*(volatile unsigned long long *)&p.st->max_key;
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < p.n; k += (long long)gridDim.x * blockDim.x) {
+        const longlong2 r = p.rng[k];
+        int32_t first = p.unk;
+        long long n = 0;
+        if (!wp_too_long(p.text, r.x, r.y, p.max_chars))
+            n = wp_search(p, r.x, r.y, max_key, [&](long long j, int32_t id) { if (j == 0) first = id; });
+        p.wp_off[k] = n ? n : 1;
+        p.wp_first[k] = n == 1 ? first : p.unk;
+    }
+    if (blockIdx.x == 0 && threadIdx.x == 0) p.wp_off[p.n] = 0;
+}
+
+// after the scan of wp_off: the ids of token k's pieces at ids[wp_off[k]]; only words of several pieces search again
+__global__ void __launch_bounds__(256) vocab_wp_write_kernel(const VocabParams p)
+{
+    const long long max_key = (long long)*(volatile unsigned long long *)&p.st->max_key;
+    for (long long k = (long long)blockIdx.x * blockDim.x + threadIdx.x; k < p.n; k += (long long)gridDim.x * blockDim.x) {
+        const long long o = p.wp_off[k];
+        if (p.wp_off[k + 1] - o == 1) { p.ids[o] = p.wp_first[k]; continue; }
+        const longlong2 r = p.rng[k];
+        wp_search(p, r.x, r.y, max_key, [&](long long j, int32_t id) { p.ids[o + j] = id; });
+    }
 }
 
 static unsigned grid_for(long long n, int per_block, int n_sm)
@@ -294,6 +420,9 @@ cudaError_t launch_vocab(VocabPhase phase, const VocabParams &p, long long n_new
     case VOCAB_COMMIT: vocab_commit_kernel<<<grid_for(p.n, 256, n_sm), 256, 0, s>>>(p); break;
     case VOCAB_COUNT: vocab_count_kernel<<<grid_for(p.n, 256, n_sm), 256, 0, s>>>(p); break;
     case VOCAB_REHASH: if (p.n_keys) vocab_rehash_kernel<<<grid_for(p.n_keys, 256, n_sm), 256, 0, s>>>(p); break;
+    case VOCAB_MAX_KEY: if (p.n_keys) vocab_max_key_kernel<<<grid_for(p.n_keys, 256, n_sm), 256, 0, s>>>(p); break;
+    case VOCAB_WP_COUNT: vocab_wp_count_kernel<<<grid_for(p.n, 256, n_sm), 256, 0, s>>>(p); break;
+    case VOCAB_WP_WRITE: if (p.n) vocab_wp_write_kernel<<<grid_for(p.n, 256, n_sm), 256, 0, s>>>(p); break;
     }
     return cudaGetLastError();
 }
@@ -305,11 +434,12 @@ cudaError_t launch_vocab_ranges(const long long *key_off, long long n, longlong2
 }
 
 // which = 0: rank[0..n] (exclusive, in place); 1: key_off[n_keys .. n_keys + n_new] (exclusive, in place, from
-// key_bytes).  tmp == nullptr: *tmp_bytes = the temporary storage the scan needs.
+// key_bytes); 2: wp_off[0..n] (exclusive, in place).  tmp == nullptr: *tmp_bytes = the temporary storage the scan needs.
 cudaError_t vocab_scan(int which, void *tmp, size_t *tmp_bytes, const VocabParams &p, long long n_new, long long key_bytes,
                        cudaStream_t s)
 {
     if (which == 0) return cub::DeviceScan::ExclusiveSum(tmp, *tmp_bytes, p.rank, p.rank, p.n + 1, s);
+    if (which == 2) return cub::DeviceScan::ExclusiveSum(tmp, *tmp_bytes, p.wp_off, p.wp_off, p.n + 1, s);
     return cub::DeviceScan::ExclusiveScan(tmp, *tmp_bytes, p.key_off + p.n_keys, p.key_off + p.n_keys, cuda::std::plus<long long>(), key_bytes,
                                           n_new + 1, s);
 }

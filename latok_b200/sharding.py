@@ -9,7 +9,8 @@ GPUs, gloo on CPU), or a host-side prefix sum when one process drives all device
 
 Token vocabularies (encode_sharded / update_sharded) add one step: every shard counts its tokens into a scratch
 vocabulary on its own device, and the caller's vocabulary merges the scratch vocabularies in shard order, which gives
-the keys, ids and counts one GPU gets from the whole batch.
+the keys, ids and counts one GPU gets from the whole batch.  wordpiece_sharded splits the tokens of every shard against
+the vocabulary or its replica on the shard's device, as encode_sharded(add=False) looks them up.
 """
 from __future__ import annotations
 
@@ -201,6 +202,22 @@ def encode_sharded(vocab, buf: np.ndarray, offsets: np.ndarray, devices: Sequenc
     if stats is not None:
         stats["remap_ms"] = [a.elapsed_time(b) for a, b in events]
     return ids, concat_offsets([o[1] for o in out], [len(o[0]) for o in out])
+
+
+def wordpiece_sharded(vocab, buf: np.ndarray, offsets: np.ndarray, devices: Sequence[int], unk: int, prefix: str = "##",
+                      max_chars: int = 100) -> Tuple[np.ndarray, np.ndarray, np.ndarray]:
+    """`vocab.wordpiece_packed(buf, offsets, unk, prefix, max_chars)` with the batch sharded over `devices`, as
+    `encode_sharded(add=False)`: every shard splits its tokens against `vocab` on `vocab`'s device and against a replica
+    of `vocab` (kept until `vocab` changes) on any other device.  The same (ids int32[P], offsets int64[S+1],
+    word_offsets int64[T+1])."""
+    buf = np.ascontiguousarray(buf, dtype=np.uint8)
+    offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+    targets = [vocab if d == vocab.engine.device else _replica(vocab, d) for d in devices]
+    parts = _run_shards(buf, offsets, devices,
+                        lambda i, b, o: targets[i].wordpiece_packed(b, o, unk, prefix, max_chars))
+    ids = np.concatenate([p[0] for p in parts])
+    pieces = [len(p[0]) for p in parts]
+    return ids, concat_offsets([p[1] for p in parts], pieces), concat_offsets([p[2] for p in parts], pieces)
 
 
 def update_sharded(vocab, buf: np.ndarray, offsets: np.ndarray, devices: Sequence[int],

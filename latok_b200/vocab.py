@@ -7,6 +7,7 @@
     frozen = Vocab.from_tokens([t for t, c in v.most_common() if c >= 5])
     ids, _ = frozen.encode(texts, add=False, unk=-1)
     m = v.merge(w)                       # Counter.update(w); m[i] = v's id of w's key i (w may be on another GPU)
+    ids, offsets, word_offsets = frozen.wordpiece(texts, unk=0)    # WordPiece pieces of every token ("##" + rest)
 
 Keys are the exact token texts (``text[s:e].strip()`` of the tokenizer, no normalisation); ids are dense and follow the
 order of first occurrence, so two vocabularies fed the same batches agree id for id.  A vocabulary lives on one GPU;
@@ -123,6 +124,57 @@ class Vocab:
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         return self._run(buf, offsets, add, unk, "device" if device else "host")
 
+    def wordpiece(self, texts: Sequence[str], unk: int, prefix: str = "##", max_chars: int = 100):
+        """WordPiece pieces of the tokens of `texts`: every token is split greedily into the longest prefix that is a
+        key, then the longest continuations that are keys as `prefix` + rest (BERT's WordpieceTokenizer, HF
+        tokenizers' WordPiece); a token of more than `max_chars` characters, or one that cannot be split, is the single
+        piece `unk`.  Returns (ids int32[P], offsets int64[S+1], word_offsets int64[T+1]): string i has the pieces
+        ids[offsets[i]:offsets[i+1]], token k the pieces ids[word_offsets[k]:word_offsets[k+1]].  Only reads the
+        vocabulary."""
+        return self._wordpiece(*pack_strings(texts), unk, prefix, max_chars, False)
+
+    def wordpiece_packed(self, buf, offsets, unk: int, prefix: str = "##", max_chars: int = 100, device: bool = False):
+        """`wordpiece` for packed UTF-8 (uint8 buffer + int64 offsets[S+1]).  device=True: ids and word_offsets are
+        CUDA tensors on the engine's device (offsets a CPU tensor)."""
+        buf = np.ascontiguousarray(buf, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        return self._wordpiece(buf, offsets, unk, prefix, max_chars, device)
+
+    def _wordpiece(self, buf, offsets, unk: int, prefix, max_chars: int, device: bool):
+        pre = prefix.encode("utf-8", "surrogatepass") if isinstance(prefix, str) else bytes(prefix)
+        pre_buf = C.create_string_buffer(pre, max(len(pre), 1))
+        e = self.engine
+        with e._lock:
+            if e._depth == 2 and e._flight:
+                raise RuntimeError("batches are in flight")
+            e.submit(buf, offsets, SPANS)
+            try:
+                _, n_tokens = e.sizes()
+                tok_off = np.empty(len(offsets), dtype=np.int64)
+                _lib.check(self._L.latok_b200_fetch(e._h, 0, 0, len(offsets) - 1, None, None, None, tok_off.ctypes.data,
+                                                    None, None))
+                if device:
+                    import torch
+                    word_off = torch.empty(n_tokens + 1, dtype=torch.int64, device=f"cuda:{e.device}")
+                    ptr = word_off.data_ptr()
+                else:
+                    word_off = np.empty(n_tokens + 1, dtype=np.int64)
+                    ptr = word_off.ctypes.data
+                n = C.c_int64(0)
+                _lib.check(self._L.latok_b200_vocab_wordpiece(e._h, self._h, pre_buf, len(pre), int(max_chars), int(unk),
+                                                              n_tokens, ptr, C.byref(n), 1 if device else 0))
+                if device:
+                    ids = torch.empty(n.value, dtype=torch.int32, device=word_off.device)
+                    _lib.check(self._L.latok_b200_vocab_wordpiece_fetch(e._h, n.value, ids.data_ptr(), 1))
+                    offs = word_off[torch.from_numpy(tok_off).to(word_off.device)].cpu()    # plumbing: S+1 gathers
+                    return ids, offs, word_off
+                ids = np.empty(n.value, dtype=np.int32)
+                _lib.check(self._L.latok_b200_vocab_wordpiece_fetch(e._h, n.value, ids.ctypes.data if n.value else None, 0))
+                return ids, word_off[tok_off], word_off
+            finally:
+                if e._depth == 2:
+                    e.release()
+
     def merge(self, other: "Vocab", device: bool = False):
         """Counter.update(other) on the device: every key of `other` is added with its count, keys new to `self` get
         the next ids in `other`'s id order.  Returns the map from `other`'s ids to `self`'s: int32 NumPy array of
@@ -225,7 +277,8 @@ class Vocab:
         return v
 
     def last_ms(self) -> float:
-        """Device time of the last encode / update / import / merge (token byte ranges and a merge's copy-in included)."""
+        """Device time of the last encode / update / import / merge / wordpiece (token byte ranges and a merge's copy-in
+        included)."""
         ms = C.c_float(0)
         _lib.check(self._L.latok_b200_vocab_last_ms(self._h, C.byref(ms)))
         return ms.value
